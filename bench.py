@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA path through the C ABI)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU decoder on the host cores
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's outputs to DIR/*.npy
 
 A *step* is one pass of the hot path (floor1 -> coupling -> floor multiply -> IMDCT -> window/overlap-add -> PCM,
 one fused kernel) over one batch of synthetic config-2 input (BASELINE.json configs[1]: 44.1 kHz stereo, 4096
@@ -209,6 +210,26 @@ def cpu_baseline_port(setup, batch, n_streams_sample):
 
 
 CORPUS_FILE = os.path.join(ROOT, "tests", "golden", "test.stereo44khz.ogg")
+DUMP_PCM_SAMPLES = 1 << 23        # 32 MB of float32 PCM values
+DUMP_STATUS_SAMPLES = 1 << 20     # 8 MB of float64 status words: a dump stays under 40 MB at any --streams / --packets
+
+
+def sample_positions(size, k):
+    """The positions a dump samples out of an array of `size` values: all of them up to k, else k drawn with a fixed seed."""
+    import numpy as np
+    if size <= k:
+        return np.arange(size)
+    return np.sort(np.random.default_rng(0).choice(size, size=k, replace=False))
+
+
+def dump_outputs(out_dir, pcm, status):
+    """Write what one step of the device-resident leg hands its caller, for comparing two builds output for output:
+    pcm.npy, the PCM arena (float32), and status.npy, the per-packet status words (float64, exact for uint32), each at
+    sample_positions(len, DUMP_*_SAMPLES): the same positions for the same command line."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "pcm.npy"), pcm[sample_positions(pcm.size, DUMP_PCM_SAMPLES)].astype(np.float32))
+    np.save(os.path.join(out_dir, "status.npy"), status[sample_positions(status.size, DUMP_STATUS_SAMPLES)].astype(np.float64))
 
 
 def workload_config(args):
@@ -277,7 +298,10 @@ def main():
     ap.add_argument("--no-e2e-dense", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/*.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -335,6 +359,8 @@ def main():
     barrier()
     ms = ev0.elapsed_time(ev1)
     launches = ctx.launch_count - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx.fetch_pcm(bh), ctx.status(bh))
     clocks = None
     if sampler:
         # the timed region lasts tens of milliseconds, nvidia-smi samples every 50 ms: keep the same kernel running

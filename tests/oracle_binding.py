@@ -21,7 +21,8 @@ def lib():
     global _LIB
     if _LIB is None:
         path = os.path.join(ORACLE_DIR, "liboracle_synth.so")
-        if not os.path.exists(path) or os.path.getmtime(path) < os.path.getmtime(os.path.join(ORACLE_DIR, "synth_oracle.c")):
+        srcs = [os.path.join(ORACLE_DIR, f) for f in ("synth_oracle.c", "vorbis_mdct.c")]
+        if not os.path.exists(path) or os.path.getmtime(path) < max(map(os.path.getmtime, srcs)):
             subprocess.check_call(["make", "-C", ORACLE_DIR, "port"], stdout=subprocess.DEVNULL)
         L = C.CDLL(path)
         L.por_inverse_db_table.restype = C.POINTER(C.c_float)
@@ -83,6 +84,14 @@ def imdct(x, kind="closed"):
     return out
 
 
+def vorbis_imdct(x):
+    """libvorbis' mdct_backward (oracle/vorbis_mdct.c), the reference's own transform: bit for bit on its dumps."""
+    x = np.ascontiguousarray(x, np.float32)
+    out = np.zeros(2 * len(x), np.float32)
+    lib().por_vorbis_mdct_backward(C.c_int(len(out)), _p(x, C.c_float), _p(out, C.c_float))
+    return out
+
+
 def window(bs0, bs1, blockflag, prev, nxt):
     n = bs1 if blockflag else bs0
     out = np.zeros(n, np.float32)
@@ -134,6 +143,40 @@ def _ref_imdct_cb():
     return C.cast(L.por_imdct_reference, IMDCT_FN)
 
 
+def dump_mdct_pairs(*goldens):
+    """(n, input, output) of every IMDCT in reference dumps: after_envelope in, pcm_after_mdct out."""
+    for g in goldens:
+        oh = of = 0
+        for n in g["blocksize"]:
+            n = int(n)
+            for _ in range(int(g["channels"])):
+                yield n, g["after_envelope"][oh:oh + n // 2], g["pcm_after_mdct"][of:of + n]
+                oh += n // 2
+                of += n
+
+
+def golden_imdct(*goldens):
+    """An IMDCT callback that answers with the transforms stored in the reference dumps `goldens`, looked up by input
+    vector (+0.0 and -0.0 alike): with it the oracle's window and overlap-add run on the reference's own mdct_backward
+    output for those streams. An input the dumps do not hold comes back as NaN, so a comparison with the dump fails."""
+    def key(n, x):
+        return n, (x + np.float32(0)).tobytes()
+    table = {key(n, x): y for n, x, y in dump_mdct_pairs(*goldens)}
+
+    def cb(user, n, x, out):
+        y = table.get(key(n, np.ctypeslib.as_array(x, shape=(n // 2,))))
+        C.memmove(out, (y if y is not None else np.full(n, np.nan, np.float32)).ctypes.data, 4 * n)
+    return IMDCT_FN(cb)
+
+
+def _imdct_kind(imdct):
+    """-> (kind, callback) for por_synth_batch*: "closed", "fast", "reference" (oracle/_ref) or a golden_imdct callback."""
+    if isinstance(imdct, IMDCT_FN):
+        return 2, imdct
+    kind = {"closed": 0, "fast": 1, "reference": 2}[imdct]
+    return kind, _ref_imdct_cb() if kind == 2 else C.cast(None, IMDCT_FN)
+
+
 def synth_batch(setups, batch: abi.Batch, imdct="fast", capture=False):
     """Run the whole-batch oracle. setups: list of abi.Setup. Returns (pcm, status[, captures])."""
     csetups = [s.to_c() for s in setups]
@@ -141,8 +184,7 @@ def synth_batch(setups, batch: abi.Batch, imdct="fast", capture=False):
     cb = batch.to_c()
     pcm = np.zeros(int(batch.pcm_floats), np.float32)
     status = np.zeros(len(batch.packets), np.uint32)
-    kind = {"closed": 0, "fast": 1, "reference": 2}[imdct]
-    fn = _ref_imdct_cb() if kind == 2 else C.cast(None, IMDCT_FN)
+    kind, fn = _imdct_kind(imdct)
     if not capture:
         rc = lib().por_synth_batch(arr, len(csetups), C.byref(cb), kind, fn, None, _p(pcm, C.c_float),
                                    _p(status, C.c_uint32))
@@ -176,8 +218,7 @@ def snr_db(test, ref):
 
 def synth_batch_raw(csetup, cbatch, imdct="fast", capture=False):
     """Whole-batch oracle on raw ctypes structs (one setup), e.g. straight from the host front-end."""
-    kind = {"closed": 0, "fast": 1, "reference": 2}[imdct]
-    fn = _ref_imdct_cb() if kind == 2 else C.cast(None, IMDCT_FN)
+    kind, fn = _imdct_kind(imdct)
     pcm = np.zeros(int(cbatch.pcm_floats), np.float32)
     P = int(cbatch.n_packets)
     status = np.zeros(P, np.uint32)

@@ -47,7 +47,7 @@ def test_descriptors_reproduce_reference_dump(golden, name):
                 assert np.array_equal(ys[yo:yo + k], g["ys"][p, c, :k]), (p, c)
                 yo += k
     # everything downstream through the oracle
-    pcm, status, cap = ob.synth_batch_raw(s, b, imdct="reference" if ob.reference_lib() is not None else "fast", capture=True)
+    pcm, status, cap = ob.synth_batch_raw(s, b, imdct=ob.golden_imdct(g), capture=True)
     assert not status.any()
     oh = of = 0
     for p, n in enumerate(g["blocksize"]):
@@ -60,7 +60,7 @@ def test_descriptors_reproduce_reference_dump(golden, name):
     out = pcm.reshape(Cn, -1)
     assert out.shape == g["pcm"].shape
     assert np.abs(out - g["pcm"]).max() <= 1e-5
-    if ob.reference_lib() is not None and name != "synth_shared_submap":      # (that one's golden PCM is libvorbis', another IMDCT)
+    if name != "synth_shared_submap":      # (that one's golden PCM is libvorbis', not bit-exact with the reference's)
         assert np.array_equal(out, g["pcm"])
     po.close()
 
@@ -84,11 +84,8 @@ def test_malformed_streams_fail_like_the_reference():
     assert lib.ParsedOgg(b"").n_streams == 0
 
 
-@pytest.mark.skipif(ob.reference_lib() is None, reason="oracle/_ref not built")
-def test_error_behaviour_matches_reference_library():
-    """Same inputs through the reference's own C API (hpp:1493): both accept or both reject."""
-    ref = ob.reference_lib()
-    ref.ogg_vorbis_full_read_from_memory.argtypes = [C.c_char_p, C.c_size_t, C.POINTER(C.c_char_p)]
+def error_cases():
+    """The intact mono fixture, three truncated or spliced copies and six copies with one bit flipped."""
     rng = np.random.default_rng(0)
     base = _load("mono44khz")
     cases = [base, base[:5000], base[:27], base[:4000] + base[4100:]]
@@ -96,15 +93,32 @@ def test_error_behaviour_matches_reference_library():
         b = bytearray(base)
         b[int(rng.integers(0, len(b)))] ^= 1 << int(rng.integers(0, 8))
         cases.append(bytes(b))
-    for data in cases:
-        err = C.c_char_p(None)
-        ref_rc = ref.ogg_vorbis_full_read_from_memory(data, len(data), C.byref(err))
+    return cases
+
+
+# What ogg_vorbis_full_read_from_memory of the reference (hpp:1493) does with error_cases(): 1 rejected, 0 accepted.
+# Not recorded by running it: its build is not part of this repository. Derived from its page checks instead, which
+# reject a truncated segment table or body (hpp:84-90) and a CRC mismatch (hpp:98; a single flipped bit always changes
+# the CRC), and the intact file decodes. Where oracle/_ref is built, the test below checks this list against the library.
+REFERENCE_REJECTS = [0, 1, 1, 1, 1, 1, 1, 1, 1, 1]
+
+
+def test_error_behaviour_matches_reference_library():
+    """Same inputs as through the reference's own C API (hpp:1493): both accept or both reject."""
+    cases = error_cases()
+    assert len(cases) == len(REFERENCE_REJECTS)
+    ref = ob.reference_lib()
+    if ref is not None:
+        ref.ogg_vorbis_full_read_from_memory.argtypes = [C.c_char_p, C.c_size_t, C.POINTER(C.c_char_p)]
+        live = [int(ref.ogg_vorbis_full_read_from_memory(d, len(d), C.byref(C.c_char_p(None))) != 0) for d in cases]
+        assert live == REFERENCE_REJECTS
+    for data, ref_rc in zip(cases, REFERENCE_REJECTS):
         try:
             lib.ParsedOgg(data).close()
             ours_rc = 0
         except lib.PovError:
             ours_rc = 1
-        assert (ref_rc != 0) == (ours_rc != 0), (len(data), err.value)
+        assert (ref_rc != 0) == (ours_rc != 0), len(data)
 
 
 def _ogg_crc(page: bytes) -> int:
@@ -179,10 +193,10 @@ def test_packets_spanning_pages(golden, name):
     po = lib.ParsedOgg(data, allow_spanning=True)
     s, b = po.get(0)
     assert b.n_packets == len(g["blocksize"])
-    pcm, status, cap = ob.synth_batch_raw(s, b, imdct="reference" if ob.reference_lib() is not None else "fast", capture=True)
+    pcm, status, cap = ob.synth_batch_raw(s, b, imdct=ob.golden_imdct(g), capture=True)
     assert not status.any()
     out = pcm.reshape(int(g["channels"]), -1)
-    assert out.shape == g["pcm"].shape and np.abs(out - g["pcm"]).max() <= 1e-5
+    assert out.shape == g["pcm"].shape and np.array_equal(out, g["pcm"])
     oh = 0
     for p, n in enumerate(g["blocksize"]):
         for c in range(int(g["channels"])):
@@ -213,10 +227,10 @@ def test_chained_and_multiplexed_logical_streams(golden, kind):
         s, b = po.get(i)
         assert s.channels == int(g["channels"]) and s.sample_rate == int(g["sample_rate"])
         assert b.n_packets == len(g["blocksize"])
-        pcm, status = ob.synth_batch_raw(s, b, imdct="reference" if ob.reference_lib() is not None else "fast")[:2]
+        pcm, status = ob.synth_batch_raw(s, b, imdct=ob.golden_imdct(g))[:2]
         assert not status.any()
         out = pcm.reshape(int(g["channels"]), -1)
-        assert out.shape == g["pcm"].shape and np.abs(out - g["pcm"]).max() <= 1e-5
+        assert out.shape == g["pcm"].shape and np.array_equal(out, g["pcm"])
     po.close()
 
 
