@@ -176,15 +176,24 @@ typedef struct pov_packet {
  * packet yields zero bits, as in the reference (Utils.hpp:389-392). The setup must carry codebook lengths and floor syntax. */
 enum { POV_INPUT_DENSE = 0, POV_INPUT_ENTRIES = 1, POV_INPUT_PACKETS = 2 };
 enum { POV_PCM_PLANAR = 0, POV_PCM_INTERLEAVED = 1 };
+/* Flag OR-ed into pov_batch.pcm_layout (POV_PCM_PLANAR | POV_PCM_S16, POV_PCM_INTERLEAVED | POV_PCM_S16): the kernels store signed
+ * 16-bit PCM instead of float32, converted at the store, so that half the bytes reach device memory and cross PCIe. Every float32
+ * sample x the same batch would hold becomes
+ *     s = clamp(round_half_even(x * 32768), -32768, 32767),   NaN -> 0
+ * (x * 32768 is exact, so s depends on x alone). On finite samples this is libvorbisfile's ov_read on x86-64; NaN, which ov_read
+ * turns into -32768, becomes 0 here (the device's saturating conversion). The intermediates of pov_batch_fetch_stage and
+ * pov_batch_features stay float32. */
+#define POV_PCM_S16 0x100u
 
 typedef struct pov_batch {
 	uint32_t input_kind;      /* POV_INPUT_DENSE | POV_INPUT_ENTRIES */
-	uint32_t pcm_layout;      /* POV_PCM_PLANAR (matches gotPcmData, hpp:971) | POV_PCM_INTERLEAVED */
+	uint32_t pcm_layout;      /* POV_PCM_PLANAR (matches gotPcmData, hpp:971) | POV_PCM_INTERLEAVED, optionally | POV_PCM_S16 */
 	uint32_t n_streams;  const pov_stream* streams;
 	uint32_t n_packets;  const pov_packet* packets;
 	const uint16_t* ys;       uint64_t n_ys;        /* Y arena */
 	const void*     payload;  uint64_t payload_bytes; /* dense spectra (float) or residue payload */
-	uint64_t pcm_floats;      /* size of the PCM arena this batch writes (floats) */
+	uint64_t pcm_floats;      /* size of the PCM arena this batch writes, in samples: floats, or int16_t with POV_PCM_S16
+	                             (pov_stream.pcm_base, pcm_frames and pov_packet.pcm_off count samples in both cases) */
 } pov_batch;
 
 /* debug stages, named after the reference's dump entries (hpp:518,560,561,585,1171,1211,1254,1265,1051) */
@@ -248,9 +257,12 @@ const char* pov_batch_kernel_name(const pov_ctx* ctx, const pov_batch_handle* h)
 /* Launch the staged path instead: one kernel per reference stage, every intermediate materialised in HBM so
  * that pov_batch_fetch_stage can return it. Produces the same PCM. */
 int  pov_batch_run_staged(pov_ctx* ctx, pov_batch_handle* h);
-/* Device->host copy of the PCM arena (pcm_floats floats; async unless `sync`). */
+/* Device->host copy of the PCM arena (pcm_floats floats; async unless `sync`). POV_ERR_ARG on a POV_PCM_S16 batch. */
 int  pov_batch_fetch_pcm(pov_ctx* ctx, pov_batch_handle* h, float* out, uint64_t n_floats, int sync);
-/* Device pointer of the PCM arena (for callers that consume PCM on the GPU). */
+/* The same for a POV_PCM_S16 batch: n_values int16 samples (<= pcm_floats). POV_ERR_ARG on a float32 batch. */
+int  pov_batch_fetch_pcm_s16(pov_ctx* ctx, pov_batch_handle* h, int16_t* out, uint64_t n_values, int sync);
+/* Device pointer of the PCM arena (for callers that consume PCM on the GPU): float[pcm_floats], or int16_t[pcm_floats] for a
+ * POV_PCM_S16 batch. */
 void* pov_batch_pcm_dev(pov_batch_handle* h);
 /* One debug stage of one (packet, channel) after pov_batch_run_staged; `out_bytes` must match the stage size. */
 int  pov_batch_fetch_stage(pov_ctx* ctx, pov_batch_handle* h, uint32_t packet, uint32_t channel, int stage,
@@ -297,6 +309,19 @@ int  pov_ogg_vorbis_decode_memory(pov_ctx* ctx, const uint8_t* data, size_t len,
                                   pov_decoded* out);
 void pov_decoded_free(pov_decoded* d);
 
+/* The same decode with signed 16-bit output (the POV_PCM_S16 conversion, done by the kernels): `pcm` equals that rule applied to
+ * what pov_ogg_vorbis_decode_memory returns. No debug dump: its format is float32. */
+typedef struct pov_decoded_s16 {
+	uint32_t channels;
+	uint32_t sample_rate;
+	uint64_t frames;          /* frames per channel */
+	uint32_t audio_packets;
+	uint32_t reserved;
+	int16_t* pcm;             /* planar [channels][frames]; owned by the library, free with pov_decoded_s16_free */
+} pov_decoded_s16;
+int  pov_ogg_vorbis_decode_memory_s16(pov_ctx* ctx, const uint8_t* data, size_t len, pov_decoded_s16* out);
+void pov_decoded_s16_free(pov_decoded_s16* d);
+
 /* Decode a corpus of independent files with `host_threads` front-end threads (0 = all cores but one, which is left to
  * the calling thread) feeding this context's GPU. The context keeps the sibling stream, device arenas and pinned
  * staging buffers of the call for the next one; POV_CORPUS_TIMING=1 prints where the calling thread's time went.
@@ -313,6 +338,15 @@ typedef int (*pov_pcm_sink)(uint32_t file_index, uint32_t channels, uint64_t fra
 int  pov_decode_corpus_pcm(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* data, const size_t* len,
                            uint32_t host_threads, pov_pcm_sink sink, void* user,
                            uint64_t* frames_out, uint64_t* total_values_out, double* checksum_out);
+
+/* The corpus decode with signed 16-bit output (POV_PCM_S16 conversion on the device): half the device -> host bytes per sample.
+ * `sink` (may be NULL: decode and count only) has the semantics of pov_decode_corpus_pcm's — file order, `planar` valid during
+ * the call only, a non-zero return stops the decode with POV_ERR_STREAM. `sum_out` is the exact integer sum of every delivered
+ * sample (independent of summation order, unlike the float64 checksum). */
+typedef int (*pov_pcm_sink_s16)(uint32_t file_index, uint32_t channels, uint64_t frames, const int16_t* planar, void* user);
+int  pov_decode_corpus_s16(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* data, const size_t* len,
+                           uint32_t host_threads, pov_pcm_sink_s16 sink, void* user,
+                           uint64_t* frames_out, uint64_t* total_values_out, int64_t* sum_out);
 
 /* Host-only front-end (no GPU needed): parse a whole Ogg/Vorbis file into descriptor batches, one per logical stream
  * (Ogg framing hpp:51-102,1433-1484; headers hpp:1283-1373; per-packet entropy decode hpp:498-517, 711-757). The

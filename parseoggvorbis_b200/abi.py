@@ -24,6 +24,7 @@ POV_OK, POV_ERR_ARG, POV_ERR_CUDA, POV_ERR_STREAM, POV_ERR_UNSUPPORTED = range(5
 POV_PKT_OK, POV_PKT_FLOOR_PREDICTED, POV_PKT_FLOOR_RANGE, POV_PKT_VQ_ENTRY = 0, 1, 2, 4
 POV_INPUT_DENSE, POV_INPUT_ENTRIES, POV_INPUT_PACKETS = 0, 1, 2
 POV_PCM_PLANAR, POV_PCM_INTERLEAVED = 0, 1
+POV_PCM_S16 = 0x100          # OR-ed into pcm_layout: the kernels store int16 PCM (see include/pov_synth.h)
 
 (POV_STAGE_FINAL_YS, POV_STAGE_STEP2_FLAG, POV_STAGE_FLOOR, POV_STAGE_FLOOR_OUTPUTS,
  POV_STAGE_AFTER_RESIDUE, POV_STAGE_AFTER_ENVELOPE, POV_STAGE_PCM_AFTER_MDCT) = range(7)
@@ -99,6 +100,11 @@ class pov_batch(C.Structure):
 class pov_decoded(C.Structure):
     _fields_ = [("channels", C.c_uint32), ("sample_rate", C.c_uint32), ("frames", C.c_uint64),
                 ("audio_packets", C.c_uint32), ("reserved", C.c_uint32), ("pcm", C.POINTER(C.c_float))]
+
+
+class pov_decoded_s16(C.Structure):
+    _fields_ = [("channels", C.c_uint32), ("sample_rate", C.c_uint32), ("frames", C.c_uint64),
+                ("audio_packets", C.c_uint32), ("reserved", C.c_uint32), ("pcm", C.POINTER(C.c_int16))]
 
 
 # numpy dtypes with the same layout as pov_stream / pov_packet (so big batches are built vectorised)

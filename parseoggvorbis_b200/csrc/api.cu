@@ -621,7 +621,8 @@ extern "C" void pov_batch_free(pov_ctx* ctx, pov_batch_handle* h) {
 extern "C" int pov_batch_upload(pov_ctx* ctx, const pov_batch* b, pov_batch_handle** out) try {
 	if(!ctx || !b || !out) return POV_ERR_ARG;
 	cudaSetDevice(ctx->device);
-	if(b->input_kind > POV_INPUT_PACKETS || b->pcm_layout > POV_PCM_INTERLEAVED) return pov_fail(ctx, POV_ERR_ARG, "pov_batch: bad input_kind/pcm_layout");
+	if(b->input_kind > POV_INPUT_PACKETS || (b->pcm_layout & ~POV_PCM_S16) > POV_PCM_INTERLEAVED) return pov_fail(ctx, POV_ERR_ARG, "pov_batch: bad input_kind/pcm_layout");
+	if(b->pcm_floats > SIZE_MAX / pcm_elem_bytes(b->pcm_layout)) return pov_fail(ctx, POV_ERR_ARG, "pov_batch: PCM arena of %llu samples does not fit the address space", (unsigned long long) b->pcm_floats);
 	if((b->n_streams && !b->streams) || (b->n_packets && !b->packets)) return pov_fail(ctx, POV_ERR_ARG, "pov_batch: null arrays");
 	if(b->input_kind == POV_INPUT_DENSE && ((uintptr_t) b->payload & 3)) return pov_fail(ctx, POV_ERR_ARG, "pov_batch: dense payload must be 4-byte aligned");
 
@@ -857,7 +858,7 @@ extern "C" int pov_batch_upload(pov_ctx* ctx, const pov_batch* b, pov_batch_hand
 		CUDA_TRY(ctx, up(h->d_runs, (uint8_t*) h->h_derived + o_runs, b_runs));
 		CUDA_TRY(ctx, cudaEventRecord(h->derived_copied, st));
 	}
-	CUDA_TRY(ctx, h->d_pcm.reserve(std::max<size_t>(sizeof(float) * b->pcm_floats, 16)));
+	CUDA_TRY(ctx, h->d_pcm.reserve(std::max<size_t>(pcm_elem_bytes(b->pcm_layout) * b->pcm_floats, 16)));
 	CUDA_TRY(ctx, h->d_status.reserve(std::max<size_t>(sizeof(uint32_t) * P, 16)));
 	CUDA_TRY(ctx, cudaMemsetAsync(h->d_status.ptr, 0, sizeof(uint32_t) * P, st));
 	if(b->input_kind != POV_INPUT_DENSE) CUDA_TRY(ctx, h->d_spectra.reserve(std::max<size_t>(sizeof(float) * dense_floats, 16)));
@@ -876,9 +877,10 @@ static DevBatchView make_view(pov_ctx* ctx, pov_batch_handle* h) {
 	else if(h->input_kind == POV_INPUT_ENTRIES) { v.spectra = (const float*) h->d_spectra.ptr; v.payload = (const uint8_t*) h->d_payload.ptr; }
 	else { v.spectra = (const float*) h->d_spectra.ptr; v.payload = (const uint8_t*) h->d_entries.ptr; }   // (what k_packet_decode writes)
 	v.inv_db = ctx->d_inv_db;
-	v.pcm = (float*) h->d_pcm.ptr;
+	v.pcm = h->d_pcm.ptr;
 	v.status = (uint32_t*) h->d_status.ptr;
-	v.n_streams = h->n_streams; v.n_packets = h->n_packets; v.pcm_layout = h->pcm_layout;
+	v.n_streams = h->n_streams; v.n_packets = h->n_packets;
+	v.pcm_layout = h->pcm_layout & ~POV_PCM_S16; v.pcm_s16 = (h->pcm_layout & POV_PCM_S16) ? 1u : 0u;
 	return v;
 }
 
@@ -1005,13 +1007,23 @@ cudaError_t pov_copy_out_async(pov_ctx* ctx, void* dst, const void* src, size_t 
 	return e;
 }
 
-extern "C" int pov_batch_fetch_pcm(pov_ctx* ctx, pov_batch_handle* h, float* out, uint64_t n_floats, int sync) try {
-	if(!ctx || !h || (!out && n_floats)) return POV_ERR_ARG;
-	if(n_floats > h->pcm_floats) return pov_fail(ctx, POV_ERR_ARG, "pov_batch_fetch_pcm: %llu floats requested, arena holds %llu", (unsigned long long) n_floats, (unsigned long long) h->pcm_floats);
+static int fetch_pcm(pov_ctx* ctx, pov_batch_handle* h, void* out, uint64_t n_values, int sync, bool s16, const char* fn) {
+	if(!ctx || !h || (!out && n_values)) return POV_ERR_ARG;
+	if(((h->pcm_layout & POV_PCM_S16) != 0) != s16)
+		return pov_fail(ctx, POV_ERR_ARG, "%s: the batch's PCM arena holds %s samples", fn, s16 ? "float32" : "int16 (POV_PCM_S16)");
+	if(n_values > h->pcm_floats) return pov_fail(ctx, POV_ERR_ARG, "%s: %llu samples requested, arena holds %llu", fn, (unsigned long long) n_values, (unsigned long long) h->pcm_floats);
 	cudaSetDevice(ctx->device);
-	if(n_floats) CUDA_TRY(ctx, pov_copy_out_async(ctx, out, h->d_pcm.ptr, n_floats * sizeof(float)));
+	if(n_values) CUDA_TRY(ctx, pov_copy_out_async(ctx, out, h->d_pcm.ptr, n_values * pcm_elem_bytes(h->pcm_layout)));
 	if(sync) CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
 	return POV_OK;
+}
+
+extern "C" int pov_batch_fetch_pcm(pov_ctx* ctx, pov_batch_handle* h, float* out, uint64_t n_floats, int sync) try {
+	return fetch_pcm(ctx, h, out, n_floats, sync, false, "pov_batch_fetch_pcm");
+} POV_NOTHROW_END(ctx)
+
+extern "C" int pov_batch_fetch_pcm_s16(pov_ctx* ctx, pov_batch_handle* h, int16_t* out, uint64_t n_values, int sync) try {
+	return fetch_pcm(ctx, h, out, n_values, sync, true, "pov_batch_fetch_pcm_s16");
 } POV_NOTHROW_END(ctx)
 
 extern "C" void* pov_batch_pcm_dev(pov_batch_handle* h) { return h ? h->d_pcm.ptr : nullptr; }

@@ -90,10 +90,13 @@ struct pov_ctx {
 	char err[512] = {0};
 };
 
+// Bytes of one PCM arena element for a pov_batch::pcm_layout value: int16 with POV_PCM_S16, float otherwise.
+inline size_t pcm_elem_bytes(uint32_t pcm_layout) { return (pcm_layout & POV_PCM_S16) ? sizeof(int16_t) : sizeof(float); }
+
 struct WarpGroup { uint32_t setup, first_run, n_runs; };   // runs of one setup: one launch of the persistent warp kernel
 
 struct pov_batch_handle {
-	uint32_t n_streams = 0, n_packets = 0, input_kind = 0, pcm_layout = 0;
+	uint32_t n_streams = 0, n_packets = 0, input_kind = 0, pcm_layout = 0;   // pcm_layout as uploaded (POV_PCM_S16 included)
 	uint64_t pcm_floats = 0, stage_floats = 0, dense_floats = 0;
 	uint32_t max_channels = 1, max_blocksize = 64, min_blocksize = 64, floor_cap = 4, res_smem = 0;
 	uint32_t floor_cap_cls[2] = {4, 4};

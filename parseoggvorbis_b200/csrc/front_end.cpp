@@ -15,6 +15,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "api_internal.h"
@@ -166,7 +167,10 @@ static int register_stream_setup_slow(pov_ctx* ctx, const StreamWork& st, uint32
 	return pov_setup_register(ctx, &a.s, id);
 }
 
-extern "C" int pov_ogg_vorbis_decode_memory(pov_ctx* ctx, const uint8_t* data, size_t len, const char* debug_out, pov_decoded* out) try {
+// Whole-file decode into a pov_decoded (T = float) or pov_decoded_s16 (T = int16_t, POV_PCM_S16 batch; never a debug dump).
+template <class T, class Out>
+static int decode_memory(pov_ctx* ctx, const uint8_t* data, size_t len, const char* debug_out, Out* out) {
+	constexpr bool kS16 = std::is_same<T, int16_t>::value;
 	if(!ctx || !out || (!data && len)) return POV_ERR_ARG;
 	memset(out, 0, sizeof *out);
 	std::vector<StreamWork> streams;
@@ -210,33 +214,47 @@ extern "C" int pov_ogg_vorbis_decode_memory(pov_ctx* ctx, const uint8_t* data, s
 	if(hb.packets.empty()) return POV_OK;
 
 	pov_batch b = hb.view();
+	if(kS16) b.pcm_layout |= POV_PCM_S16;
 	pov_batch_handle* h = nullptr;
 	int rc = pov_batch_upload(ctx, &b, &h);
 	if(rc) return rc;
 	rc = debug_out ? pov_batch_run_staged(ctx, h) : pov_batch_run(ctx, h);
-	std::vector<float> arena(hb.pcm_floats);
-	if(!rc) rc = pov_batch_fetch_pcm(ctx, h, arena.data(), arena.size(), 1);
+	std::vector<T> arena(hb.pcm_floats);
+	if(!rc) {
+		if constexpr(kS16) rc = pov_batch_fetch_pcm_s16(ctx, h, arena.data(), arena.size(), 1);
+		else rc = pov_batch_fetch_pcm(ctx, h, arena.data(), arena.size(), 1);
+	}
 	if(!rc) rc = pov_batch_status(ctx, h, nullptr, 0);
-	if(!rc && debug_out) {
-		StageHost sg;
-		rc = pov_batch_fetch_stage_all(ctx, h, sg);
-		std::string werr;
-		if(!rc && !write_debug_dump(debug_out, *use[0], *h, 0, sg, arena.data(), werr)) rc = pov_fail(ctx, POV_ERR_ARG, "debug dump: %s", werr.c_str());
+	if constexpr(!kS16) {
+		if(!rc && debug_out) {
+			StageHost sg;
+			rc = pov_batch_fetch_stage_all(ctx, h, sg);
+			std::string werr;
+			if(!rc && !write_debug_dump(debug_out, *use[0], *h, 0, sg, arena.data(), werr)) rc = pov_fail(ctx, POV_ERR_ARG, "debug dump: %s", werr.c_str());
+		}
 	}
 	pov_batch_free(ctx, h);
 	if(rc) return rc;
 	// planar [C][frames] across the (chained) streams
-	float* pcm = (float*) malloc(sizeof(float) * std::max<uint64_t>(1, frames * C));
+	T* pcm = (T*) malloc(sizeof(T) * std::max<uint64_t>(1, frames * C));
 	if(!pcm) return pov_fail(ctx, POV_ERR_ARG, "out of memory");
 	uint64_t at = 0;
 	for(size_t i = 0; i < use.size(); ++i) {
 		const pov_stream& rec = hb.streams[i];
 		for(uint32_t c = 0; c < C; ++c)
-			memcpy(pcm + (uint64_t) c * frames + at, arena.data() + rec.pcm_base + (uint64_t) c * rec.pcm_frames, sizeof(float) * rec.pcm_frames);
+			memcpy(pcm + (uint64_t) c * frames + at, arena.data() + rec.pcm_base + (uint64_t) c * rec.pcm_frames, sizeof(T) * rec.pcm_frames);
 		at += rec.pcm_frames;
 	}
 	out->pcm = pcm;
 	return POV_OK;
+}
+
+extern "C" int pov_ogg_vorbis_decode_memory(pov_ctx* ctx, const uint8_t* data, size_t len, const char* debug_out, pov_decoded* out) try {
+	return decode_memory<float>(ctx, data, len, debug_out, out);
+} POV_NOTHROW_END(ctx)
+
+extern "C" int pov_ogg_vorbis_decode_memory_s16(pov_ctx* ctx, const uint8_t* data, size_t len, pov_decoded_s16* out) try {
+	return decode_memory<int16_t>(ctx, data, len, nullptr, out);
 } POV_NOTHROW_END(ctx)
 
 extern "C" void pov_decoded_free(pov_decoded* d) {
@@ -245,10 +263,17 @@ extern "C" void pov_decoded_free(pov_decoded* d) {
 	d->pcm = nullptr;
 }
 
+extern "C" void pov_decoded_s16_free(pov_decoded_s16* d) {
+	if(!d) return;
+	free(d->pcm);
+	d->pcm = nullptr;
+}
+
 // ---------------------------------------------------------------------------------------------------------------
 // corpus decode: `host_threads` front-end workers parse files into chunks, the calling thread feeds the GPU
 // ---------------------------------------------------------------------------------------------------------------
-cudaError_t pov_checksum_launch(const float* pcm, uint64_t n, double* d_sum, cudaStream_t st, uint64_t* launches);
+// float64 sum of a float arena into *(double*) d_sum, or (s16) exact int64 sum of an int16 arena into *(uint64_t*) d_sum
+cudaError_t pov_checksum_launch(const void* pcm, bool s16, uint64_t n, void* d_sum, cudaStream_t st, uint64_t* launches);
 
 namespace {
 struct PinnedBuf { uint8_t* p = nullptr; size_t cap = 0; };
@@ -277,9 +302,9 @@ struct CorpusState {
 	struct Slot {
 		pov_ctx* ctx = nullptr;                // slot 0: the caller's context; slot 1: the sibling, so that the copies of one
 		                                       // chunk never wait for the other chunk's work
-		double* d_sum = nullptr;
+		void* d_sum = nullptr;                 // 8 bytes: float64 checksum, or the int64 sum of an int16 decode
 		pov_batch_handle* h = nullptr;
-		float* pinned = nullptr; size_t pinned_cap = 0;
+		uint8_t* pinned = nullptr; size_t pinned_cap = 0;     // the chunk's PCM arena (float or int16)
 		uint32_t* status = nullptr; size_t status_cap = 0;
 		cudaEvent_t done = nullptr;
 		cudaEvent_t t_begin = nullptr, t_kernels = nullptr, t_end = nullptr;   // POV_CORPUS_TIMING only
@@ -341,23 +366,47 @@ void corpus_state_free(void* p) { delete (CorpusState*) p; }
 inline size_t align16(size_t x) { return (x + 15) & ~(size_t) 15; }
 }  // namespace
 
+// Output format of a corpus decode: float32 (sink, checksum) or int16 (POV_PCM_S16: sink16, sum16).
+struct CorpusOut {
+	bool s16 = false;
+	pov_pcm_sink sink = nullptr;
+	pov_pcm_sink_s16 sink16 = nullptr;
+	void* user = nullptr;
+	double* checksum = nullptr;
+	int64_t* sum16 = nullptr;
+};
+
 static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* data, const size_t* len, uint32_t host_threads,
-                         pov_pcm_sink sink, void* sink_user, uint64_t* frames_out, uint64_t* total_values_out, double* checksum_out);
+                         const CorpusOut& fmt, uint64_t* frames_out, uint64_t* total_values_out);
 
 extern "C" int pov_decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* data, const size_t* len,
                                  uint32_t host_threads, uint64_t* frames_out, uint64_t* total_values_out, double* checksum_out) try {
-	return decode_corpus(ctx, n_files, data, len, host_threads, nullptr, nullptr, frames_out, total_values_out, checksum_out);
+	CorpusOut fmt;
+	fmt.checksum = checksum_out;
+	return decode_corpus(ctx, n_files, data, len, host_threads, fmt, frames_out, total_values_out);
 } POV_NOTHROW_END(ctx)
 
 extern "C" int pov_decode_corpus_pcm(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* data, const size_t* len, uint32_t host_threads,
                                      pov_pcm_sink sink, void* user, uint64_t* frames_out, uint64_t* total_values_out, double* checksum_out) try {
 	if(!sink) return pov_fail(ctx, POV_ERR_ARG, "pov_decode_corpus_pcm: null sink");
-	return decode_corpus(ctx, n_files, data, len, host_threads, sink, user, frames_out, total_values_out, checksum_out);
+	CorpusOut fmt;
+	fmt.sink = sink; fmt.user = user; fmt.checksum = checksum_out;
+	return decode_corpus(ctx, n_files, data, len, host_threads, fmt, frames_out, total_values_out);
+} POV_NOTHROW_END(ctx)
+
+extern "C" int pov_decode_corpus_s16(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* data, const size_t* len, uint32_t host_threads,
+                                     pov_pcm_sink_s16 sink, void* user, uint64_t* frames_out, uint64_t* total_values_out, int64_t* sum_out) try {
+	CorpusOut fmt;
+	fmt.s16 = true; fmt.sink16 = sink; fmt.user = user; fmt.sum16 = sum_out;
+	return decode_corpus(ctx, n_files, data, len, host_threads, fmt, frames_out, total_values_out);
 } POV_NOTHROW_END(ctx)
 
 static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* data, const size_t* len, uint32_t host_threads,
-                         pov_pcm_sink sink, void* sink_user, uint64_t* frames_out, uint64_t* total_values_out, double* checksum_out) {
+                         const CorpusOut& fmt, uint64_t* frames_out, uint64_t* total_values_out) {
 	if(!ctx || (n_files && (!data || !len))) return POV_ERR_ARG;
+	const bool has_sink = fmt.s16 ? fmt.sink16 != nullptr : fmt.sink != nullptr;
+	const uint32_t pcm_layout = POV_PCM_PLANAR | (fmt.s16 ? POV_PCM_S16 : 0u);
+	const size_t esz = pcm_elem_bytes(pcm_layout);                      // bytes per PCM sample in the arenas and over PCIe
 	cudaSetDevice(ctx->device);
 	// automatic: every core but one — the calling thread validates, queues and retires chunks and must not be time-sliced
 	// against the parsers (measured on 16 cores: 15 workers 6.8e9 samples/s and stable, 16 workers 2.6-3.7e9)
@@ -396,7 +445,7 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 			cs->slot[k].ctx = cs->sibling[k - 1];
 		}
 		for(auto& sl : cs->slot) {
-			if(cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming) != cudaSuccess || cudaMalloc(&sl.d_sum, sizeof(double)) != cudaSuccess)
+			if(cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming) != cudaSuccess || cudaMalloc(&sl.d_sum, 8) != cudaSuccess)
 				return pov_fail(ctx, POV_ERR_CUDA, "pov_decode_corpus: cudaEventCreate / cudaMalloc failed");
 		}
 		ctx->corpus = cs.release();
@@ -405,7 +454,7 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 	CorpusState& cs = *(CorpusState*) ctx->corpus;
 	cs.max_bufs = std::max(cs.max_bufs, max_ready + host_threads + CorpusState::kSlots + 1);       // queued + being filled + in flight + one spare
 	for(auto& sl : cs.slot)
-		if(cudaMemsetAsync(sl.d_sum, 0, sizeof(double), sl.ctx->stream) != cudaSuccess) return pov_fail(ctx, POV_ERR_CUDA, "pov_decode_corpus: cudaMemset failed");
+		if(cudaMemsetAsync(sl.d_sum, 0, 8, sl.ctx->stream) != cudaSuccess) return pov_fail(ctx, POV_ERR_CUDA, "pov_decode_corpus: cudaMemset failed");
 	uint64_t sibling_launches0 = 0, sibling_h2d0 = 0, sibling_d2h0 = 0;
 	for(pov_ctx* sb : cs.sibling) { sibling_launches0 += sb->launches; sibling_h2d0 += sb->h2d_bytes; sibling_d2h0 += sb->d2h_bytes; }
 
@@ -476,7 +525,7 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 					memcpy(q + o_ys, hb.ys.data(), hb.ys.size() * sizeof(uint16_t));
 					memcpy(q + o_pl, hb.payload.data(), hb.payload.size());
 					pov_batch& b = ck->view;
-					b.input_kind = hb.raw ? POV_INPUT_PACKETS : POV_INPUT_ENTRIES; b.pcm_layout = POV_PCM_PLANAR;
+					b.input_kind = hb.raw ? POV_INPUT_PACKETS : POV_INPUT_ENTRIES; b.pcm_layout = pcm_layout;
 					ck->streams = (pov_stream*) (q + o_st);
 					b.n_streams = (uint32_t) hb.streams.size(); b.streams = ck->streams;
 					b.n_packets = (uint32_t) hb.packets.size(); b.packets = (const pov_packet*) (q + o_pk);
@@ -513,6 +562,7 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 
 	uint64_t total = 0;
 	double h_sum = 0;
+	int64_t h_sum16 = 0;
 	// Two batch slots: while the GPU transforms chunk i and copies its PCM and status words to pinned host memory, the
 	// calling thread validates and queues chunk i+1. A slot is checked (status words) and reused two chunks later.
 	typedef CorpusState::Slot Slot;
@@ -544,12 +594,14 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 			}
 		// the output edge (hpp:966-973 gotPcmData, hpp:1047-1053): every logical stream of the chunk, in file order, from the
 		// calling thread; the samples stay valid during the callback only (they live in this slot's pinned buffer)
-		if(out == POV_OK && sink && !stopped && sl.in_flight && sl.n_packets) {
+		if(out == POV_OK && has_sink && !stopped && sl.in_flight && sl.n_packets) {
 			const Chunk& ck = *sl.in_flight;
 			for(uint32_t i = 0; i < ck.view.n_streams && out == POV_OK; ++i) {
 				const pov_stream& rec = ck.streams[i];
 				if(rec.pcm_frames == 0) continue;                  // hpp:1045: nothing is delivered for an empty chunk
-				if(sink(ck.stream_file[i], ck.stream_channels[i], rec.pcm_frames, sl.pinned + rec.pcm_base, sink_user) != 0)
+				const void* planar = sl.pinned + rec.pcm_base * esz;
+				if((fmt.s16 ? fmt.sink16(ck.stream_file[i], ck.stream_channels[i], rec.pcm_frames, (const int16_t*) planar, fmt.user)
+				            : fmt.sink(ck.stream_file[i], ck.stream_channels[i], rec.pcm_frames, (const float*) planar, fmt.user)) != 0)
 					out = pov_fail(ctx, POV_ERR_STREAM, "file %u: check failed: callbacks.gotPcmData(channelPcms) (hpp:1052: the sink asked to stop)", ck.stream_file[i]);
 			}
 		}
@@ -608,7 +660,7 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 		t_run += now() - t0; t0 = now();
 		if(rc && cx != ctx) pov_fail(ctx, rc, "%s", pov_last_error(cx));
 		if(!rc) {
-			const size_t need = pcm_floats * sizeof(float);
+			const size_t need = pcm_floats * esz;
 			if(need > sl.pinned_cap) {
 				if(sl.pinned) cudaFreeHost(sl.pinned);
 				sl.pinned = nullptr;
@@ -622,7 +674,7 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 				sl.status_cap = sneed + sneed / 4;
 				if(cudaMallocHost((void**) &sl.status, sl.status_cap) != cudaSuccess) { sl.status_cap = 0; rc = pov_fail(ctx, POV_ERR_CUDA, "cudaMallocHost failed"); break; }
 			}
-			cudaError_t e = pov_checksum_launch((const float*) pov_batch_pcm_dev(sl.h), pcm_floats, sl.d_sum, cx->stream, &cx->launches);
+			cudaError_t e = pov_checksum_launch(pov_batch_pcm_dev(sl.h), fmt.s16, pcm_floats, sl.d_sum, cx->stream, &cx->launches);
 			if(e != cudaSuccess) { rc = pov_fail(ctx, POV_ERR_CUDA, "checksum kernel: %s", cudaGetErrorString(e)); break; }
 			if(timing) cudaEventRecord(sl.t_kernels, cx->stream);
 			if(timeline) cudaEventRecord(tl[4 * ci + 2], cx->stream);
@@ -668,11 +720,13 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 	ready.clear();
 	for(auto& sl : cs.slot) {
 		double part = 0;
+		int64_t part16 = 0;
 		if(rc == POV_OK &&
-		   (cudaMemcpyAsync(&part, sl.d_sum, sizeof(double), cudaMemcpyDeviceToHost, sl.ctx->stream) != cudaSuccess ||
+		   (cudaMemcpyAsync(fmt.s16 ? (void*) &part16 : (void*) &part, sl.d_sum, 8, cudaMemcpyDeviceToHost, sl.ctx->stream) != cudaSuccess ||
 		    cudaStreamSynchronize(sl.ctx->stream) != cudaSuccess))
 			rc = pov_fail(ctx, POV_ERR_CUDA, "pov_decode_corpus: checksum copy failed");
 		h_sum += part;
+		h_sum16 += part16;
 		cudaStreamSynchronize(sl.ctx->stream);
 	}
 	{
@@ -683,7 +737,8 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 		ctx->d2h_bytes += b1 - sibling_d2h0;
 	}
 	if(total_values_out) *total_values_out = total;
-	if(checksum_out) *checksum_out = h_sum;
+	if(fmt.checksum) *fmt.checksum = h_sum;
+	if(fmt.sum16) *fmt.sum16 = h_sum16;
 	return rc;
 }
 

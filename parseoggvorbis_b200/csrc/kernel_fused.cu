@@ -18,6 +18,7 @@
 #include "kernels.h"
 #include "fft_core.cuh"
 #include "floor_core.cuh"
+#include "pcm_out.cuh"
 #include <stdlib.h>
 
 namespace pov {
@@ -322,8 +323,9 @@ struct OlaGeom {
 //   out = (0 + prev[n_prev/2 + j] * w_prev) + cur[j + shift] * w_cur        (hpp:1008-1017 in gather form)
 // plo = lo half of the previous frame's D, chi = hi half of the current frame's D. Inside a region the case of both
 // terms is fixed (every boundary is a multiple of 16), so all branches below are block-uniform.
+template <class TPcm>
 __device__ __forceinline__ void ola_region(const OlaGeom& G, const float* __restrict__ plo, const float* __restrict__ chi,
-                                           float* __restrict__ dst, int j0, int j1, int tid, int nthreads) {
+                                           TPcm* __restrict__ dst, int j0, int j1, int tid, int nthreads) {
 	const bool has_p = j0 < G.rbp + G.pr, p_rev = j0 < G.Hp, p_slope = j0 >= G.rbp;
 	const int ic0 = j0 + G.shift;
 	const bool has_c = ic0 >= G.lb, c_rev = ic0 >= G.H, c_slope = ic0 < G.lb + G.lc;
@@ -351,7 +353,7 @@ __device__ __forceinline__ void ola_region(const OlaGeom& G, const float* __rest
 			acc.x = __fadd_rn(acc.x, __fmul_rn(y.x, w.x)); acc.y = __fadd_rn(acc.y, __fmul_rn(y.y, w.y));
 			acc.z = __fadd_rn(acc.z, __fmul_rn(y.z, w.z)); acc.w = __fadd_rn(acc.w, __fmul_rn(y.w, w.w));
 		}
-		*reinterpret_cast<float4*>(dst + j) = acc;
+		pcm_store4(dst + j, acc);
 	}
 }
 
@@ -373,7 +375,8 @@ __device__ __forceinline__ float ola_one(const OlaGeom& G, const float* __restri
 }
 
 // kSpec = true: the batch only holds 256/2048 setups, so only those two FFT sizes are instantiated (smaller code).
-template <int kThreads, int kMinBlocks, bool kSpec>
+// TPcm: float, or int16_t for POV_PCM_S16 (converted at the store, pcm_out.cuh).
+template <int kThreads, int kMinBlocks, bool kSpec, class TPcm>
 __global__ void __launch_bounds__(kThreads, kMinBlocks) k_fused_synth(FusedParams P) {
 	extern __shared__ __align__(128) unsigned char smem[];
 	__shared__ __align__(8) uint64_t s_bar;
@@ -577,7 +580,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) k_fused_synth(FusedParam
 						for(int k = 0; k < 6; ++k) if(bnd[k] > j0 && bnd[k] < j1) j1 = bnd[k];
 						for(int c = 0; c < C; ++c)
 							ola_region(G, prev_lo + (size_t) c * G.Hp, cur_hi + (size_t) c * Q,
-							           b.pcm + chan_base + (uint64_t) c * st.pcm_frames, j0, j1, ola_tid, ola_n);
+							           reinterpret_cast<TPcm*>(b.pcm) + chan_base + (uint64_t) c * st.pcm_frames, j0, j1, ola_tid, ola_n);
 						j0 = j1;
 					}
 				} else {
@@ -588,7 +591,7 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) k_fused_synth(FusedParam
 						const float v = ola_one(G, prev_lo + (size_t) c * G.Hp, cur_hi + (size_t) c * Q, (int) j);
 						const uint64_t fidx = pc.pcm_off + j;
 						const uint64_t o = planar ? st.pcm_base + (uint64_t) c * st.pcm_frames + fidx : st.pcm_base + fidx * (uint64_t) C + c;
-						b.pcm[o] = v;
+						reinterpret_cast<TPcm*>(b.pcm)[o] = pcm_value<TPcm>(v);
 					}
 				}
 			}
@@ -642,16 +645,23 @@ size_t fused_smem_bytes(uint32_t max_channels, uint32_t max_blocksize, uint32_t 
 	return smem;
 }
 
-template <int kThreads, int kMinBlocks, bool kSpec>
+template <int kThreads, int kMinBlocks, bool kSpec, class TPcm>
 static cudaError_t launch_variant(const FusedParams& P, uint32_t n_runs, size_t smem, cudaStream_t st) {
-	cudaError_t e = cudaFuncSetAttribute(k_fused_synth<kThreads, kMinBlocks, kSpec>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
+	cudaError_t e = cudaFuncSetAttribute(k_fused_synth<kThreads, kMinBlocks, kSpec, TPcm>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
 	if(e != cudaSuccess) return e;
 	// The twiddle / rotation / window tables (~15 KB for 256/2048) are read through L1 by every CTA: leave L1 enough
 	// room for them instead of maximising resident CTAs (tuning knob: POV_SMEM_CARVEOUT = percent of the 228 KB).
 	static const int carve = [] { const char* e = getenv("POV_SMEM_CARVEOUT"); return e ? atoi(e) : 100; }();
-	cudaFuncSetAttribute(k_fused_synth<kThreads, kMinBlocks, kSpec>, cudaFuncAttributePreferredSharedMemoryCarveout, carve);
-	k_fused_synth<kThreads, kMinBlocks, kSpec><<<n_runs, kThreads, smem, st>>>(P);
+	cudaFuncSetAttribute(k_fused_synth<kThreads, kMinBlocks, kSpec, TPcm>, cudaFuncAttributePreferredSharedMemoryCarveout, carve);
+	k_fused_synth<kThreads, kMinBlocks, kSpec, TPcm><<<n_runs, kThreads, smem, st>>>(P);
 	return cudaGetLastError();
+}
+
+template <class TPcm>
+static cudaError_t launch_fused_as(const FusedParams& P, uint32_t threads, bool only_256_2048, uint32_t n_runs, size_t smem, cudaStream_t st) {
+	if(threads == 128) return only_256_2048 ? launch_variant<128, 5, true, TPcm>(P, n_runs, smem, st) : launch_variant<128, 5, false, TPcm>(P, n_runs, smem, st);
+	if(threads == 256) return only_256_2048 ? launch_variant<256, 2, true, TPcm>(P, n_runs, smem, st) : launch_variant<256, 2, false, TPcm>(P, n_runs, smem, st);
+	return launch_variant<512, 1, false, TPcm>(P, n_runs, smem, st);
 }
 
 cudaError_t launch_fused(const DevBatchView& b, const DevRun* runs, uint32_t n_runs, uint32_t max_channels,
@@ -665,10 +675,8 @@ cudaError_t launch_fused(const DevBatchView& b, const DevRun* runs, uint32_t n_r
 	P.b = b;
 	P.runs = runs;
 	if(smem > 227 * 1024) return cudaErrorInvalidConfiguration;
-	cudaError_t e;
-	if(threads == 128) e = only_256_2048 ? launch_variant<128, 5, true>(P, n_runs, smem, st) : launch_variant<128, 5, false>(P, n_runs, smem, st);
-	else if(threads == 256) e = only_256_2048 ? launch_variant<256, 2, true>(P, n_runs, smem, st) : launch_variant<256, 2, false>(P, n_runs, smem, st);
-	else e = launch_variant<512, 1, false>(P, n_runs, smem, st);
+	const cudaError_t e = b.pcm_s16 ? launch_fused_as<int16_t>(P, threads, only_256_2048, n_runs, smem, st)
+	                                : launch_fused_as<float>(P, threads, only_256_2048, n_runs, smem, st);
 	if(launches) ++*launches;
 	return e;
 }

@@ -25,6 +25,7 @@
 // packet per run).
 #include "kernels.h"
 #include "fft_core.cuh"
+#include "pcm_out.cuh"
 #include <stdlib.h>
 #include <algorithm>
 #include <type_traits>
@@ -934,9 +935,9 @@ __device__ __forceinline__ float ola_one(const OlaGeom& G, const float* __restri
 // out[j..j+3] and out[1020-j..1023-j] (j < 512) from the same four vectors (TDAC symmetry of both frames and windows).
 // kTm = 1: window slopes from tensor memory. kTm = 2: also the D halves in the storage order of fft512_tm — lane L reads
 // storage quad 32 i + L (and its mirror 127 - that), which holds the true quad tq = [sq6][sq1][sq0][sq5][sq2][sq4][sq3].
-template <int Q, bool kStrided, int kTm>
+template <int Q, bool kStrided, int kTm, class TPcm>
 __device__ __forceinline__ void ola_long_long(const float* __restrict__ plo, const float* __restrict__ chi, const float* __restrict__ sl,
-                                              float* __restrict__ dst, int stride, int lane, uint32_t tm, float* __restrict__ stage = nullptr) {
+                                              TPcm* __restrict__ dst, int stride, int lane, uint32_t tm, float* __restrict__ stage = nullptr) {
 	// n = 4Q: the chunk has 2Q samples, half of them (Q) below the centre; 8 samples per lane and iteration
 #pragma unroll kOlaUnroll
 	for(int i = 0; i < Q / 128; ++i) {
@@ -964,30 +965,30 @@ __device__ __forceinline__ void ola_long_long(const float* __restrict__ plo, con
 		o2.z = __fadd_rn(__fmul_rn(-p.z, wa.y), __fmul_rn(-c.y, wb.z));
 		o2.w = __fadd_rn(__fmul_rn(-p.w, wa.x), __fmul_rn(-c.x, wb.w));
 		if constexpr(!kStrided) {
-			__stcs(reinterpret_cast<float4*>(dst + j), o1);
-			__stcs(reinterpret_cast<float4*>(dst + (2 * Q - 4) - j), o2);
+			pcm_store4_cs(dst + j, o1);
+			pcm_store4_cs(dst + (2 * Q - 4) - j, o2);
 		} else {
 			// interleaved PCM: sample j of this channel lives at dst[j * channels]. The lane's four samples would be four stores
 			// 16 * channels bytes apart from the next lane's; through a 512-byte stage (the step's curve block, dead by now) every
 			// store instruction covers 32 consecutive frames instead, i.e. a quarter of the sectors.
 			if constexpr(kTm == 2) {          // (fft512_tm's storage order: lanes are not frame-consecutive; plain strided stores)
-				float* a = dst + (size_t) j * stride;
-				float* b = dst + (size_t) ((2 * Q - 4) - j) * stride;
-				a[0] = o1.x; a[stride] = o1.y; a[2 * stride] = o1.z; a[3 * stride] = o1.w;
-				b[0] = o2.x; b[stride] = o2.y; b[2 * stride] = o2.z; b[3 * stride] = o2.w;
+				TPcm* a = dst + (size_t) j * stride;
+				TPcm* b = dst + (size_t) ((2 * Q - 4) - j) * stride;
+				a[0] = pcm_value<TPcm>(o1.x); a[stride] = pcm_value<TPcm>(o1.y); a[2 * stride] = pcm_value<TPcm>(o1.z); a[3 * stride] = pcm_value<TPcm>(o1.w);
+				b[0] = pcm_value<TPcm>(o2.x); b[stride] = pcm_value<TPcm>(o2.y); b[2 * stride] = pcm_value<TPcm>(o2.z); b[3 * stride] = pcm_value<TPcm>(o2.w);
 				continue;
 			}
 			*reinterpret_cast<float4*>(stage + 4 * lane) = o1;
 			__syncwarp();
-			float* a = dst + (size_t) (128 * i + lane) * stride;
+			TPcm* a = dst + (size_t) (128 * i + lane) * stride;
 #pragma unroll
-			for(int k = 0; k < 4; ++k) a[(size_t) (32 * k) * stride] = stage[32 * k + lane];
+			for(int k = 0; k < 4; ++k) a[(size_t) (32 * k) * stride] = pcm_value<TPcm>(stage[32 * k + lane]);
 			__syncwarp();
 			*reinterpret_cast<float4*>(stage + 124 - 4 * lane) = o2;
 			__syncwarp();
-			float* b = dst + (size_t) ((2 * Q - 128) - 128 * i + lane) * stride;
+			TPcm* b = dst + (size_t) ((2 * Q - 128) - 128 * i + lane) * stride;
 #pragma unroll
-			for(int k = 0; k < 4; ++k) b[(size_t) (32 * k) * stride] = stage[32 * k + lane];
+			for(int k = 0; k < 4; ++k) b[(size_t) (32 * k) * stride] = pcm_value<TPcm>(stage[32 * k + lane]);
 			__syncwarp();
 		}
 	}
@@ -1008,7 +1009,9 @@ __device__ __forceinline__ int curve_mode(const FastTables* tb, uint32_t mapping
 
 // kWide: a floor of 33..64 posts is reachable (compile time, so that the common case keeps its constants: 32 records per long
 // curve, 36-byte Y records, 32-bit step-2 masks); instantiated with the generic coupling class only.
-template <int Q0, int Q1, bool kPlanar, int kMaxNL, bool kWide>
+// TPcm: float, or int16_t for POV_PCM_S16 (converted at the store, pcm_out.cuh). A template parameter like kPlanar: a run-time
+// flag of comparable weight (the 64-post floors) measured 6.5 % slower (DESIGN.md §3).
+template <int Q0, int Q1, bool kPlanar, class TPcm, int kMaxNL, bool kWide>
 __global__ void __launch_bounds__(kThreads, 1) k_warp_synth(const Params P) {
 	using M = Map<Q0, Q1>;
 	constexpr int N0 = 4 * Q0, N1 = 4 * Q1;              // block sizes
@@ -1135,11 +1138,11 @@ __global__ void __launch_bounds__(kThreads, 1) k_warp_synth(const Params P) {
 		const float* spec_base = b.spectra + spec0;
 		// where this run's first chunk starts in the PCM arena, for this channel (one pointer instead of the stream record):
 		//   planar:      pcm_base + ch * pcm_frames + frame,  + 1 per frame;   interleaved: pcm_base + frame * C + ch,  + C per frame
-		float* out0;
+		TPcm* out0;
 		bool first_of_stream;                   // the run starts at its stream's first packet, which only primes the overlap (hpp:1021)
 		{
 			const pov_stream st = b.streams[pk0->stream];
-			out0 = b.pcm + (planar ? st.pcm_base + (uint64_t) ch * st.pcm_frames + pcm0 : st.pcm_base + pcm0 * (uint64_t) C + (uint64_t) ch);
+			out0 = reinterpret_cast<TPcm*>(b.pcm) + (planar ? st.pcm_base + (uint64_t) ch * st.pcm_frames + pcm0 : st.pcm_base + pcm0 * (uint64_t) C + (uint64_t) ch);
 			first_of_stream = run.first_packet == st.first_packet;
 		}
 		__syncwarp();
@@ -1279,8 +1282,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_warp_synth(const Params P) {
 #else
 				if(emits) {
 #endif
-					float* const dst = out0 + (planar ? (size_t) w.pcm_rel : (size_t) w.pcm_rel * (size_t) C);
-					if(flag && prev_n == N1 && lc == N1 / 2 && prev_right == N1 / 2 && emit == (uint32_t) (N1 / 2) && (!planar || ((size_t) dst & 15) == 0)) {
+					TPcm* const dst = out0 + (planar ? (size_t) w.pcm_rel : (size_t) w.pcm_rel * (size_t) C);
+					if(flag && prev_n == N1 && lc == N1 / 2 && prev_right == N1 / 2 && emit == (uint32_t) (N1 / 2) && (!planar || ((size_t) dst & (4 * sizeof(TPcm) - 1)) == 0)) {
 						if constexpr(planar) ola_long_long<Q1, false, kTm>(prev_lo, cur_hi, s_slope1, dst, 1, lane, tmw);
 						else ola_long_long<Q1, true, kTm>(prev_lo, cur_hi, s_slope1, dst, C, lane, tmw, reinterpret_cast<float*>(curves));
 					} else {
@@ -1294,7 +1297,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_warp_synth(const Params P) {
 						G.pperm = (kTm == 2) && prev_perm; G.cperm = (kTm == 2) && flag && !kLongGrouped;     // (compile-time false unless kTm == 2)
 						for(uint32_t j = (uint32_t) lane; j < emit; j += 32u) {
 							const float v = ola_one(G, prev_lo, cur_hi, (int) j);
-							dst[planar ? (size_t) j : (size_t) j * (size_t) C] = v;
+							dst[planar ? (size_t) j : (size_t) j * (size_t) C] = pcm_value<TPcm>(v);
 						}
 					}
 				}
@@ -1378,26 +1381,31 @@ size_t warp_kernel_smem_bytes(uint32_t bs0, uint32_t bs1, uint32_t short_posts_c
 uint32_t warp_kernel_max_run(bool wide) { return wide ? (uint32_t) (wk::kPktCap * wk::kFsStride / 72) - 1u : (uint32_t) wk::kPktCap - 1u; }
 uint32_t warp_kernel_warps(void) { return (uint32_t) wk::kWarps; }
 
-template <int Q0, int Q1, bool kPlanar, int kMaxNL, bool kWide = false>
+template <int Q0, int Q1, bool kPlanar, class TPcm, int kMaxNL, bool kWide = false>
 static cudaError_t launch_one(const wk::Params& P, uint32_t grid, size_t smem, cudaStream_t st) {
-	cudaError_t e = cudaFuncSetAttribute(wk::k_warp_synth<Q0, Q1, kPlanar, kMaxNL, kWide>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
+	cudaError_t e = cudaFuncSetAttribute(wk::k_warp_synth<Q0, Q1, kPlanar, TPcm, kMaxNL, kWide>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
 	if(e != cudaSuccess) return e;
-	wk::k_warp_synth<Q0, Q1, kPlanar, kMaxNL, kWide><<<grid, wk::kThreads, smem, st>>>(P);
+	wk::k_warp_synth<Q0, Q1, kPlanar, TPcm, kMaxNL, kWide><<<grid, wk::kThreads, smem, st>>>(P);
 	return cudaGetLastError();
+}
+
+template <int Q0, int Q1, class TPcm>
+static cudaError_t launch_geom(const wk::Params& P, uint32_t max_nl, bool wide, uint32_t grid, size_t smem, cudaStream_t st) {
+	if(wide) return P.b.pcm_layout == POV_PCM_PLANAR ? launch_one<Q0, Q1, true, TPcm, 4, true>(P, grid, smem, st) : launch_one<Q0, Q1, false, TPcm, 4, true>(P, grid, smem, st);
+	const int cls = max_nl <= 1 ? 1 : max_nl == 2 ? 2 : 4;
+	if(P.b.pcm_layout == POV_PCM_PLANAR) {
+		if(cls == 1) return launch_one<Q0, Q1, true, TPcm, 1>(P, grid, smem, st);
+		if(cls == 2) return launch_one<Q0, Q1, true, TPcm, 2>(P, grid, smem, st);
+		return launch_one<Q0, Q1, true, TPcm, 4>(P, grid, smem, st);
+	}
+	if(cls == 1) return launch_one<Q0, Q1, false, TPcm, 1>(P, grid, smem, st);
+	if(cls == 2) return launch_one<Q0, Q1, false, TPcm, 2>(P, grid, smem, st);
+	return launch_one<Q0, Q1, false, TPcm, 4>(P, grid, smem, st);
 }
 
 template <int Q0, int Q1>
 static cudaError_t launch_geom(const wk::Params& P, uint32_t max_nl, bool wide, uint32_t grid, size_t smem, cudaStream_t st) {
-	if(wide) return P.b.pcm_layout == POV_PCM_PLANAR ? launch_one<Q0, Q1, true, 4, true>(P, grid, smem, st) : launch_one<Q0, Q1, false, 4, true>(P, grid, smem, st);
-	const int cls = max_nl <= 1 ? 1 : max_nl == 2 ? 2 : 4;
-	if(P.b.pcm_layout == POV_PCM_PLANAR) {
-		if(cls == 1) return launch_one<Q0, Q1, true, 1>(P, grid, smem, st);
-		if(cls == 2) return launch_one<Q0, Q1, true, 2>(P, grid, smem, st);
-		return launch_one<Q0, Q1, true, 4>(P, grid, smem, st);
-	}
-	if(cls == 1) return launch_one<Q0, Q1, false, 1>(P, grid, smem, st);
-	if(cls == 2) return launch_one<Q0, Q1, false, 2>(P, grid, smem, st);
-	return launch_one<Q0, Q1, false, 4>(P, grid, smem, st);
+	return P.b.pcm_s16 ? launch_geom<Q0, Q1, int16_t>(P, max_nl, wide, grid, smem, st) : launch_geom<Q0, Q1, float>(P, max_nl, wide, grid, smem, st);
 }
 
 cudaError_t launch_warp(const DevBatchView& b, const DevRun* runs, uint32_t n_runs, uint32_t channels, const FastTables* d_tabs,

@@ -16,9 +16,10 @@ struct DevBatchView {
 	const uint64_t*   spec_off;      // per packet: float offset of its [C][n/2] block inside `spectra`
 	const uint8_t*    payload;       // residue payload arena (POV_INPUT_ENTRIES) or nullptr
 	const float*      inv_db;        // floor1_inverse_dB_table[256] (src/inverse_db_table.h:13-78), device copy
-	float*            pcm;
+	void*             pcm;           // PCM arena: float, or int16_t when pcm_s16
 	uint32_t*         status;        // [n_packets]
-	uint32_t n_streams, n_packets, pcm_layout;
+	uint32_t n_streams, n_packets, pcm_layout;   // pcm_layout: POV_PCM_PLANAR | POV_PCM_INTERLEAVED (without POV_PCM_S16)
+	uint32_t pcm_s16;                // the kernels store PCM as int16 (pcm_out.cuh: pcm_s16)
 };
 
 // Staged (debug) path: every intermediate is materialised.

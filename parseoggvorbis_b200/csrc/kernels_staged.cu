@@ -11,6 +11,7 @@
 #include "kernels.h"
 #include "fft_core.cuh"
 #include "floor_core.cuh"
+#include "pcm_out.cuh"
 
 namespace pov {
 
@@ -328,6 +329,7 @@ __device__ __forceinline__ void slope_lengths(const DevSetup& su, const pov_pack
 	right = (int) ((flag && (pk.window_flags & 2)) ? su.blocksize[1] : su.blocksize[0]) / 2;
 }
 
+template <class TPcm>
 __global__ void __launch_bounds__(256) k_ola_staged(DevBatchView b, DevStageBuffers sb, uint32_t max_channels) {
 	const uint32_t p = blockIdx.x / max_channels, c = blockIdx.x % max_channels;
 	const pov_packet pk = b.packets[p];
@@ -355,7 +357,7 @@ __global__ void __launch_bounds__(256) k_ola_staged(DevBatchView b, DevStageBuff
 		const uint64_t f = pk.pcm_off + j;
 		const uint64_t o = (b.pcm_layout == POV_PCM_PLANAR) ? st.pcm_base + (uint64_t) c * st.pcm_frames + f
 		                                                    : st.pcm_base + f * su.channels + c;
-		b.pcm[o] = acc;
+		reinterpret_cast<TPcm*>(b.pcm)[o] = pcm_value<TPcm>(acc);
 	}
 }
 
@@ -373,6 +375,21 @@ __global__ void __launch_bounds__(256) k_checksum(const float* __restrict__ pcm,
 		double t = 0;
 		for(int i = 0; i < 8; ++i) t += part[i];
 		atomicAdd(sum, t);
+	}
+}
+
+// exact integer sum of an int16 PCM arena (POV_PCM_S16): two's-complement accumulation in 64 bits, independent of the order
+__global__ void __launch_bounds__(256) k_checksum_s16(const int16_t* __restrict__ pcm, uint64_t n, unsigned long long* __restrict__ sum) {
+	long long acc = 0;
+	for(uint64_t i = (uint64_t) blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t) gridDim.x * blockDim.x) acc += pcm[i];
+	for(int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+	__shared__ long long part[8];
+	if((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = acc;
+	__syncthreads();
+	if(threadIdx.x == 0) {
+		long long t = 0;
+		for(int i = 0; i < 8; ++i) t += part[i];
+		atomicAdd(sum, (unsigned long long) t);
 	}
 }
 
@@ -400,7 +417,8 @@ cudaError_t launch_staged(const DevBatchView& b, const DevStageBuffers& sb, uint
 	k_couple_dot<<<b.n_packets, 256, 0, st>>>(b, sb);
 	const size_t smem = kImdctSmemFloat2 * sizeof(float2) + kImdctSmemD * sizeof(float);
 	k_imdct_staged<<<(unsigned) cps, kImdctThreads, smem, st>>>(b, sb, max_channels);
-	k_ola_staged<<<(unsigned) cps, 256, 0, st>>>(b, sb, max_channels);
+	if(b.pcm_s16) k_ola_staged<int16_t><<<(unsigned) cps, 256, 0, st>>>(b, sb, max_channels);
+	else k_ola_staged<float><<<(unsigned) cps, 256, 0, st>>>(b, sb, max_channels);
 	if(launches) *launches += 4;
 	return cudaGetLastError();
 }
@@ -466,10 +484,11 @@ cudaError_t launch_mdct_backward(const DevSetup*, uint32_t n, uint64_t count, co
 
 }  // namespace pov
 
-cudaError_t pov_checksum_launch(const float* pcm, uint64_t n, double* d_sum, cudaStream_t st, uint64_t* launches) {
+cudaError_t pov_checksum_launch(const void* pcm, bool s16, uint64_t n, void* d_sum, cudaStream_t st, uint64_t* launches) {
 	if(n == 0) return cudaSuccess;
 	const unsigned blocks = (unsigned) ((n + 256ull * 16 - 1) / (256ull * 16) > 1184 ? 1184 : (n + 256ull * 16 - 1) / (256ull * 16));
-	pov::k_checksum<<<blocks ? blocks : 1, 256, 0, st>>>(pcm, n, d_sum);
+	if(s16) pov::k_checksum_s16<<<blocks ? blocks : 1, 256, 0, st>>>((const int16_t*) pcm, n, (unsigned long long*) d_sum);
+	else pov::k_checksum<<<blocks ? blocks : 1, 256, 0, st>>>((const float*) pcm, n, (double*) d_sum);
 	if(launches) ++*launches;
 	return cudaGetLastError();
 }

@@ -21,14 +21,16 @@ _LIB: Optional[C.CDLL] = None
 SYMBOLS = [
     "pov_abi_version", "pov_inverse_db_table", "pov_window", "pov_ctx_create", "pov_ctx_destroy", "pov_last_error", "pov_ctx_stream",
     "pov_ctx_launch_count", "pov_ctx_io_bytes", "pov_ctx_set_device_entropy", "pov_ctx_set_page_spanning", "pov_ogg_parse_memory_ex", "pov_setup_register", "pov_setup_entry_bits", "pov_setup_get_window",
-    "pov_batch_upload", "pov_batch_run", "pov_batch_kernel_name", "pov_batch_run_staged", "pov_batch_fetch_pcm", "pov_batch_pcm_dev",
+    "pov_batch_upload", "pov_batch_run", "pov_batch_kernel_name", "pov_batch_run_staged", "pov_batch_fetch_pcm", "pov_batch_fetch_pcm_s16", "pov_batch_pcm_dev",
     "pov_batch_fetch_stage", "pov_batch_status", "pov_batch_sync", "pov_batch_free", "pov_batch_features", "pov_batch_fetch_fast_floor", "pov_mdct_backward_batch",
     "pov_ogg_vorbis_decode_memory", "pov_decoded_free", "pov_decode_corpus", "pov_decode_corpus_pcm", "pov_ogg_vorbis_full_read_from_memory",
+    "pov_ogg_vorbis_decode_memory_s16", "pov_decoded_s16_free", "pov_decode_corpus_s16",
     "pov_ogg_parse_memory", "pov_parsed_stream_count", "pov_parsed_get", "pov_parsed_free",
 ]
 
 
 SINK_FN = C.CFUNCTYPE(C.c_int, C.c_uint32, C.c_uint32, C.c_uint64, C.POINTER(C.c_float), C.c_void_p)
+SINK_S16_FN = C.CFUNCTYPE(C.c_int, C.c_uint32, C.c_uint32, C.c_uint64, C.POINTER(C.c_int16), C.c_void_p)
 
 
 class PovError(RuntimeError):
@@ -74,6 +76,7 @@ def load() -> C.CDLL:
     L.pov_batch_kernel_name.argtypes = [vp, vp]
     L.pov_batch_kernel_name.restype = C.c_char_p
     L.pov_batch_fetch_pcm.argtypes = [vp, vp, C.POINTER(C.c_float), u64, i32]
+    L.pov_batch_fetch_pcm_s16.argtypes = [vp, vp, C.POINTER(C.c_int16), u64, i32]
     L.pov_batch_pcm_dev.argtypes = [vp]
     L.pov_batch_pcm_dev.restype = vp
     L.pov_batch_fetch_stage.argtypes = [vp, vp, u32, u32, i32, vp, u64]
@@ -87,10 +90,15 @@ def load() -> C.CDLL:
     L.pov_ogg_vorbis_decode_memory.argtypes = [vp, C.c_char_p, C.c_size_t, C.c_char_p, C.POINTER(abi.pov_decoded)]
     L.pov_decoded_free.argtypes = [C.POINTER(abi.pov_decoded)]
     L.pov_decoded_free.restype = None
+    L.pov_ogg_vorbis_decode_memory_s16.argtypes = [vp, C.c_char_p, C.c_size_t, C.POINTER(abi.pov_decoded_s16)]
+    L.pov_decoded_s16_free.argtypes = [C.POINTER(abi.pov_decoded_s16)]
+    L.pov_decoded_s16_free.restype = None
     L.pov_decode_corpus.argtypes = [vp, u32, C.POINTER(C.c_char_p), C.POINTER(C.c_size_t), u32,
                                     C.POINTER(u64), C.POINTER(u64), C.POINTER(C.c_double)]
     L.pov_decode_corpus_pcm.argtypes = [vp, u32, C.POINTER(C.c_char_p), C.POINTER(C.c_size_t), u32, SINK_FN, vp,
                                         C.POINTER(u64), C.POINTER(u64), C.POINTER(C.c_double)]
+    L.pov_decode_corpus_s16.argtypes = [vp, u32, C.POINTER(C.c_char_p), C.POINTER(C.c_size_t), u32, SINK_S16_FN, vp,
+                                        C.POINTER(u64), C.POINTER(u64), C.POINTER(C.c_int64)]
     L.pov_ogg_vorbis_full_read_from_memory.argtypes = [C.c_char_p, C.c_size_t, C.POINTER(C.c_char_p)]
     L.pov_ogg_parse_memory.argtypes = [C.c_char_p, C.c_size_t, C.POINTER(vp), C.POINTER(C.c_char_p)]
     L.pov_ogg_parse_memory_ex.argtypes = [C.c_char_p, C.c_size_t, u32, C.POINTER(vp), C.POINTER(C.c_char_p)]
@@ -244,10 +252,21 @@ class SynthContext:
         self._check(self.L.pov_batch_sync(self.ctx, bh.h))
 
     def fetch_pcm(self, bh: BatchHandle, out: Optional[np.ndarray] = None, sync: bool = True) -> np.ndarray:
+        """The batch's PCM arena: float32, or int16 for a batch uploaded with pcm_layout | POV_PCM_S16."""
         n = int(bh.batch.pcm_floats)
+        if bh.batch.pcm_layout & abi.POV_PCM_S16:
+            return self.fetch_pcm_s16(bh, out, sync)
         if out is None:
             out = np.empty(n, np.float32)
         self._check(self.L.pov_batch_fetch_pcm(self.ctx, bh.h, out.ctypes.data_as(C.POINTER(C.c_float)), n, int(sync)))
+        return out
+
+    def fetch_pcm_s16(self, bh: BatchHandle, out: Optional[np.ndarray] = None, sync: bool = True) -> np.ndarray:
+        """pov_batch_fetch_pcm_s16: the int16 arena of a POV_PCM_S16 batch (PovError on a float32 batch)."""
+        n = int(bh.batch.pcm_floats)
+        if out is None:
+            out = np.empty(n, np.int16)
+        self._check(self.L.pov_batch_fetch_pcm_s16(self.ctx, bh.h, out.ctypes.data_as(C.POINTER(C.c_int16)), n, int(sync)))
         return out
 
     def pcm_dev_ptr(self, bh: BatchHandle) -> int:
@@ -279,18 +298,25 @@ class SynthContext:
                                                    out.ctypes.data_as(C.POINTER(C.c_float))))
         return out
 
-    def decode_ogg(self, data: bytes, debug_out: Optional[str] = None):
-        """Whole-file decode through the host front-end + GPU. Returns (pcm [C, frames], sample_rate, n_packets)."""
-        d = abi.pov_decoded()
-        dbg = debug_out.encode() if debug_out else None
-        self._check(self.L.pov_ogg_vorbis_decode_memory(self.ctx, data, len(data), dbg, C.byref(d)))
+    def decode_ogg(self, data: bytes, debug_out: Optional[str] = None, s16: bool = False):
+        """Whole-file decode through the host front-end + GPU. Returns (pcm [C, frames], sample_rate, n_packets).
+        s16: int16 PCM converted on the device (pov_ogg_vorbis_decode_memory_s16; no debug dump)."""
+        if s16:
+            if debug_out:
+                raise ValueError("the debug dump is float32: decode_ogg(s16=True) takes no debug_out")
+            d, dtype, free = abi.pov_decoded_s16(), np.int16, self.L.pov_decoded_s16_free
+            self._check(self.L.pov_ogg_vorbis_decode_memory_s16(self.ctx, data, len(data), C.byref(d)))
+        else:
+            d, dtype, free = abi.pov_decoded(), np.float32, self.L.pov_decoded_free
+            dbg = debug_out.encode() if debug_out else None
+            self._check(self.L.pov_ogg_vorbis_decode_memory(self.ctx, data, len(data), dbg, C.byref(d)))
         try:
             n = int(d.channels) * int(d.frames)
             pcm = np.ctypeslib.as_array(d.pcm, shape=(n,)).copy().reshape(int(d.channels), int(d.frames)) if n else \
-                np.zeros((int(d.channels), 0), np.float32)
+                np.zeros((int(d.channels), 0), dtype)
             return pcm, int(d.sample_rate), int(d.audio_packets)
         finally:
-            self.L.pov_decoded_free(C.byref(d))
+            free(C.byref(d))
 
     FEATURE_KINDS = {"floor_final_ys": 0, "floor_final_ys_rendered": 1, "residue_ys": 2, "residue_ys_with_floor": 3}
 
@@ -322,8 +348,11 @@ class SynthContext:
         finally:
             po.close()
 
-    def decode_corpus(self, files, host_threads: int = 0):
-        """files: list of bytes. Returns (frames per file, total PCM values, checksum)."""
+    def decode_corpus(self, files, host_threads: int = 0, s16: bool = False):
+        """files: list of bytes. Returns (frames per file, total PCM values, checksum). s16: int16 PCM (pov_decode_corpus_s16,
+        half the device -> host bytes); the checksum is then the exact integer sum of every sample."""
+        if s16:
+            return self._decode_corpus_s16(files, None, host_threads)
         n = len(files)
         arr = (C.c_char_p * n)(*files)
         lens = (C.c_size_t * n)(*[len(f) for f in files])
@@ -334,10 +363,13 @@ class SynthContext:
                                              frames.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(total), C.byref(chk)))
         return frames, int(total.value), float(chk.value)
 
-    def decode_corpus_pcm(self, files, sink, host_threads: int = 0):
+    def decode_corpus_pcm(self, files, sink, host_threads: int = 0, s16: bool = False):
         """The corpus decode with its output edge (pov_decode_corpus_pcm): `sink(file_index, pcm)` is called from this thread
         for every logical stream, in file order, with a (channels, frames) float32 array that is only valid during the call;
-        a true return value stops the decode (PovError, like the reference's CHECK(callbacks.gotPcmData(...)))."""
+        a true return value stops the decode (PovError, like the reference's CHECK(callbacks.gotPcmData(...))).
+        s16: the arrays are int16 (pov_decode_corpus_s16) and the returned checksum is the exact integer sum."""
+        if s16:
+            return self._decode_corpus_s16(files, sink, host_threads)
         n = len(files)
         arr = (C.c_char_p * n)(*files)
         lens = (C.c_size_t * n)(*[len(f) for f in files])
@@ -352,3 +384,20 @@ class SynthContext:
         self._check(self.L.pov_decode_corpus_pcm(self.ctx, n, arr, lens, host_threads, _sink, None,
                                                  frames.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(total), C.byref(chk)))
         return frames, int(total.value), float(chk.value)
+
+    def _decode_corpus_s16(self, files, sink, host_threads: int):
+        n = len(files)
+        arr = (C.c_char_p * n)(*files)
+        lens = (C.c_size_t * n)(*[len(f) for f in files])
+        frames = np.zeros(n, np.uint64)
+        total = C.c_uint64(0)
+        chk = C.c_int64(0)
+        _sink = C.cast(None, SINK_S16_FN)
+        if sink is not None:
+            @SINK_S16_FN
+            def _sink(file_index, channels, nframes, planar, user):
+                pcm = np.ctypeslib.as_array(planar, shape=(int(channels), int(nframes)))
+                return 1 if sink(int(file_index), pcm) else 0
+        self._check(self.L.pov_decode_corpus_s16(self.ctx, n, arr, lens, host_threads, _sink, None,
+                                                 frames.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(total), C.byref(chk)))
+        return frames, int(total.value), int(chk.value)
