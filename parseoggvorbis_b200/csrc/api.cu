@@ -358,7 +358,6 @@ extern "C" int pov_setup_register(pov_ctx* ctx, const pov_setup* s, uint32_t* id
 	rec.max_posts = max_posts;
 	// residues
 	std::vector<DevResidue> residues(s->n_residues);
-	uint32_t max_res_smem = 0;
 	for(uint32_t i = 0; i < s->n_residues; ++i) {
 		const pov_residue& r = s->residues[i];
 		if(r.type > 2) return pov_fail(ctx, POV_ERR_ARG, "pov_setup: residue %u type %u (hpp:634)", i, r.type);
@@ -375,11 +374,7 @@ extern "C" int pov_setup_register(pov_ctx* ctx, const pov_setup* s, uint32_t* id
 			const uint32_t dim = s->codebooks[bk].dim;
 			if(r.partition_size % dim) return pov_fail(ctx, POV_ERR_UNSUPPORTED, "pov_setup: residue %u: codebook %u dim %u does not divide partition size %u", i, bk, dim, r.partition_size);
 		}
-		const uint32_t vlen = s->channels * (s->blocksize[1] / 2);
-		const uint32_t parts = vlen / r.partition_size + 1;
-		max_res_smem = std::max<uint32_t>(max_res_smem, vlen * 4 + 8 * parts * s->channels * 4 + 64);
 	}
-	rec.res_smem = max_res_smem;
 	// mappings
 	std::vector<DevMapping> maps(s->n_mappings);
 	for(uint32_t i = 0; i < s->n_mappings; ++i) {
@@ -415,6 +410,27 @@ extern "C" int pov_setup_register(pov_ctx* ctx, const pov_setup* s, uint32_t* id
 		const int cls = s->modes[i].blockflag ? 1 : 0;
 		for(uint32_t k = 0; k < m.n_submaps; ++k)
 			rec.posts_cls[cls] = std::max<uint32_t>(rec.posts_cls[cls], floors[m.submap_floor[k]].n_posts);
+	}
+	// k_residue_apply's need, from the submaps each mode decodes: the working vector of one submap (nch * n/2 floats, for
+	// every residue type) and its 8 * partitions * vectors read cursors
+	if(s->n_residues) {
+		uint64_t acc_max = 0, cur_max = 0, both_max = 0;
+		for(uint32_t mo = 0; mo < s->n_modes; ++mo) {
+			const DevMapping& mp = maps[s->modes[mo].mapping];
+			const uint32_t half = s->blocksize[s->modes[mo].blockflag ? 1 : 0] / 2;
+			for(uint32_t sm = 0; sm < mp.n_submaps; ++sm) {
+				uint32_t nch = 0;
+				for(uint32_t c = 0; c < s->channels; ++c) nch += (mp.mux[c] == sm);
+				const DevResidue& r = residues[mp.submap_residue[sm]];
+				const uint32_t vch = r.type == 2 ? 1 : nch, vlen = r.type == 2 ? nch * half : half;
+				const uint64_t parts = (std::min(r.end, vlen) - std::min(r.begin, vlen)) / r.partition_size;
+				const uint64_t acc = (uint64_t) nch * half, cur = 8 * parts * vch;
+				acc_max = std::max(acc_max, acc); cur_max = std::max(cur_max, cur); both_max = std::max(both_max, acc + cur);
+			}
+		}
+		rec.res_smem = (uint32_t) (both_max * 4 + 64);
+		rec.res_acc_smem = (uint32_t) (acc_max * 4 + 64);
+		rec.res_cursors = (uint32_t) cur_max;
 	}
 	rec.n_modes = s->n_modes;
 	memcpy(rec.mode_blockflag, d.mode_blockflag, sizeof rec.mode_blockflag);
@@ -603,7 +619,7 @@ extern "C" int pov_setup_get_window(const pov_ctx* ctx, uint32_t id, int blockfl
 static void release_batch(pov_batch_handle* h) {
 	h->d_streams.release(); h->d_packets.release(); h->d_ys.release(); h->d_payload.release(); h->d_spec_off.release();
 	h->d_stage_off.release(); h->d_runs.release(); h->d_pcm.release(); h->d_status.release(); h->d_spectra.release();
-	h->d_entries.release(); h->d_pk_off.release();
+	h->d_entries.release(); h->d_pk_off.release(); h->d_res_cursor.release();
 	h->d_feat_rows.release(); h->d_feat_floors.release(); h->d_feat_out.release();
 	h->st_final_ys.release(); h->st_flag.release(); h->st_floor.release(); h->st_floor_out.release();
 	h->st_env.release(); h->st_mdct.release();
@@ -642,7 +658,7 @@ extern "C" int pov_batch_upload(pov_ctx* ctx, const pov_batch* b, pov_batch_hand
 	h->pk_ys_off.resize(raw_packets ? P : 0); h->pk_ent_off.resize(raw_packets ? P : 0); h->pk_raw_off.resize(raw_packets ? P : 0);
 	h->ys_cap = h->ent_cap = 0;
 	h->runs.clear();
-	uint32_t maxC = 1, maxbs = 64, minbs = 8192, maxposts = 2, res_smem = 0, posts_cls[2] = {2, 2};
+	uint32_t maxC = 1, maxbs = 64, minbs = 8192, maxposts = 2, res_smem = 0, res_acc_smem = 0, res_cursors = 0, posts_cls[2] = {2, 2};
 	bool only_std = true;
 	uint32_t table_float2 = 0;
 	uint64_t dense_floats = 0, stage_floats = 0, expect_first = 0;
@@ -689,6 +705,7 @@ extern "C" int pov_batch_upload(pov_ctx* ctx, const pov_batch* b, pov_batch_hand
 			return pov_fail(ctx, POV_ERR_ARG, "pov_batch: stream %u: PCM region exceeds pcm_floats", si);
 		maxC = std::max(maxC, C); maxbs = std::max(maxbs, su.blocksize[1]); minbs = std::min(minbs, su.blocksize[0]);
 		maxposts = std::max(maxposts, su.max_posts); res_smem = std::max(res_smem, su.res_smem);
+		res_acc_smem = std::max(res_acc_smem, su.res_acc_smem); res_cursors = std::max(res_cursors, su.res_cursors);
 		if(su.blocksize[0] != 256 || su.blocksize[1] != 2048) only_std = false;
 		table_float2 = std::max(table_float2, su.table_float2);
 		posts_cls[0] = std::max(posts_cls[0], su.posts_cls[0]); posts_cls[1] = std::max(posts_cls[1], su.posts_cls[1]);
@@ -812,7 +829,7 @@ extern "C" int pov_batch_upload(pov_ctx* ctx, const pov_batch* b, pov_batch_hand
 	h->max_channels = maxC; h->max_blocksize = maxbs; h->min_blocksize = std::min(minbs, maxbs);
 	h->floor_cap = (maxposts + 3u) & ~3u;
 	h->floor_cap_cls[0] = (posts_cls[0] + 3u) & ~3u; h->floor_cap_cls[1] = (posts_cls[1] + 3u) & ~3u;
-	h->res_smem = res_smem;
+	h->res_smem = res_smem; h->res_acc_smem = res_acc_smem; h->res_cursors = res_cursors;
 	h->only_256_2048 = only_std && b->n_streams > 0;
 	h->table_float2 = table_float2;
 	h->stage_floats = stage_floats;
@@ -894,7 +911,17 @@ static int run_residue_if_needed(pov_ctx* ctx, pov_batch_handle* h, const DevBat
 		CUDA_TRY(ctx, launch_packet_decode(raw, (pov_packet*) h->d_packets.ptr, (uint16_t*) h->d_ys.ptr, (uint8_t*) h->d_entries.ptr, off, off + h->n_packets,
 		                                   off + 2 * (size_t) h->n_packets, h->n_packets, ctx->stream, &ctx->launches));
 	}
-	CUDA_TRY(ctx, launch_residue_apply(v, (float*) h->d_spectra.ptr, h->res_smem, ctx->stream, &ctx->launches));
+	if(h->res_smem <= residue_apply_max_dynamic_smem()) {
+		CUDA_TRY(ctx, launch_residue_apply(v, (float*) h->d_spectra.ptr, h->res_smem, nullptr, 0, h->n_packets, ctx->stream, &ctx->launches));
+		return POV_OK;
+	}
+	// The cursors do not fit next to the working vector (small partitions of long multichannel blocks): they go to a global
+	// scratch of res_cursors words per block, at most 256 MB of it, and the blocks loop over the packets.
+	const uint64_t per = std::max<uint32_t>(h->res_cursors, 1);
+	const uint32_t grid = (uint32_t) std::max<uint64_t>(1, std::min<uint64_t>(h->n_packets, (256ull << 20) / (4 * per)));
+	CUDA_TRY(ctx, h->d_res_cursor.reserve(4 * per * grid));
+	CUDA_TRY(ctx, launch_residue_apply(v, (float*) h->d_spectra.ptr, h->res_acc_smem, (uint32_t*) h->d_res_cursor.ptr, (uint32_t) per, grid,
+	                                   ctx->stream, &ctx->launches));
 	return POV_OK;
 }
 

@@ -32,7 +32,10 @@ struct BlockTables {              // per blocksize n: DCT-IV rotation, FFT twidd
 
 struct SetupRec {
 	uint32_t channels = 0, sample_rate = 0, blocksize[2] = {0, 0};
-	uint32_t n_modes = 0, entry_bits = 16, max_posts = 2, res_smem = 0;
+	uint32_t n_modes = 0, entry_bits = 16, max_posts = 2;
+	// k_residue_apply, per packet of the worst mode: dynamic shared memory with the read cursors in it (res_smem), without
+	// them (res_acc_smem: the working vector only), and the cursor count (res_cursors, global scratch when they do not fit)
+	uint32_t res_smem = 0, res_acc_smem = 0, res_cursors = 0;
 	uint32_t posts_cls[2] = {2, 2};   // largest floor (posts) reachable from short / long modes
 	uint32_t table_float2 = 0;        // float2 slots of the fused kernel's shared-memory tables for this setup
 	uint8_t mode_blockflag[POV_MAX_MODES] = {0};
@@ -98,7 +101,7 @@ struct WarpGroup { uint32_t setup, first_run, n_runs; };   // runs of one setup:
 struct pov_batch_handle {
 	uint32_t n_streams = 0, n_packets = 0, input_kind = 0, pcm_layout = 0;   // pcm_layout as uploaded (POV_PCM_S16 included)
 	uint64_t pcm_floats = 0, stage_floats = 0, dense_floats = 0;
-	uint32_t max_channels = 1, max_blocksize = 64, min_blocksize = 64, floor_cap = 4, res_smem = 0;
+	uint32_t max_channels = 1, max_blocksize = 64, min_blocksize = 64, floor_cap = 4, res_smem = 0, res_acc_smem = 0, res_cursors = 0;
 	uint32_t floor_cap_cls[2] = {4, 4};
 	uint32_t table_float2 = 0;
 	bool fused_ok = true, staged_ready = false, only_256_2048 = false;
@@ -116,6 +119,7 @@ struct pov_batch_handle {
 	std::vector<DevRun> runs;
 	DevBuf d_streams, d_packets, d_ys, d_payload, d_spec_off, d_stage_off, d_runs, d_pcm, d_status, d_spectra;
 	DevBuf d_entries, d_pk_off;                      // POV_INPUT_PACKETS: entries payload written by k_packet_decode; ys_off | ent_off
+	DevBuf d_res_cursor;                             // k_residue_apply's read cursors when they do not fit its shared memory
 	DevBuf st_final_ys, st_flag, st_floor, st_floor_out, st_env, st_mdct;
 	// pinned copy of the derived arrays (spec_off | runs): sources of asynchronous copies, so they must not be pageable
 	// (a pageable source makes the "async" copy wait for the stream) and must outlive the copy (derived_copied)

@@ -33,8 +33,11 @@ struct DevStageBuffers {
 	float*    pcm_after_mdct;    // n-sized
 };
 
-cudaError_t launch_residue_apply(const DevBatchView& b, float* spectra_out, size_t smem_bytes, cudaStream_t st,
-                                 uint64_t* launches);
+// cursor_scratch == nullptr: one block per packet, read cursors in shared memory after the working vector. Otherwise `grid`
+// blocks loop over the packets and block i keeps its cursors at cursor_scratch + i * cursor_stride.
+cudaError_t launch_residue_apply(const DevBatchView& b, float* spectra_out, size_t smem_bytes, uint32_t* cursor_scratch,
+                                 uint32_t cursor_stride, uint32_t grid, cudaStream_t st, uint64_t* launches);
+size_t residue_apply_max_dynamic_smem();   // the current device's opt-in limit less k_residue_apply's static tables
 cudaError_t launch_staged(const DevBatchView& b, const DevStageBuffers& sb, uint32_t max_channels, cudaStream_t st,
                           uint64_t* launches);
 cudaError_t launch_fused(const DevBatchView& b, const DevRun* runs, uint32_t n_runs, uint32_t max_channels,

@@ -69,10 +69,13 @@ __global__ void __launch_bounds__(kFloorWarps * 32) k_floor1(DevBatchView b, Dev
 // residue VQ application: one block per packet. Entries are in the reference's decode order (pass, partition,
 // channel, vector); an exclusive scan of the per-(pass,partition,channel) vector counts gives every partition
 // its read cursor, so partitions are independent while each bin still receives its <= 8 addends in pass order.
+// The cursors live in shared memory after the submap's working vector, or, when g_cursor is set (too many partitions
+// for shared memory), in g_cursor + blockIdx.x * cursor_stride; the blocks then loop over the packets.
 // ---------------------------------------------------------------------------------------------------------------
 constexpr int kResThreads = 256;
 
-__global__ void __launch_bounds__(kResThreads) k_residue_apply(DevBatchView b, float* __restrict__ spectra_out) {
+__global__ void __launch_bounds__(kResThreads) k_residue_apply(DevBatchView b, float* __restrict__ spectra_out,
+                                                               uint32_t* __restrict__ g_cursor, uint32_t cursor_stride) {
 	extern __shared__ __align__(16) unsigned char res_smem[];
 	__shared__ uint32_t s_scan[kResThreads / 32];
 	__shared__ uint32_t s_carry;
@@ -82,129 +85,132 @@ __global__ void __launch_bounds__(kResThreads) k_residue_apply(DevBatchView b, f
 	__shared__ uint32_t s_nent[POV_MAX_CODEBOOKS];          // 0: no lookup table (lookup_type 0) -> every entry is invalid
 	__shared__ uint16_t s_dim[POV_MAX_CODEBOOKS];
 	__shared__ uint8_t s_books[POV_MAX_CLASSES * 8];
-	const uint32_t p = blockIdx.x;
-	const pov_packet pk = b.packets[p];
-	const DevSetup& su = setup_of(b, pk);
-	const uint32_t C = su.channels;
-	const uint32_t n = su.blocksize[su.mode_blockflag[pk.mode]], half = n / 2;
-	const DevMapping& mp = su.mappings[su.mode_mapping[pk.mode]];
-	float* out = spectra_out + b.spec_off[p];
-	float* acc = reinterpret_cast<float*>(res_smem);                 // [nch*half] working vector of one submap
-	uint32_t* cursor = reinterpret_cast<uint32_t*>(acc + (size_t) C * half);   // [8*parts*nch] exclusive offsets
-	const uint32_t n_books = min(su.n_codebooks, (uint32_t) POV_MAX_CODEBOOKS);
-	for(uint32_t i = threadIdx.x; i < n_books; i += blockDim.x) {
-		const DevCodebook cb = su.codebooks[i];
-		s_vq[i] = cb.vq;
-		s_nent[i] = cb.lookup_type ? cb.n_entries : 0u;
-		s_dim[i] = (uint16_t) min(cb.dim, 0xFFFFu);
-	}
+	for(uint32_t p = blockIdx.x; p < b.n_packets; p += gridDim.x) {
+		__syncthreads();                                         // the previous packet is done with the shared tables
+		const pov_packet pk = b.packets[p];
+		const DevSetup& su = setup_of(b, pk);
+		const uint32_t C = su.channels;
+		const uint32_t n = su.blocksize[su.mode_blockflag[pk.mode]], half = n / 2;
+		const DevMapping& mp = su.mappings[su.mode_mapping[pk.mode]];
+		float* out = spectra_out + b.spec_off[p];
+		float* acc = reinterpret_cast<float*>(res_smem);                 // [nch*half] working vector of one submap
+		const uint32_t n_books = min(su.n_codebooks, (uint32_t) POV_MAX_CODEBOOKS);
+		for(uint32_t i = threadIdx.x; i < n_books; i += blockDim.x) {
+			const DevCodebook cb = su.codebooks[i];
+			s_vq[i] = cb.vq;
+			s_nent[i] = cb.lookup_type ? cb.n_entries : 0u;
+			s_dim[i] = (uint16_t) min(cb.dim, 0xFFFFu);
+		}
 
-	// nonzero propagate (hpp:1174-1180) decides which channels the residue touches
-	uint32_t used = pk.floor_used;
-	for(uint32_t k = 0; k < mp.n_couplings; ++k) {
-		const uint32_t m = mp.coupling_mag[k], a = mp.coupling_ang[k];
-		if(((used >> m) | (used >> a)) & 1) used |= (1u << m) | (1u << a);
-	}
-	const uint8_t* pl = b.payload + pk.spec_off;
-	uint32_t bad = 0;
-	for(uint32_t s = 0; s < mp.n_submaps; ++s) {
-		uint32_t chs[POV_MAX_CHANNELS], nch = 0;
-		for(uint32_t c = 0; c < C; ++c) if(mp.mux[c] == s) chs[nch++] = c;
-		const DevResidue& rs = su.residues[mp.submap_residue[s]];
-		// type 2 decodes ONE interleaved vector of length nch*half that is always "used" (hpp:685-694)
-		const uint32_t rtype = rs.type;
-		const uint32_t vch = (rtype == 2) ? 1u : nch;
-		const uint32_t vlen = (rtype == 2) ? nch * half : half;
-		const uint32_t lb = min(rs.begin, vlen), le = min(rs.end, vlen);
-		const uint32_t psize = rs.partition_size;
-		const uint32_t parts = (le - lb) / psize;
-		const uint32_t n_entries = *reinterpret_cast<const uint32_t*>(pl);
-		const uint8_t* cls = pl + 4;
-		const uint32_t cls_bytes = (vch * parts + 3u) & ~3u;
-		const uint8_t* ent = cls + cls_bytes;
-		const bool ent16 = su.entry_bits == 16;
-		const uint32_t ent_bytes = (n_entries * (su.entry_bits / 8) + 3u) & ~3u;
-		pl = ent + ent_bytes;
+		// nonzero propagate (hpp:1174-1180) decides which channels the residue touches
+		uint32_t used = pk.floor_used;
+		for(uint32_t k = 0; k < mp.n_couplings; ++k) {
+			const uint32_t m = mp.coupling_mag[k], a = mp.coupling_ang[k];
+			if(((used >> m) | (used >> a)) & 1) used |= (1u << m) | (1u << a);
+		}
+		const uint8_t* pl = b.payload + pk.spec_off;
+		uint32_t bad = 0;
+		for(uint32_t s = 0; s < mp.n_submaps; ++s) {
+			uint32_t chs[POV_MAX_CHANNELS], nch = 0;
+			for(uint32_t c = 0; c < C; ++c) if(mp.mux[c] == s) chs[nch++] = c;
+			const DevResidue& rs = su.residues[mp.submap_residue[s]];
+			// type 2 decodes ONE interleaved vector of length nch*half that is always "used" (hpp:685-694)
+			const uint32_t rtype = rs.type;
+			const uint32_t vch = (rtype == 2) ? 1u : nch;
+			const uint32_t vlen = (rtype == 2) ? nch * half : half;
+			const uint32_t lb = min(rs.begin, vlen), le = min(rs.end, vlen);
+			const uint32_t psize = rs.partition_size;
+			const uint32_t parts = (le - lb) / psize;
+			uint32_t* cursor = g_cursor ? g_cursor + (size_t) blockIdx.x * cursor_stride          // [8*parts*vch] exclusive offsets
+			                            : reinterpret_cast<uint32_t*>(acc + (size_t) nch * half);
+			const uint32_t n_entries = *reinterpret_cast<const uint32_t*>(pl);
+			const uint8_t* cls = pl + 4;
+			const uint32_t cls_bytes = (vch * parts + 3u) & ~3u;
+			const uint8_t* ent = cls + cls_bytes;
+			const bool ent16 = su.entry_bits == 16;
+			const uint32_t ent_bytes = (n_entries * (su.entry_bits / 8) + 3u) & ~3u;
+			pl = ent + ent_bytes;
 
-		__syncthreads();                                     // previous submap done with s_books / acc; book tables visible
-		for(uint32_t i = threadIdx.x; i < rs.n_class * 8u; i += blockDim.x) s_books[i] = rs.books[i];
-		for(uint32_t i = threadIdx.x; i < vch * vlen; i += blockDim.x) acc[i] = 0.f;
-		if(threadIdx.x == 0) s_carry = 0;
-		__syncthreads();
-		// vector counts in decode order (pass, partition, channel) + block-wide exclusive scan: warp shuffles, one
-		// shared-memory hop between the warps
-		const uint32_t items = 8 * parts * vch;
-		const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
-		for(uint32_t base = 0; base < items; base += blockDim.x) {
-			const uint32_t it = base + threadIdx.x;
-			uint32_t cnt = 0;
-			if(it < items) {
-				const uint32_t j = it % vch, part = (it / vch) % parts, pass = it / (vch * parts);
+			__syncthreads();                                     // previous submap done with s_books / acc; book tables visible
+			for(uint32_t i = threadIdx.x; i < rs.n_class * 8u; i += blockDim.x) s_books[i] = rs.books[i];
+			for(uint32_t i = threadIdx.x; i < vch * vlen; i += blockDim.x) acc[i] = 0.f;
+			if(threadIdx.x == 0) s_carry = 0;
+			__syncthreads();
+			// vector counts in decode order (pass, partition, channel) + block-wide exclusive scan: warp shuffles, one
+			// shared-memory hop between the warps
+			const uint32_t items = 8 * parts * vch;
+			const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+			for(uint32_t base = 0; base < items; base += blockDim.x) {
+				const uint32_t it = base + threadIdx.x;
+				uint32_t cnt = 0;
+				if(it < items) {
+					const uint32_t j = it % vch, part = (it / vch) % parts, pass = it / (vch * parts);
+					const bool ch_used = (rtype == 2) ? true : ((used >> chs[j]) & 1);
+					if(ch_used) {
+						const uint32_t book = s_books[cls[j * parts + part] * 8 + pass];
+						if(book != POV_NO_BOOK && book < n_books) cnt = psize / s_dim[book];
+					}
+				}
+				uint32_t incl = cnt;
+	#pragma unroll
+				for(int o = 1; o < 32; o <<= 1) {
+					const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
+					if((int) lane >= o) incl += v;
+				}
+				if(lane == 31) s_scan[warp] = incl;
+				__syncthreads();
+				uint32_t before = s_carry;
+				for(uint32_t w = 0; w < warp; ++w) before += s_scan[w];
+				if(it < items) cursor[it] = before + incl - cnt;
+				__syncthreads();
+				if(threadIdx.x == blockDim.x - 1) s_carry = before + incl;
+				__syncthreads();
+			}
+			// apply: one thread per BIN. A bin receives at most one addend per pass (hpp:734-752), so it can gather its own
+			// addends in pass order: the same additions, in the same order, as the reference's vector-by-vector accumulation
+			// (which starts from the zero-initialised vector), with every thread of the block busy instead of one per partition.
+			for(uint32_t idx = threadIdx.x; idx < parts * vch * psize; idx += blockDim.x) {
+				const uint32_t o = idx % psize, w = idx / psize;
+				const uint32_t j = w % vch, part = w / vch;
 				const bool ch_used = (rtype == 2) ? true : ((used >> chs[j]) & 1);
-				if(ch_used) {
-					const uint32_t book = s_books[cls[j * parts + part] * 8 + pass];
-					if(book != POV_NO_BOOK && book < n_books) cnt = psize / s_dim[book];
+				if(!ch_used) continue;
+				const uint32_t cl = cls[j * parts + part];
+				float sum = 0.f;
+	#pragma unroll
+				for(uint32_t pass = 0; pass < 8; ++pass) {
+					const uint32_t book = s_books[cl * 8 + pass];
+					if(book == POV_NO_BOOK) continue;
+					if(book >= n_books) { bad |= POV_PKT_VQ_ENTRY; continue; }
+					const uint32_t dim = s_dim[book];
+					const uint32_t nvec = psize / dim;
+					// type 0: v[k + l*nvec] (hpp:734-743); types 1/2: v[k*dim + l] (hpp:744-752)
+					uint32_t k, l;
+					if(rtype == 0) { if(nvec == 0) continue; l = o / nvec; k = o - l * nvec; if(l >= dim) continue; }
+					else { k = o / dim; l = o - k * dim; if(k >= nvec) continue; }
+					const uint32_t cur = cursor[(pass * parts + part) * vch + j] + k;
+					if(cur >= n_entries) { bad |= POV_PKT_VQ_ENTRY; continue; }
+					const uint32_t e = ent16 ? reinterpret_cast<const uint16_t*>(ent)[cur] : reinterpret_cast<const uint32_t*>(ent)[cur];
+					if(e >= s_nent[book]) { bad |= POV_PKT_VQ_ENTRY; continue; }
+					sum += __ldg(&s_vq[book][(size_t) e * dim + l]);
+				}
+				acc[(size_t) j * vlen + lb + part * psize + o] = sum;
+			}
+			__syncthreads();
+			// scatter to the channel-major dense layout (de-interleave for type 2, hpp:690-692)
+			if(rtype == 2) {
+				for(uint32_t i = threadIdx.x; i < nch * half; i += blockDim.x) {
+					const uint32_t j = i % nch, bin = i / nch;
+					out[(size_t) chs[j] * half + bin] = acc[i];
+				}
+			} else {
+				for(uint32_t i = threadIdx.x; i < nch * half; i += blockDim.x) {
+					const uint32_t j = i / half, bin = i % half;
+					out[(size_t) chs[j] * half + bin] = acc[i];
 				}
 			}
-			uint32_t incl = cnt;
-#pragma unroll
-			for(int o = 1; o < 32; o <<= 1) {
-				const uint32_t v = __shfl_up_sync(0xffffffffu, incl, o);
-				if((int) lane >= o) incl += v;
-			}
-			if(lane == 31) s_scan[warp] = incl;
-			__syncthreads();
-			uint32_t before = s_carry;
-			for(uint32_t w = 0; w < warp; ++w) before += s_scan[w];
-			if(it < items) cursor[it] = before + incl - cnt;
-			__syncthreads();
-			if(threadIdx.x == blockDim.x - 1) s_carry = before + incl;
-			__syncthreads();
 		}
-		// apply: one thread per BIN. A bin receives at most one addend per pass (hpp:734-752), so it can gather its own
-		// addends in pass order: the same additions, in the same order, as the reference's vector-by-vector accumulation
-		// (which starts from the zero-initialised vector), with every thread of the block busy instead of one per partition.
-		for(uint32_t idx = threadIdx.x; idx < parts * vch * psize; idx += blockDim.x) {
-			const uint32_t o = idx % psize, w = idx / psize;
-			const uint32_t j = w % vch, part = w / vch;
-			const bool ch_used = (rtype == 2) ? true : ((used >> chs[j]) & 1);
-			if(!ch_used) continue;
-			const uint32_t cl = cls[j * parts + part];
-			float sum = 0.f;
-#pragma unroll
-			for(uint32_t pass = 0; pass < 8; ++pass) {
-				const uint32_t book = s_books[cl * 8 + pass];
-				if(book == POV_NO_BOOK) continue;
-				if(book >= n_books) { bad |= POV_PKT_VQ_ENTRY; continue; }
-				const uint32_t dim = s_dim[book];
-				const uint32_t nvec = psize / dim;
-				// type 0: v[k + l*nvec] (hpp:734-743); types 1/2: v[k*dim + l] (hpp:744-752)
-				uint32_t k, l;
-				if(rtype == 0) { if(nvec == 0) continue; l = o / nvec; k = o - l * nvec; if(l >= dim) continue; }
-				else { k = o / dim; l = o - k * dim; if(k >= nvec) continue; }
-				const uint32_t cur = cursor[(pass * parts + part) * vch + j] + k;
-				if(cur >= n_entries) { bad |= POV_PKT_VQ_ENTRY; continue; }
-				const uint32_t e = ent16 ? reinterpret_cast<const uint16_t*>(ent)[cur] : reinterpret_cast<const uint32_t*>(ent)[cur];
-				if(e >= s_nent[book]) { bad |= POV_PKT_VQ_ENTRY; continue; }
-				sum += __ldg(&s_vq[book][(size_t) e * dim + l]);
-			}
-			acc[(size_t) j * vlen + lb + part * psize + o] = sum;
-		}
-		__syncthreads();
-		// scatter to the channel-major dense layout (de-interleave for type 2, hpp:690-692)
-		if(rtype == 2) {
-			for(uint32_t i = threadIdx.x; i < nch * half; i += blockDim.x) {
-				const uint32_t j = i % nch, bin = i / nch;
-				out[(size_t) chs[j] * half + bin] = acc[i];
-			}
-		} else {
-			for(uint32_t i = threadIdx.x; i < nch * half; i += blockDim.x) {
-				const uint32_t j = i / half, bin = i % half;
-				out[(size_t) chs[j] * half + bin] = acc[i];
-			}
-		}
+		if(bad) atomicOr(&b.status[p], bad);
 	}
-	if(bad) atomicOr(&b.status[p], bad);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -396,15 +402,24 @@ __global__ void __launch_bounds__(256) k_checksum_s16(const int16_t* __restrict_
 // ---------------------------------------------------------------------------------------------------------------
 // launchers
 // ---------------------------------------------------------------------------------------------------------------
-cudaError_t launch_residue_apply(const DevBatchView& b, float* spectra_out, size_t smem, cudaStream_t st,
-                                 uint64_t* launches) {
+size_t residue_apply_max_dynamic_smem() {
+	int dev = 0, optin = 0;
+	cudaFuncAttributes fa;
+	if(cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess ||
+	   cudaFuncGetAttributes(&fa, k_residue_apply) != cudaSuccess)
+		return 48 * 1024 - 8 * 1024;
+	return (size_t) optin > fa.sharedSizeBytes ? (size_t) optin - fa.sharedSizeBytes : 0;
+}
+
+cudaError_t launch_residue_apply(const DevBatchView& b, float* spectra_out, size_t smem, uint32_t* cursor_scratch,
+                                 uint32_t cursor_stride, uint32_t grid, cudaStream_t st, uint64_t* launches) {
 	if(b.n_packets == 0) return cudaSuccess;
-	// smem = max over the batch of (C * n/2 floats + 8 * partitions * channels cursors), computed at upload
+	// smem = max over the batch's submaps of (nch * n/2 floats [+ 8 * partitions * vectors cursors]), computed at upload
 	if(smem > 48 * 1024) {
 		cudaError_t e = cudaFuncSetAttribute(k_residue_apply, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
 		if(e != cudaSuccess) return e;
 	}
-	k_residue_apply<<<b.n_packets, kResThreads, smem, st>>>(b, spectra_out);
+	k_residue_apply<<<grid, kResThreads, smem, st>>>(b, spectra_out, cursor_scratch, cursor_stride);
 	if(launches) ++*launches;
 	return cudaGetLastError();
 }
