@@ -135,7 +135,9 @@ typedef struct pov_stream {
 	uint32_t first_packet;
 	uint32_t n_packets;
 	uint32_t reserved;
-	uint64_t pcm_frames;      /* sum of emit_frames of its packets = frames this stream yields in this batch */
+	uint64_t pcm_frames;      /* sum of emit_frames of its packets = frames this stream yields in this batch. Planar: this is
+	                             also the channel stride, and it may exceed that sum (a padded layout); frames past the sum
+	                             are not written. The kernels use no other property of it. */
 	uint64_t pcm_base;        /* float index of channel 0 / frame 0 in the PCM arena. Planar: channel c, frame f
 	                             lives at pcm_base + c*pcm_frames + f. Interleaved: pcm_base + f*channels + c. */
 } pov_stream;
@@ -262,8 +264,16 @@ int  pov_batch_fetch_pcm(pov_ctx* ctx, pov_batch_handle* h, float* out, uint64_t
 /* The same for a POV_PCM_S16 batch: n_values int16 samples (<= pcm_floats). POV_ERR_ARG on a float32 batch. */
 int  pov_batch_fetch_pcm_s16(pov_ctx* ctx, pov_batch_handle* h, int16_t* out, uint64_t n_values, int sync);
 /* Device pointer of the PCM arena (for callers that consume PCM on the GPU): float[pcm_floats], or int16_t[pcm_floats] for a
- * POV_PCM_S16 batch. */
+ * POV_PCM_S16 batch; after pov_batch_upload_into, the caller's pcm_dev. */
 void* pov_batch_pcm_dev(pov_batch_handle* h);
+/* pov_batch_upload with the PCM going to memory the caller owns: the kernels of every later run of the handle (pov_batch_run,
+ * pov_batch_run_staged, the staged run pov_batch_features may start) write the PCM to `pcm_dev`, device memory of the context's
+ * GPU holding batch->pcm_floats samples (float32, or int16 with POV_PCM_S16), aligned to a sample. The handle allocates no PCM
+ * arena; pov_batch_pcm_dev returns pcm_dev and the fetch calls copy from it. The writes are issued on pov_ctx_stream(ctx): the
+ * caller orders its own work against that stream. Only the PCM regions of the batch's streams are written (planar: channels x
+ * emitted frames at pcm_base + c*pcm_frames), so padding between and after them keeps what the caller put there. A handle that
+ * a plain pov_batch_upload reuses gets its own arena again. */
+int  pov_batch_upload_into(pov_ctx* ctx, const pov_batch* batch, void* pcm_dev, pov_batch_handle** out);
 /* One debug stage of one (packet, channel) after pov_batch_run_staged; `out_bytes` must match the stage size. */
 int  pov_batch_fetch_stage(pov_ctx* ctx, pov_batch_handle* h, uint32_t packet, uint32_t channel, int stage,
                            void* out, uint64_t out_bytes);
@@ -347,6 +357,57 @@ typedef int (*pov_pcm_sink_s16)(uint32_t file_index, uint32_t channels, uint64_t
 int  pov_decode_corpus_s16(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* data, const size_t* len,
                            uint32_t host_threads, pov_pcm_sink_s16 sink, void* user,
                            uint64_t* frames_out, uint64_t* total_values_out, int64_t* sum_out);
+
+/* Host-only (no GPU needed): one record per logical stream the corpus decode decodes — every Vorbis stream of every file that
+ * reaches a complete setup, in file order and, inside a file, in the order the corpus decode delivers them (a chained file has
+ * several). It runs the corpus decode's own parse (raw-packet mode, `host_threads` threads, 0 = all cores but one) and discards
+ * the packets, so `frames` is what the decode produces. flags: POV_PARSE_ALLOW_SPANNING (see pov_ogg_parse_memory_ex; the
+ * corpus decode follows pov_ctx_set_page_spanning). A framing or header error fails with POV_ERR_STREAM and the text
+ * pov_decode_corpus gives for it ("file k: check failed: ..."), in *error_out (per-thread buffer). On success *out holds
+ * *n_streams_out records (NULL when there are none), allocated by the library: free with pov_corpus_streams_free.
+ * Callers use it to size and lay out the output of pov_decode_corpus_device, or to bucket files by length. */
+typedef struct pov_stream_info {
+	uint32_t file;            /* index into the corpus */
+	uint32_t channels;
+	uint32_t sample_rate;
+	uint32_t reserved;
+	uint64_t frames;          /* frames per channel the decode yields for this stream */
+} pov_stream_info;
+int  pov_corpus_streams(uint32_t n_files, const uint8_t* const* data, const size_t* len, uint32_t flags, uint32_t host_threads,
+                        pov_stream_info** out, uint64_t* n_streams_out, const char** error_out);
+void pov_corpus_streams_free(pov_stream_info* p);
+
+/* Where pov_decode_corpus_device writes: one planar region per record of the stream table (pov_corpus_streams), in device
+ * memory the caller owns on the context's GPU (a torch tensor, for example). Stream i, channel c, frame f lands at sample index
+ * stream_base[i] + c * channel_stride[i] + f of pcm_dev. Strides and bases that are multiples of 4 keep the kernels on their
+ * vector stores; any values work. */
+typedef struct pov_device_pcm {
+	uint32_t pcm_layout;              /* POV_PCM_PLANAR, optionally | POV_PCM_S16 (int16 samples); interleaved is refused */
+	uint32_t n_streams;               /* records of the stream table */
+	void*    pcm_dev;                 /* float32 or int16 samples on the context's device, aligned to a sample */
+	uint64_t capacity;                /* samples at pcm_dev */
+	const uint64_t* stream_base;      /* [n_streams] sample index of channel 0, frame 0 */
+	const uint64_t* channel_stride;   /* [n_streams] samples between channels, >= frames */
+	const uint32_t* file;             /* [n_streams] from the table: checked against what is parsed */
+	const uint32_t* channels;         /* [n_streams] from the table: checked against what is parsed */
+	const uint64_t* frames;           /* [n_streams] from the table: checked against what is parsed */
+	void*    cuda_stream;             /* the caller's cudaStream_t, or NULL (legacy default stream): no PCM write starts before
+	                                     the work queued on it when the call is made */
+} pov_device_pcm;
+/* The corpus decode with the PCM landing in the caller's device memory: only compressed packets go host -> device and only the
+ * per-packet status words come back (pov_ctx_io_bytes counts 4 bytes per audio packet device -> host). Same workers, chunks
+ * and errors as pov_decode_corpus_pcm.
+ * - Before anything is launched the regions are validated: layout, null pointers, channels > 0, stride >= frames,
+ *   base + channels * stride <= capacity, no two regions [base, base + channels * stride) overlapping. POV_ERR_ARG otherwise.
+ * - Every parsed stream is compared with the record at its index (file, channels, frames) before its chunk is uploaded; a
+ *   mismatch, more streams than n_streams, or fewer at the end, is POV_ERR_ARG naming the file. Chunks uploaded before that
+ *   point have written their streams.
+ * - The library writes exactly [base + c * stride, base + c * stride + frames) for c < channels of every stream: padding keeps
+ *   whatever the caller put there.
+ * - The call returns after every chunk has finished on the device, so on success the PCM is complete and visible to any stream.
+ * frames_out[n_files] (may be NULL) and *total_values_out are as in pov_decode_corpus. */
+int  pov_decode_corpus_device(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* data, const size_t* len, uint32_t host_threads,
+                              const pov_device_pcm* out, uint64_t* frames_out, uint64_t* total_values_out);
 
 /* Host-only front-end (no GPU needed): parse a whole Ogg/Vorbis file into descriptor batches, one per logical stream
  * (Ogg framing hpp:51-102,1433-1484; headers hpp:1283-1373; per-packet entropy decode hpp:498-517, 711-757). The

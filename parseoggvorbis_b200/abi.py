@@ -25,6 +25,7 @@ POV_PKT_OK, POV_PKT_FLOOR_PREDICTED, POV_PKT_FLOOR_RANGE, POV_PKT_VQ_ENTRY = 0, 
 POV_INPUT_DENSE, POV_INPUT_ENTRIES, POV_INPUT_PACKETS = 0, 1, 2
 POV_PCM_PLANAR, POV_PCM_INTERLEAVED = 0, 1
 POV_PCM_S16 = 0x100          # OR-ed into pcm_layout: the kernels store int16 PCM (see include/pov_synth.h)
+POV_PARSE_RAW_PACKETS, POV_PARSE_ALLOW_SPANNING = 1, 2     # flags of pov_ogg_parse_memory_ex / pov_corpus_streams
 
 (POV_STAGE_FINAL_YS, POV_STAGE_STEP2_FLAG, POV_STAGE_FLOOR, POV_STAGE_FLOOR_OUTPUTS,
  POV_STAGE_AFTER_RESIDUE, POV_STAGE_AFTER_ENVELOPE, POV_STAGE_PCM_AFTER_MDCT) = range(7)
@@ -105,6 +106,20 @@ class pov_decoded(C.Structure):
 class pov_decoded_s16(C.Structure):
     _fields_ = [("channels", C.c_uint32), ("sample_rate", C.c_uint32), ("frames", C.c_uint64),
                 ("audio_packets", C.c_uint32), ("reserved", C.c_uint32), ("pcm", C.POINTER(C.c_int16))]
+
+
+class pov_stream_info(C.Structure):
+    """One record of pov_corpus_streams' stream table."""
+    _fields_ = [("file", C.c_uint32), ("channels", C.c_uint32), ("sample_rate", C.c_uint32), ("reserved", C.c_uint32),
+                ("frames", C.c_uint64)]
+
+
+class pov_device_pcm(C.Structure):
+    """Output description of pov_decode_corpus_device: per stream-table record a planar region of the caller's device memory."""
+    _fields_ = [("pcm_layout", C.c_uint32), ("n_streams", C.c_uint32), ("pcm_dev", C.c_void_p), ("capacity", C.c_uint64),
+                ("stream_base", C.POINTER(C.c_uint64)), ("channel_stride", C.POINTER(C.c_uint64)),
+                ("file", C.POINTER(C.c_uint32)), ("channels", C.POINTER(C.c_uint32)), ("frames", C.POINTER(C.c_uint64)),
+                ("cuda_stream", C.c_void_p)]
 
 
 # numpy dtypes with the same layout as pov_stream / pov_packet (so big batches are built vectorised)

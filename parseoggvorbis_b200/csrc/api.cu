@@ -634,7 +634,32 @@ extern "C" void pov_batch_free(pov_ctx* ctx, pov_batch_handle* h) {
 	delete h;
 }
 
+// Device memory of the context's GPU, aligned to `align` bytes: where pov_batch_upload_into / pov_decode_corpus_device may write.
+int pov_check_pcm_dev(pov_ctx* ctx, const void* p, size_t align, const char* fn) {
+	if(!p) return pov_fail(ctx, POV_ERR_ARG, "%s: null pcm_dev", fn);
+	if((uintptr_t) p % align) return pov_fail(ctx, POV_ERR_ARG, "%s: pcm_dev is not aligned to a %zu-byte sample", fn, align);
+	cudaPointerAttributes a;
+	if(cudaPointerGetAttributes(&a, p) != cudaSuccess) { (void) cudaGetLastError(); return pov_fail(ctx, POV_ERR_ARG, "%s: pcm_dev is not a CUDA pointer", fn); }
+	if((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != ctx->device)
+		return pov_fail(ctx, POV_ERR_ARG, "%s: pcm_dev is not device memory of the context's device %d", fn, ctx->device);
+	return POV_OK;
+}
+
+static int batch_upload(pov_ctx* ctx, const pov_batch* b, void* pcm_dev, pov_batch_handle** out);
+
 extern "C" int pov_batch_upload(pov_ctx* ctx, const pov_batch* b, pov_batch_handle** out) try {
+	return batch_upload(ctx, b, nullptr, out);
+} POV_NOTHROW_END(ctx)
+
+extern "C" int pov_batch_upload_into(pov_ctx* ctx, const pov_batch* b, void* pcm_dev, pov_batch_handle** out) try {
+	if(!ctx || !b || !out) return POV_ERR_ARG;
+	cudaSetDevice(ctx->device);
+	const int rc = pov_check_pcm_dev(ctx, pcm_dev, pcm_elem_bytes(b->pcm_layout), "pov_batch_upload_into");
+	return rc ? rc : batch_upload(ctx, b, pcm_dev, out);
+} POV_NOTHROW_END(ctx)
+
+// pcm_dev == nullptr: the handle's own PCM arena
+static int batch_upload(pov_ctx* ctx, const pov_batch* b, void* pcm_dev, pov_batch_handle** out) {
 	if(!ctx || !b || !out) return POV_ERR_ARG;
 	cudaSetDevice(ctx->device);
 	if(b->input_kind > POV_INPUT_PACKETS || (b->pcm_layout & ~POV_PCM_S16) > POV_PCM_INTERLEAVED) return pov_fail(ctx, POV_ERR_ARG, "pov_batch: bad input_kind/pcm_layout");
@@ -875,13 +900,15 @@ extern "C" int pov_batch_upload(pov_ctx* ctx, const pov_batch* b, pov_batch_hand
 		CUDA_TRY(ctx, up(h->d_runs, (uint8_t*) h->h_derived + o_runs, b_runs));
 		CUDA_TRY(ctx, cudaEventRecord(h->derived_copied, st));
 	}
-	CUDA_TRY(ctx, h->d_pcm.reserve(std::max<size_t>(pcm_elem_bytes(b->pcm_layout) * b->pcm_floats, 16)));
+	if(pcm_dev) h->d_pcm.release();          // (cudaFree waits for the device: the previous run has written its arena)
+	else CUDA_TRY(ctx, h->d_pcm.reserve(std::max<size_t>(pcm_elem_bytes(b->pcm_layout) * b->pcm_floats, 16)));
+	h->pcm_ext = pcm_dev;
 	CUDA_TRY(ctx, h->d_status.reserve(std::max<size_t>(sizeof(uint32_t) * P, 16)));
 	CUDA_TRY(ctx, cudaMemsetAsync(h->d_status.ptr, 0, sizeof(uint32_t) * P, st));
 	if(b->input_kind != POV_INPUT_DENSE) CUDA_TRY(ctx, h->d_spectra.reserve(std::max<size_t>(sizeof(float) * dense_floats, 16)));
 	if(fresh) *out = fresh.release();
 	return POV_OK;
-} POV_NOTHROW_END(ctx)
+}
 
 static DevBatchView make_view(pov_ctx* ctx, pov_batch_handle* h) {
 	DevBatchView v;
@@ -894,7 +921,7 @@ static DevBatchView make_view(pov_ctx* ctx, pov_batch_handle* h) {
 	else if(h->input_kind == POV_INPUT_ENTRIES) { v.spectra = (const float*) h->d_spectra.ptr; v.payload = (const uint8_t*) h->d_payload.ptr; }
 	else { v.spectra = (const float*) h->d_spectra.ptr; v.payload = (const uint8_t*) h->d_entries.ptr; }   // (what k_packet_decode writes)
 	v.inv_db = ctx->d_inv_db;
-	v.pcm = h->d_pcm.ptr;
+	v.pcm = h->pcm();
 	v.status = (uint32_t*) h->d_status.ptr;
 	v.n_streams = h->n_streams; v.n_packets = h->n_packets;
 	v.pcm_layout = h->pcm_layout & ~POV_PCM_S16; v.pcm_s16 = (h->pcm_layout & POV_PCM_S16) ? 1u : 0u;
@@ -1040,7 +1067,7 @@ static int fetch_pcm(pov_ctx* ctx, pov_batch_handle* h, void* out, uint64_t n_va
 		return pov_fail(ctx, POV_ERR_ARG, "%s: the batch's PCM arena holds %s samples", fn, s16 ? "float32" : "int16 (POV_PCM_S16)");
 	if(n_values > h->pcm_floats) return pov_fail(ctx, POV_ERR_ARG, "%s: %llu samples requested, arena holds %llu", fn, (unsigned long long) n_values, (unsigned long long) h->pcm_floats);
 	cudaSetDevice(ctx->device);
-	if(n_values) CUDA_TRY(ctx, pov_copy_out_async(ctx, out, h->d_pcm.ptr, n_values * pcm_elem_bytes(h->pcm_layout)));
+	if(n_values) CUDA_TRY(ctx, pov_copy_out_async(ctx, out, h->pcm(), n_values * pcm_elem_bytes(h->pcm_layout)));
 	if(sync) CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
 	return POV_OK;
 }
@@ -1053,7 +1080,7 @@ extern "C" int pov_batch_fetch_pcm_s16(pov_ctx* ctx, pov_batch_handle* h, int16_
 	return fetch_pcm(ctx, h, out, n_values, sync, true, "pov_batch_fetch_pcm_s16");
 } POV_NOTHROW_END(ctx)
 
-extern "C" void* pov_batch_pcm_dev(pov_batch_handle* h) { return h ? h->d_pcm.ptr : nullptr; }
+extern "C" void* pov_batch_pcm_dev(pov_batch_handle* h) { return h ? h->pcm() : nullptr; }
 
 extern "C" int pov_batch_status(pov_ctx* ctx, pov_batch_handle* h, uint32_t* out, uint32_t n) try {
 	if(!ctx || !h) return POV_ERR_ARG;

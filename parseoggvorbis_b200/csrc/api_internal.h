@@ -118,6 +118,8 @@ struct pov_batch_handle {
 	DevBuf d_feat_rows, d_feat_floors, d_feat_out;   // pov_batch_features
 	std::vector<DevRun> runs;
 	DevBuf d_streams, d_packets, d_ys, d_payload, d_spec_off, d_stage_off, d_runs, d_pcm, d_status, d_spectra;
+	void* pcm_ext = nullptr;                         // pov_batch_upload_into: the caller's PCM memory (then d_pcm is empty)
+	void* pcm() const { return pcm_ext ? pcm_ext : d_pcm.ptr; }
 	DevBuf d_entries, d_pk_off;                      // POV_INPUT_PACKETS: entries payload written by k_packet_decode; ys_off | ent_off
 	DevBuf d_res_cursor;                             // k_residue_apply's read cursors when they do not fit its shared memory
 	DevBuf st_final_ys, st_flag, st_floor, st_floor_out, st_env, st_mdct;

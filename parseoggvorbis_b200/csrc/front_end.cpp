@@ -6,6 +6,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <atomic>
 #include <chrono>
 #include <condition_variable>
@@ -270,6 +271,80 @@ extern "C" void pov_decoded_s16_free(pov_decoded_s16* d) {
 }
 
 // ---------------------------------------------------------------------------------------------------------------
+// stream table of a corpus (host only): the corpus workers' parse, packets discarded
+// ---------------------------------------------------------------------------------------------------------------
+extern "C" int pov_corpus_streams(uint32_t n_files, const uint8_t* const* data, const size_t* len, uint32_t flags, uint32_t host_threads,
+                                  pov_stream_info** out, uint64_t* n_streams_out, const char** error_out) {
+	static thread_local char errbuf[512];
+	if(!out || !n_streams_out || (n_files && (!data || !len))) return POV_ERR_ARG;
+	*out = nullptr; *n_streams_out = 0;
+	try {
+	if(host_threads == 0) { const uint32_t hc = std::thread::hardware_concurrency(); host_threads = hc > 1 ? hc - 1 : 1; }
+	host_threads = std::max(1u, std::min(host_threads, n_files));
+	std::vector<std::vector<pov_stream_info>> per_file(n_files);
+	std::vector<std::string> error(n_files);
+	std::atomic<uint32_t> next(0), first_error(n_files);
+	auto worker = [&]() {
+		std::vector<StreamWork> file;
+		ParseOptions opt;
+		opt.raw_packets = true;
+		opt.allow_spanning = (flags & POV_PARSE_ALLOW_SPANNING) != 0;
+		for(;;) {
+			const uint32_t i = next.fetch_add(1);
+			if(i >= n_files || i > first_error.load()) return;          // (files after a failed one are not needed)
+			try {
+				ParseError err;
+				file.clear();
+				if(!parse_ogg_file(data[i], len[i], file, err, opt)) {
+					error[i] = "file " + std::to_string(i) + ": check failed: " + err.msg;
+					uint32_t f = first_error.load();
+					while(i < f && !first_error.compare_exchange_weak(f, i)) {}
+					continue;
+				}
+				for(const StreamWork& st : file) {
+					if(!st.have_setup) continue;
+					pov_stream_info r;
+					memset(&r, 0, sizeof r);
+					r.file = i; r.channels = st.setup.channels; r.sample_rate = st.setup.sample_rate; r.frames = st.frames;
+					per_file[i].push_back(r);
+				}
+			} catch(...) {
+				error[i] = "file " + std::to_string(i) + ": out of memory or internal error while parsing";
+				uint32_t f = first_error.load();
+				while(i < f && !first_error.compare_exchange_weak(f, i)) {}
+			}
+		}
+	};
+	std::vector<std::thread> pool;
+	for(uint32_t t = 1; t < host_threads; ++t) pool.emplace_back(worker);
+	worker();
+	for(auto& t : pool) t.join();
+	if(first_error.load() < n_files) {
+		snprintf(errbuf, sizeof errbuf, "%s", error[first_error.load()].c_str());
+		if(error_out) *error_out = errbuf;
+		return POV_ERR_STREAM;
+	}
+	uint64_t n = 0;
+	for(const auto& v : per_file) n += v.size();
+	if(n) {
+		pov_stream_info* p = (pov_stream_info*) malloc(n * sizeof(pov_stream_info));
+		if(!p) throw std::bad_alloc();
+		uint64_t at = 0;
+		for(const auto& v : per_file) { memcpy(p + at, v.data(), v.size() * sizeof(pov_stream_info)); at += v.size(); }
+		*out = p;
+	}
+	*n_streams_out = n;
+	return POV_OK;
+	} catch(...) {
+		snprintf(errbuf, sizeof errbuf, "out of memory or internal error while building the stream table");
+		if(error_out) *error_out = errbuf;
+		return POV_ERR_ARG;
+	}
+}
+
+extern "C" void pov_corpus_streams_free(pov_stream_info* p) { free(p); }
+
+// ---------------------------------------------------------------------------------------------------------------
 // corpus decode: `host_threads` front-end workers parse files into chunks, the calling thread feeds the GPU
 // ---------------------------------------------------------------------------------------------------------------
 // float64 sum of a float arena into *(double*) d_sum, or (s16) exact int64 sum of an int16 arena into *(uint64_t*) d_sum
@@ -289,6 +364,7 @@ struct Chunk {
 	std::vector<StreamWork> setups;            // one representative stream (headers only) per distinct setup
 	std::vector<uint64_t> frames;              // per file
 	std::vector<uint32_t> stream_file, stream_channels;   // per stream of the batch: file index (corpus-wide), channel count
+	std::vector<uint64_t> stream_frames;       // per stream of the batch
 	std::string error;
 };
 
@@ -366,9 +442,11 @@ void corpus_state_free(void* p) { delete (CorpusState*) p; }
 inline size_t align16(size_t x) { return (x + 15) & ~(size_t) 15; }
 }  // namespace
 
-// Output format of a corpus decode: float32 (sink, checksum) or int16 (POV_PCM_S16: sink16, sum16).
+// Output format of a corpus decode: float32 (sink, checksum), int16 (POV_PCM_S16: sink16, sum16), or the caller's device
+// memory (dev: float32 or int16 by dev->pcm_layout; no PCM leaves the device).
 struct CorpusOut {
 	bool s16 = false;
+	const pov_device_pcm* dev = nullptr;
 	pov_pcm_sink sink = nullptr;
 	pov_pcm_sink_s16 sink16 = nullptr;
 	void* user = nullptr;
@@ -398,6 +476,52 @@ extern "C" int pov_decode_corpus_s16(pov_ctx* ctx, uint32_t n_files, const uint8
                                      pov_pcm_sink_s16 sink, void* user, uint64_t* frames_out, uint64_t* total_values_out, int64_t* sum_out) try {
 	CorpusOut fmt;
 	fmt.s16 = true; fmt.sink16 = sink; fmt.user = user; fmt.sum16 = sum_out;
+	return decode_corpus(ctx, n_files, data, len, host_threads, fmt, frames_out, total_values_out);
+} POV_NOTHROW_END(ctx)
+
+int pov_check_pcm_dev(pov_ctx* ctx, const void* p, size_t align, const char* fn);      // api.cu
+
+// Everything about the caller's regions that can be checked before a launch: pov_decode_corpus_device writes nothing otherwise.
+static int validate_device_pcm(pov_ctx* ctx, const pov_device_pcm* o) {
+	const char* fn = "pov_decode_corpus_device";
+	if(!o) return pov_fail(ctx, POV_ERR_ARG, "%s: null output description", fn);
+	if((o->pcm_layout & ~POV_PCM_S16) != POV_PCM_PLANAR) return pov_fail(ctx, POV_ERR_ARG, "%s: pcm_layout 0x%x: only POV_PCM_PLANAR, optionally | POV_PCM_S16", fn, o->pcm_layout);
+	const uint32_t n = o->n_streams;
+	if(n == 0) return POV_OK;
+	if(!o->stream_base || !o->channel_stride || !o->file || !o->channels || !o->frames) return pov_fail(ctx, POV_ERR_ARG, "%s: null table arrays", fn);
+	int rc = pov_check_pcm_dev(ctx, o->pcm_dev, pcm_elem_bytes(o->pcm_layout), fn);
+	if(rc) return rc;
+	if(o->capacity > SIZE_MAX / pcm_elem_bytes(o->pcm_layout)) return pov_fail(ctx, POV_ERR_ARG, "%s: capacity of %llu samples does not fit the address space", fn, (unsigned long long) o->capacity);
+	std::vector<uint32_t> order(n);
+	for(uint32_t i = 0; i < n; ++i) {
+		const uint64_t base = o->stream_base[i], stride = o->channel_stride[i], C = o->channels[i];
+		if(C == 0 || C > POV_MAX_CHANNELS) return pov_fail(ctx, POV_ERR_ARG, "%s: stream %u: %llu channels", fn, i, (unsigned long long) C);
+		if(stride < o->frames[i]) return pov_fail(ctx, POV_ERR_ARG, "%s: stream %u: channel stride %llu < %llu frames", fn, i, (unsigned long long) stride, (unsigned long long) o->frames[i]);
+		if(base > o->capacity || stride > (o->capacity - base) / C)          // (subtraction form: nothing may wrap)
+			return pov_fail(ctx, POV_ERR_ARG, "%s: stream %u: region [%llu, +%llu x %llu) exceeds the capacity of %llu samples", fn, i,
+			                (unsigned long long) base, (unsigned long long) C, (unsigned long long) stride, (unsigned long long) o->capacity);
+		order[i] = i;
+	}
+	std::sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return o->stream_base[a] < o->stream_base[b]; });
+	uint64_t end = 0;                                  // end of the regions before, in base order (empty regions overlap nothing)
+	uint32_t last = 0;
+	for(uint32_t b : order) {
+		if(o->channel_stride[b] == 0) continue;
+		if(o->stream_base[b] < end) return pov_fail(ctx, POV_ERR_ARG, "%s: the regions of streams %u and %u overlap", fn, last, b);
+		const uint64_t e = o->stream_base[b] + o->channels[b] * o->channel_stride[b];
+		if(e > end) { end = e; last = b; }
+	}
+	return POV_OK;
+}
+
+extern "C" int pov_decode_corpus_device(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* data, const size_t* len, uint32_t host_threads,
+                                        const pov_device_pcm* out, uint64_t* frames_out, uint64_t* total_values_out) try {
+	if(!ctx) return POV_ERR_ARG;
+	cudaSetDevice(ctx->device);
+	const int rc = validate_device_pcm(ctx, out);
+	if(rc) return rc;
+	CorpusOut fmt;
+	fmt.s16 = (out->pcm_layout & POV_PCM_S16) != 0; fmt.dev = out;
 	return decode_corpus(ctx, n_files, data, len, host_threads, fmt, frames_out, total_values_out);
 } POV_NOTHROW_END(ctx)
 
@@ -455,6 +579,15 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 	cs.max_bufs = std::max(cs.max_bufs, max_ready + host_threads + CorpusState::kSlots + 1);       // queued + being filled + in flight + one spare
 	for(auto& sl : cs.slot)
 		if(cudaMemsetAsync(sl.d_sum, 0, 8, sl.ctx->stream) != cudaSuccess) return pov_fail(ctx, POV_ERR_CUDA, "pov_decode_corpus: cudaMemset failed");
+	if(fmt.dev) {
+		// device output: no PCM write may start before the work the caller has queued on its stream (e.g. a fill of the tensor)
+		cudaEvent_t ev = nullptr;
+		cudaError_t e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+		if(e == cudaSuccess) e = cudaEventRecord(ev, (cudaStream_t) fmt.dev->cuda_stream);
+		for(auto& sl : cs.slot) if(e == cudaSuccess) e = cudaStreamWaitEvent(sl.ctx->stream, ev, 0);
+		if(ev) cudaEventDestroy(ev);
+		if(e != cudaSuccess) return pov_fail(ctx, POV_ERR_CUDA, "pov_decode_corpus_device: ordering after the caller's stream: %s", cudaGetErrorString(e));
+	}
 	uint64_t sibling_launches0 = 0, sibling_h2d0 = 0, sibling_d2h0 = 0;
 	for(pov_ctx* sb : cs.sibling) { sibling_launches0 += sb->launches; sibling_h2d0 += sb->h2d_bytes; sibling_d2h0 += sb->d2h_bytes; }
 
@@ -485,7 +618,7 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 			for(int attempt = 0; attempt < 2; ++attempt) {       // (second round only if a stream cannot be walked on the device)
 			bool mixed = false;
 			hb.clear(); hb.raw = opt.raw_packets;
-			ck->setups.clear(); ck->stream_file.clear(); ck->stream_channels.clear(); ck->frames.assign(ck->n_files, 0);
+			ck->setups.clear(); ck->stream_file.clear(); ck->stream_channels.clear(); ck->stream_frames.clear(); ck->frames.assign(ck->n_files, 0);
 			for(uint32_t i = 0; i < ck->n_files && ck->error.empty(); ++i) {
 				ParseError err;
 				file.clear();
@@ -502,6 +635,7 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 					ck->frames[i] += st.frames;
 					ck->stream_file.push_back(ck->first_file + i);
 					ck->stream_channels.push_back(st.setup.channels);
+					ck->stream_frames.push_back(st.frames);
 					if(k == ck->setups.size()) {
 						st.packets.clear(); st.ys.clear(); st.payload.clear();
 						ck->setups.push_back(std::move(st));
@@ -561,6 +695,7 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 	for(uint32_t t = 0; t < host_threads; ++t) pool.emplace_back(worker);
 
 	uint64_t total = 0;
+	uint64_t dev_stream = 0;                             // device output: index of the next stream-table record
 	double h_sum = 0;
 	int64_t h_sum16 = 0;
 	// Two batch slots: while the GPU transforms chunk i and copies its PCM and status words to pinned host memory, the
@@ -629,6 +764,26 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 		if(timeline) tl_host[4 * ci] = t0 - t_begin;
 		if(!ck->error.empty()) { rc = pov_fail(ctx, POV_ERR_STREAM, "%s", ck->error.c_str()); cs.release(ck->buf); break; }
 		if(frames_out) for(uint32_t i = 0; i < ck->n_files; ++i) frames_out[ck->first_file + i] = ck->frames[i];
+		if(fmt.dev) {
+			// each parsed stream against the caller's record at its index, then to the caller's region (the kernels address planar
+			// PCM as pcm_base + c * pcm_frames + f, so pcm_frames is the channel stride)
+			const pov_device_pcm& o = *fmt.dev;
+			for(size_t i = 0; i < ck->stream_file.size() && rc == POV_OK; ++i, ++dev_stream) {
+				const uint64_t k = dev_stream;
+				if(k >= o.n_streams)
+					rc = pov_fail(ctx, POV_ERR_ARG, "file %u: pov_decode_corpus_device: more logical streams than the %u records of the stream table",
+					              ck->stream_file[i], o.n_streams);
+				else if(o.file[k] != ck->stream_file[i] || o.channels[k] != ck->stream_channels[i] || o.frames[k] != ck->stream_frames[i])
+					rc = pov_fail(ctx, POV_ERR_ARG, "file %u: pov_decode_corpus_device: stream %llu is (file %u, %u channels, %llu frames), the table says "
+					              "(file %u, %u channels, %llu frames)", ck->stream_file[i], (unsigned long long) k, ck->stream_file[i], ck->stream_channels[i],
+					              (unsigned long long) ck->stream_frames[i], o.file[k], o.channels[k], (unsigned long long) o.frames[k]);
+				else if(ck->view.n_packets) {
+					ck->streams[i].pcm_base = o.stream_base[k];
+					ck->streams[i].pcm_frames = o.channel_stride[k];
+				}
+			}
+			if(rc) { cs.release(ck->buf); break; }
+		}
 		if(ck->view.n_packets == 0) { cs.release(ck->buf); continue; }
 		Slot& sl = cs.slot[ci % CorpusState::kSlots];
 		pov_ctx* cx = sl.ctx;
@@ -643,12 +798,13 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 		if(rc) { cs.release(ck->buf); break; }
 		t_retire += now() - t0; t0 = now();
 		if(timeline) tl_host[4 * ci + 1] = t0 - t_begin;
-		const pov_batch b = ck->view;
-		const uint64_t pcm_floats = b.pcm_floats;
+		pov_batch b = ck->view;
+		const uint64_t pcm_floats = b.pcm_floats;          // samples the chunk yields
+		if(fmt.dev) b.pcm_floats = fmt.dev->capacity;
 		const uint32_t n_packets = b.n_packets;
 		if(timing) cudaEventRecord(sl.t_begin, cx->stream);
 		if(timeline) cudaEventRecord(tl[4 * ci], cx->stream);
-		rc = pov_batch_upload(cx, &b, &sl.h);
+		rc = fmt.dev ? pov_batch_upload_into(cx, &b, fmt.dev->pcm_dev, &sl.h) : pov_batch_upload(cx, &b, &sl.h);
 		if(timeline) cudaEventRecord(tl[4 * ci + 1], cx->stream);      // pinned sources: the copies are queued, the chunk stays alive until retire()
 		sl.in_flight = std::move(ck);
 		sl.busy = true;                            // from here on retire() has to wait for the stream before the buffer is reused
@@ -660,7 +816,7 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 		t_run += now() - t0; t0 = now();
 		if(rc && cx != ctx) pov_fail(ctx, rc, "%s", pov_last_error(cx));
 		if(!rc) {
-			const size_t need = pcm_floats * esz;
+			const size_t need = fmt.dev ? 0 : pcm_floats * esz;
 			if(need > sl.pinned_cap) {
 				if(sl.pinned) cudaFreeHost(sl.pinned);
 				sl.pinned = nullptr;
@@ -674,14 +830,16 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 				sl.status_cap = sneed + sneed / 4;
 				if(cudaMallocHost((void**) &sl.status, sl.status_cap) != cudaSuccess) { sl.status_cap = 0; rc = pov_fail(ctx, POV_ERR_CUDA, "cudaMallocHost failed"); break; }
 			}
-			cudaError_t e = pov_checksum_launch(pov_batch_pcm_dev(sl.h), fmt.s16, pcm_floats, sl.d_sum, cx->stream, &cx->launches);
-			if(e != cudaSuccess) { rc = pov_fail(ctx, POV_ERR_CUDA, "checksum kernel: %s", cudaGetErrorString(e)); break; }
+			if(!fmt.dev) {
+				cudaError_t e = pov_checksum_launch(pov_batch_pcm_dev(sl.h), fmt.s16, pcm_floats, sl.d_sum, cx->stream, &cx->launches);
+				if(e != cudaSuccess) { rc = pov_fail(ctx, POV_ERR_CUDA, "checksum kernel: %s", cudaGetErrorString(e)); break; }
+			}
 			if(timing) cudaEventRecord(sl.t_kernels, cx->stream);
 			if(timeline) cudaEventRecord(tl[4 * ci + 2], cx->stream);
-			// delivery of the PCM and the status words to the host, on the slot's copy-out stream: the next chunk's copy-in and
-			// kernels on cx->stream are then not queued behind the other slots' copy-outs (they only wait for this one)
-			cudaError_t ce = pov_copy_out_async(cx, sl.pinned, pov_batch_pcm_dev(sl.h), need, true, false);
-			if(ce == cudaSuccess) ce = pov_copy_out_async(cx, sl.status, sl.h->d_status.ptr, sneed, false, true);
+			// delivery of the PCM (not for device output) and the status words to the host, on the slot's copy-out stream: the next
+			// chunk's copy-in and kernels on cx->stream are then not queued behind the other slots' copy-outs (they only wait for this one)
+			cudaError_t ce = need ? pov_copy_out_async(cx, sl.pinned, pov_batch_pcm_dev(sl.h), need, true, false) : cudaSuccess;
+			if(ce == cudaSuccess) ce = pov_copy_out_async(cx, sl.status, sl.h->d_status.ptr, sneed, need == 0, true);
 			if(ce != cudaSuccess) rc = pov_fail(ctx, POV_ERR_CUDA, "pov_decode_corpus: copy-out failed: %s", cudaGetErrorString(ce));
 			if(timing) cudaEventRecord(sl.t_end, cx->out_stream);
 			if(timeline) cudaEventRecord(tl[4 * ci + 3], cx->out_stream);
@@ -696,6 +854,9 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 		const int r2 = retire(cs.slot[(n_chunks + k) % CorpusState::kSlots]);
 		if(rc == POV_OK) rc = r2;
 	}
+	if(rc == POV_OK && fmt.dev && dev_stream != fmt.dev->n_streams)
+		rc = pov_fail(ctx, POV_ERR_ARG, "pov_decode_corpus_device: the corpus has %llu logical streams, the stream table %u",
+		              (unsigned long long) dev_stream, fmt.dev->n_streams);
 	if(timing)
 		fprintf(stderr, "pov_decode_corpus: %u chunks in %.3f s on the calling thread: wait for parsed chunks %.3f, "
 		        "setup ids + wait for the slot %.3f, validate+queue upload %.3f, launch %.3f, fetch/issue %.3f; on the streams (sum over chunks): "
@@ -721,7 +882,7 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 	for(auto& sl : cs.slot) {
 		double part = 0;
 		int64_t part16 = 0;
-		if(rc == POV_OK &&
+		if(rc == POV_OK && !fmt.dev &&
 		   (cudaMemcpyAsync(fmt.s16 ? (void*) &part16 : (void*) &part, sl.d_sum, 8, cudaMemcpyDeviceToHost, sl.ctx->stream) != cudaSuccess ||
 		    cudaStreamSynchronize(sl.ctx->stream) != cudaSuccess))
 			rc = pov_fail(ctx, POV_ERR_CUDA, "pov_decode_corpus: checksum copy failed");

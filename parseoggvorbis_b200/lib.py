@@ -7,7 +7,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
-from typing import Optional
+from typing import NamedTuple, Optional
 
 import numpy as np
 
@@ -26,6 +26,7 @@ SYMBOLS = [
     "pov_ogg_vorbis_decode_memory", "pov_decoded_free", "pov_decode_corpus", "pov_decode_corpus_pcm", "pov_ogg_vorbis_full_read_from_memory",
     "pov_ogg_vorbis_decode_memory_s16", "pov_decoded_s16_free", "pov_decode_corpus_s16",
     "pov_ogg_parse_memory", "pov_parsed_stream_count", "pov_parsed_get", "pov_parsed_free",
+    "pov_batch_upload_into", "pov_corpus_streams", "pov_corpus_streams_free", "pov_decode_corpus_device",
 ]
 
 
@@ -111,8 +112,76 @@ def load() -> C.CDLL:
     L.pov_parsed_get.argtypes = [vp, u32, C.POINTER(abi.pov_setup), C.POINTER(abi.pov_batch)]
     L.pov_parsed_free.argtypes = [vp]
     L.pov_parsed_free.restype = None
+    L.pov_batch_upload_into.argtypes = [vp, C.POINTER(abi.pov_batch), vp, C.POINTER(vp)]
+    L.pov_corpus_streams.argtypes = [u32, C.POINTER(C.c_char_p), C.POINTER(C.c_size_t), u32, u32,
+                                     C.POINTER(C.POINTER(abi.pov_stream_info)), C.POINTER(u64), C.POINTER(C.c_char_p)]
+    L.pov_corpus_streams_free.argtypes = [C.POINTER(abi.pov_stream_info)]
+    L.pov_corpus_streams_free.restype = None
+    L.pov_decode_corpus_device.argtypes = [vp, u32, C.POINTER(C.c_char_p), C.POINTER(C.c_size_t), u32, C.POINTER(abi.pov_device_pcm),
+                                           C.POINTER(u64), C.POINTER(u64)]
     _LIB = L
     return L
+
+
+class StreamTable(NamedTuple):
+    """One entry per logical stream of a corpus, in decode order (pov_corpus_streams)."""
+    file: np.ndarray           # uint32, index into the corpus
+    channels: np.ndarray       # uint32
+    sample_rate: np.ndarray    # uint32
+    frames: np.ndarray         # uint64, frames per channel the decode yields
+
+    def __len__(self):
+        return len(self.file)
+
+
+_STREAM_INFO_DTYPE = np.dtype([("file", "<u4"), ("channels", "<u4"), ("sample_rate", "<u4"), ("reserved", "<u4"), ("frames", "<u8")])
+assert _STREAM_INFO_DTYPE.itemsize == C.sizeof(abi.pov_stream_info)
+
+
+def corpus_streams(files, allow_spanning: bool = False, host_threads: int = 0) -> StreamTable:
+    """The stream table of a corpus without a GPU: the corpus decode's own parse with the packets discarded, so `frames` is
+    what decode_corpus / decode_corpus_device produce. A framing or header error raises PovError with the corpus decode's
+    text ("file k: check failed: ...")."""
+    L = load()
+    n = len(files)
+    arr = (C.c_char_p * n)(*files)
+    lens = (C.c_size_t * n)(*[len(f) for f in files])
+    out = C.POINTER(abi.pov_stream_info)()
+    count = C.c_uint64(0)
+    err = C.c_char_p(None)
+    rc = L.pov_corpus_streams(n, arr, lens, abi.POV_PARSE_ALLOW_SPANNING if allow_spanning else 0, host_threads, C.byref(out),
+                              C.byref(count), C.byref(err))
+    if rc != 0:
+        raise PovError(rc, (err.value or b"?").decode())
+    try:
+        m = int(count.value)
+        rec = np.ctypeslib.as_array(C.cast(out, C.POINTER(C.c_uint8)), shape=(m * C.sizeof(abi.pov_stream_info),)).view(
+            _STREAM_INFO_DTYPE) if m else np.zeros(0, _STREAM_INFO_DTYPE)
+        return StreamTable(rec["file"].copy(), rec["channels"].copy(), rec["sample_rate"].copy(), rec["frames"].copy())
+    finally:
+        L.pov_corpus_streams_free(out)
+
+
+def _round4(x):
+    return (np.asarray(x, np.uint64) + np.uint64(3)) // np.uint64(4) * np.uint64(4)
+
+
+class DeviceCorpus(NamedTuple):
+    """What decode_corpus_device returns: the PCM tensor, the stream table and where each stream lives in the tensor."""
+    pcm: "object"              # torch tensor on the context's device
+    table: StreamTable
+    base: np.ndarray           # uint64 [streams], sample index of channel 0, frame 0 (in pcm's flat storage)
+    stride: np.ndarray         # uint64 [streams], samples between channels
+    frames_per_file: np.ndarray
+    total_values: int
+
+    def stream(self, i: int):
+        """(channels, frames) view of stream i."""
+        c, f = int(self.table.channels[i]), int(self.table.frames[i])
+        if self.pcm.dim() == 3:
+            return self.pcm[i, :c, :f]
+        b, s = int(self.base[i]), int(self.stride[i])
+        return self.pcm[b:b + c * s].view(c, s)[:, :f]
 
 
 class ParsedOgg:
@@ -158,6 +227,7 @@ class BatchHandle:
         self.ctx = ctx
         self.batch = batch          # keeps the host arrays alive
         self.h = C.c_void_p(None)
+        self.pcm_out = None         # upload(pcm_out=...): the caller's tensor the kernels write
 
     def free(self):
         if self.h:
@@ -182,6 +252,8 @@ class SynthContext:
         if rc != 0:
             raise PovError(rc, (err.value or b"?").decode())
         self._setups = []
+        self.device = device
+        self._spanning = int(os.environ.get("POV_ALLOW_SPANNING", "0") or 0) != 0     # the context's default (api.cu)
 
     def close(self):
         if self.ctx:
@@ -208,6 +280,7 @@ class SynthContext:
 
     def set_page_spanning(self, on: bool):
         self.L.pov_ctx_set_page_spanning(self.ctx, 1 if on else 0)
+        self._spanning = bool(on)
 
     def set_device_entropy(self, on: bool):
         self.L.pov_ctx_set_device_entropy(self.ctx, 1 if on else 0)
@@ -231,15 +304,52 @@ class SynthContext:
                                                 out.ctypes.data_as(C.POINTER(C.c_float)), n))
         return out
 
-    def upload(self, batch: abi.Batch, reuse: Optional[BatchHandle] = None) -> BatchHandle:
+    def _pcm_tensor(self, t, s16: bool, samples: int, what: str):
+        """Checks of a caller's PCM tensor: contiguous, on this context's GPU, dtype of the format, room for `samples`."""
+        import torch
+        want = torch.int16 if s16 else torch.float32
+        if not isinstance(t, torch.Tensor) or t.device != torch.device("cuda", self.device) or not t.is_contiguous():
+            raise PovError(abi.POV_ERR_ARG, "%s: a contiguous tensor on cuda:%d is needed" % (what, self.device))
+        if t.dtype != want:
+            raise PovError(abi.POV_ERR_ARG, "%s: dtype %s, the format needs %s" % (what, t.dtype, want))
+        if t.numel() < samples:
+            raise PovError(abi.POV_ERR_ARG, "%s: %d samples, %d needed" % (what, t.numel(), samples))
+
+    def _ctx_stream(self):
+        import torch
+        return torch.cuda.ExternalStream(self.stream_ptr, device=torch.device("cuda", self.device))
+
+    def upload(self, batch: abi.Batch, reuse: Optional[BatchHandle] = None, pcm_out=None) -> BatchHandle:
+        """pcm_out: a contiguous CUDA tensor on this context's device (float32, or int16 for a POV_PCM_S16 batch) with room for
+        batch.pcm_floats samples; the kernels then write the PCM there (pov_batch_upload_into) instead of the handle's arena.
+        The context's stream is ordered after the work queued on torch's current stream, and run() / run_staged() make the
+        current stream wait for the kernels, so the tensor is used in plain stream order on both sides."""
         bh = reuse if reuse is not None else BatchHandle(self, batch)
         bh.batch = batch
         cb = batch.to_c()
-        self._check(self.L.pov_batch_upload(self.ctx, C.byref(cb), C.byref(bh.h)))
+        if pcm_out is None:
+            bh.pcm_out = None
+            self._check(self.L.pov_batch_upload(self.ctx, C.byref(cb), C.byref(bh.h)))
+            return bh
+        import torch
+        self._pcm_tensor(pcm_out, bool(batch.pcm_layout & abi.POV_PCM_S16), int(batch.pcm_floats), "upload(pcm_out)")
+        ev = torch.cuda.Event()
+        ev.record(torch.cuda.current_stream(self.device))
+        self._ctx_stream().wait_event(ev)
+        self._check(self.L.pov_batch_upload_into(self.ctx, C.byref(cb), C.c_void_p(pcm_out.data_ptr()), C.byref(bh.h)))
+        bh.pcm_out = pcm_out
         return bh
+
+    def _after_run(self, bh: BatchHandle):
+        if bh.pcm_out is not None:          # torch's current stream waits for the kernels that write the caller's tensor
+            import torch
+            ev = torch.cuda.Event()
+            ev.record(self._ctx_stream())
+            torch.cuda.current_stream(self.device).wait_event(ev)
 
     def run(self, bh: BatchHandle):
         self._check(self.L.pov_batch_run(self.ctx, bh.h))
+        self._after_run(bh)
 
     def kernel_name(self, bh: BatchHandle) -> str:
         """Kernel that run() launches for this batch (k_warp_synth / k_fused_synth / staged)."""
@@ -247,6 +357,7 @@ class SynthContext:
 
     def run_staged(self, bh: BatchHandle):
         self._check(self.L.pov_batch_run_staged(self.ctx, bh.h))
+        self._after_run(bh)
 
     def sync(self, bh: BatchHandle):
         self._check(self.L.pov_batch_sync(self.ctx, bh.h))
@@ -401,3 +512,65 @@ class SynthContext:
         self._check(self.L.pov_decode_corpus_s16(self.ctx, n, arr, lens, host_threads, _sink, None,
                                                  frames.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(total), C.byref(chk)))
         return frames, int(total.value), int(chk.value)
+
+    def decode_corpus_into(self, files, pcm, table: StreamTable, base, stride, s16: bool = False, host_threads: int = 0):
+        """pov_decode_corpus_device into a tensor the caller laid out: stream i of `table`, channel c, frame f lands at flat
+        sample index base[i] + c * stride[i] + f of `pcm` (contiguous, on this context's GPU, float32 or int16 with s16).
+        Nothing else of `pcm` is written. No PCM write starts before the work queued on torch's current stream, and the call
+        returns when the PCM is complete. Returns (frames per file, total PCM values)."""
+        import torch
+        n, m = len(files), len(table)
+        base = np.ascontiguousarray(base, np.uint64)
+        stride = np.ascontiguousarray(stride, np.uint64)
+        if base.shape != (m,) or stride.shape != (m,):
+            raise PovError(abi.POV_ERR_ARG, "decode_corpus_into: base and stride need one entry per stream-table record")
+        self._pcm_tensor(pcm, s16, 0, "decode_corpus_into(pcm)")
+        file = np.ascontiguousarray(table.file, np.uint32)
+        channels = np.ascontiguousarray(table.channels, np.uint32)
+        tframes = np.ascontiguousarray(table.frames, np.uint64)
+        o = abi.pov_device_pcm()
+        o.pcm_layout = abi.POV_PCM_PLANAR | (abi.POV_PCM_S16 if s16 else 0)
+        o.n_streams = m
+        o.pcm_dev = pcm.data_ptr() or None
+        o.capacity = pcm.numel()
+        o.stream_base = base.ctypes.data_as(C.POINTER(C.c_uint64))
+        o.channel_stride = stride.ctypes.data_as(C.POINTER(C.c_uint64))
+        o.file = file.ctypes.data_as(C.POINTER(C.c_uint32))
+        o.channels = channels.ctypes.data_as(C.POINTER(C.c_uint32))
+        o.frames = tframes.ctypes.data_as(C.POINTER(C.c_uint64))
+        o.cuda_stream = torch.cuda.current_stream(self.device).cuda_stream or None
+        arr = (C.c_char_p * n)(*files)
+        lens = (C.c_size_t * n)(*[len(f) for f in files])
+        frames = np.zeros(n, np.uint64)
+        total = C.c_uint64(0)
+        self._check(self.L.pov_decode_corpus_device(self.ctx, n, arr, lens, host_threads, C.byref(o),
+                                                    frames.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(total)))
+        return frames, int(total.value)
+
+    def decode_corpus_device(self, files, layout: str = "padded", s16: bool = False, host_threads: int = 0) -> DeviceCorpus:
+        """Decode a corpus straight into a new torch tensor on this context's GPU; only compressed packets go to the device
+        and only status words come back. layout "padded": (streams, max channels, T) zeros, T = the longest stream rounded
+        up to 4; "packed": one flat tensor, each stream's channels `frames rounded up to 4` apart, back to back. Padding
+        stays 0. s16: int16 samples (the POV_PCM_S16 conversion). The stream table is parsed with this context's page-spanning
+        setting."""
+        import torch
+        table = corpus_streams(files, allow_spanning=self._spanning, host_threads=host_threads)
+        m = len(table)
+        ch = table.channels.astype(np.uint64)
+        dtype = torch.int16 if s16 else torch.float32
+        dev = torch.device("cuda", self.device)
+        if layout == "padded":
+            T = int(_round4(table.frames.max())) if m else 0
+            maxc = int(ch.max()) if m else 0
+            pcm = torch.zeros((m, maxc, T), dtype=dtype, device=dev)
+            stride = np.full(m, T, np.uint64)
+            base = np.arange(m, dtype=np.uint64) * np.uint64(maxc * T)
+        elif layout == "packed":
+            stride = _round4(table.frames)
+            sizes = ch * stride
+            base = (np.cumsum(sizes) - sizes).astype(np.uint64)
+            pcm = torch.zeros(int(sizes.sum()), dtype=dtype, device=dev)
+        else:
+            raise ValueError("layout must be 'padded' or 'packed'")
+        frames, total = self.decode_corpus_into(files, pcm, table, base, stride, s16=s16, host_threads=host_threads)
+        return DeviceCorpus(pcm, table, base, stride, frames, total)
