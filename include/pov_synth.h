@@ -409,6 +409,56 @@ typedef struct pov_device_pcm {
 int  pov_decode_corpus_device(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* data, const size_t* len, uint32_t host_threads,
                               const pov_device_pcm* out, uint64_t* frames_out, uint64_t* total_values_out);
 
+/* Resampling and mono downmix of the device corpus decode (pov_decode_corpus_device_resampled).
+ * A stream at rate `in` resampled to rate `out`: g = gcd(in, out), L = out / g (up), M = in / g (down).
+ * - L = M = 1: the output is a copy of the decoded samples (no filter).
+ * - Otherwise R = max(L, M), hl = 10 R (half_len), N = 2 hl + 1 taps, the design of scipy.signal.resample_poly's default:
+ *   h[n] = fc sinc(fc (n - hl)) I0(5 sqrt(1 - ((n - hl) / hl)^2)) / I0(5) with fc = 1 / R, normalised to unit sum, times L;
+ *   computed in float64 on the host and rounded once to float32.
+ * - Output frames: ceil(frames L / M). Output sample y[j] = sum_i x[i] h[j M + hl - i L] over taps inside [0, N) and inputs inside
+ *   [0, frames), zero outside: scipy.signal.resample_poly(x, out, in) with padtype='constant'. The kernel evaluates it in
+ *   polyphase form, phase (j M + hl) mod L with inputs x[floor((j M + hl) / L) - k] and taps h[phase + k L], k ascending from 0,
+ *   one fmaf each, from 0.0f; the result does not depend on chunks, tiles or layouts.
+ * - POV_RESAMPLE_MONO: the channels are averaged first, s = x0; s = s + x1 (rounded); ...; m = s * (1.0f / C) (rounded), then
+ *   resampled as one channel. Without it every channel is resampled on its own.
+ * - int16 output (POV_PCM_S16) is the POV_PCM_S16 rule applied to the float32 y at the store; the filter can overshoot full
+ *   scale, and such samples saturate.
+ * - Supported: max(L, M) <= POV_RESAMPLE_MAX_PHASES (tables of up to 40961 taps). Larger ratios (2048 -> 2049 Hz, 44056 -> 48000
+ *   Hz) are POV_ERR_UNSUPPORTED. */
+#define POV_RESAMPLE_MONO 1u
+#define POV_RESAMPLE_MAX_PHASES 2048u
+typedef struct pov_resample {
+	uint32_t out_rate;              /* Hz; 0 = each stream keeps its rate (L = M = 1: downmix only, or a plain copy) */
+	uint32_t flags;                 /* POV_RESAMPLE_MONO */
+	const uint32_t* sample_rate;    /* [n_streams] from the stream table: checked against what is parsed, like channels / frames */
+} pov_resample;
+
+/* Host only (no GPU): the reduced ratio (*up = L, *down = M), *half_len = hl and, when `taps` is not NULL, the N = 2 hl + 1
+ * float32 taps h[0..N) of the in_rate -> out_rate filter above. L = M = 1 (out_rate 0 or equal to in_rate) is a copy:
+ * *half_len = 0 and no taps are written. taps_cap < N with taps != NULL, or in_rate = 0, is POV_ERR_ARG; max(L, M) past
+ * POV_RESAMPLE_MAX_PHASES is POV_ERR_UNSUPPORTED (the ratio is still reported). */
+int  pov_resample_filter(uint32_t in_rate, uint32_t out_rate, uint32_t* up, uint32_t* down, uint32_t* half_len,
+                         float* taps, uint32_t taps_cap);
+
+/* pov_decode_corpus_device with every stream downmixed (POV_RESAMPLE_MONO) and/or resampled to rs->out_rate on the device, as
+ * defined above, before it lands in the caller's memory (float32, or int16 with POV_PCM_S16). The synthesis writes each chunk
+ * into a float32 device arena of the context (every channel 4-aligned, so the decoded samples equal what
+ * pov_decode_corpus_device writes into 4-aligned regions), and one resample kernel per chunk reads it and writes the regions.
+ * - out->file, channels and frames are the native stream table, checked against what is parsed as in pov_decode_corpus_device;
+ *   rs->sample_rate is checked the same way (a mismatch is POV_ERR_ARG naming the file).
+ * - Stream i owns out_channels x channel_stride[i] samples from stream_base[i], out_channels = 1 with POV_RESAMPLE_MONO and
+ *   channels[i] otherwise; channel_stride[i] must be at least its output frames. Exactly
+ *   [base + c * stride, base + c * stride + output frames) is written for c < out_channels.
+ * - Before anything is launched: the checks of pov_decode_corpus_device on these output regions, a null `rs`, a null
+ *   rs->sample_rate with n_streams > 0, unknown flags (POV_ERR_ARG), and a ratio past POV_RESAMPLE_MAX_PHASES for any record
+ *   (POV_ERR_UNSUPPORTED naming the stream, both rates and the phase count).
+ * - frames_out[n_files] (may be NULL) are the native frames per file; *total_values_out counts the samples written.
+ * Device memory: besides the caller's regions, up to four float32 chunk arenas stay allocated on the context (about 190 MB
+ * each for chunks of 256 stereo files of 2 s at 44.1 kHz) and a filter table per ratio used (at most 160 KB each). */
+int  pov_decode_corpus_device_resampled(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* data, const size_t* len,
+                                        uint32_t host_threads, const pov_device_pcm* out, const pov_resample* rs,
+                                        uint64_t* frames_out, uint64_t* total_values_out);
+
 /* Host-only front-end (no GPU needed): parse a whole Ogg/Vorbis file into descriptor batches, one per logical stream
  * (Ogg framing hpp:51-102,1433-1484; headers hpp:1283-1373; per-packet entropy decode hpp:498-517, 711-757). The
  * setup/batch returned by pov_parsed_get point into memory owned by the handle (POV_INPUT_ENTRIES, setup_id 0). */

@@ -26,6 +26,8 @@ POV_INPUT_DENSE, POV_INPUT_ENTRIES, POV_INPUT_PACKETS = 0, 1, 2
 POV_PCM_PLANAR, POV_PCM_INTERLEAVED = 0, 1
 POV_PCM_S16 = 0x100          # OR-ed into pcm_layout: the kernels store int16 PCM (see include/pov_synth.h)
 POV_PARSE_RAW_PACKETS, POV_PARSE_ALLOW_SPANNING = 1, 2     # flags of pov_ogg_parse_memory_ex / pov_corpus_streams
+POV_RESAMPLE_MONO = 1        # pov_resample.flags: average the channels before resampling
+POV_RESAMPLE_MAX_PHASES = 2048   # largest max(L, M) of a supported resampling ratio
 
 (POV_STAGE_FINAL_YS, POV_STAGE_STEP2_FLAG, POV_STAGE_FLOOR, POV_STAGE_FLOOR_OUTPUTS,
  POV_STAGE_AFTER_RESIDUE, POV_STAGE_AFTER_ENVELOPE, POV_STAGE_PCM_AFTER_MDCT) = range(7)
@@ -120,6 +122,11 @@ class pov_device_pcm(C.Structure):
                 ("stream_base", C.POINTER(C.c_uint64)), ("channel_stride", C.POINTER(C.c_uint64)),
                 ("file", C.POINTER(C.c_uint32)), ("channels", C.POINTER(C.c_uint32)), ("frames", C.POINTER(C.c_uint64)),
                 ("cuda_stream", C.c_void_p)]
+
+
+class pov_resample(C.Structure):
+    """Resampling / downmix of pov_decode_corpus_device_resampled."""
+    _fields_ = [("out_rate", C.c_uint32), ("flags", C.c_uint32), ("sample_rate", C.POINTER(C.c_uint32))]
 
 
 # numpy dtypes with the same layout as pov_stream / pov_packet (so big batches are built vectorised)

@@ -22,6 +22,7 @@
 #include "api_internal.h"
 #include "debug_dump.h"
 #include "kernels.h"
+#include "resample.h"
 #include "vorbis_parse.h"
 
 using namespace pov;
@@ -365,6 +366,7 @@ struct Chunk {
 	std::vector<uint64_t> frames;              // per file
 	std::vector<uint32_t> stream_file, stream_channels;   // per stream of the batch: file index (corpus-wide), channel count
 	std::vector<uint64_t> stream_frames;       // per stream of the batch
+	std::vector<uint32_t> stream_rate;         // per stream of the batch: sample rate
 	std::string error;
 };
 
@@ -385,6 +387,8 @@ struct CorpusState {
 		cudaEvent_t done = nullptr;
 		cudaEvent_t t_begin = nullptr, t_kernels = nullptr, t_end = nullptr;   // POV_CORPUS_TIMING only
 		uint32_t n_packets = 0, first_file = 0;
+		ResampleDesc* rs_host = nullptr; size_t rs_cap = 0;  // resampled output: the chunk's descriptors (pinned source of their upload)
+		DevBuf rs_dev;
 		std::unique_ptr<Chunk> in_flight;      // its pinned buffer is the source of copies that may still be running
 		bool busy = false;
 	} slot[kSlots];
@@ -392,6 +396,8 @@ struct CorpusState {
 	std::condition_variable pcv;
 	std::vector<PinnedBuf> free_bufs;
 	uint32_t n_bufs = 0, max_bufs = 0;
+	struct Filter { float* taps = nullptr; uint32_t K = 0, hl = 0; };
+	std::map<std::pair<uint32_t, uint32_t>, Filter> filters;   // by (L, M): polyphase tables [K][L] on the device, shared by the slots
 
 	PinnedBuf acquire(size_t need, const std::atomic<bool>& stop) {
 		PinnedBuf b;
@@ -429,11 +435,14 @@ struct CorpusState {
 			if(sl.h) pov_batch_free(sl.ctx, sl.h);
 			if(sl.pinned) cudaFreeHost(sl.pinned);
 			if(sl.status) cudaFreeHost(sl.status);
+			if(sl.rs_host) cudaFreeHost(sl.rs_host);
+			sl.rs_dev.release();
 			if(sl.done) cudaEventDestroy(sl.done);
 			if(sl.t_begin) { cudaEventDestroy(sl.t_begin); cudaEventDestroy(sl.t_kernels); cudaEventDestroy(sl.t_end); }
 			if(sl.d_sum) cudaFree(sl.d_sum);
 		}
 		for(auto& b : free_bufs) cudaFreeHost(b.p);
+		for(auto& f : filters) if(f.second.taps) cudaFree(f.second.taps);
 		for(pov_ctx* sb : sibling) if(sb) pov_ctx_destroy(sb);
 	}
 };
@@ -443,10 +452,12 @@ inline size_t align16(size_t x) { return (x + 15) & ~(size_t) 15; }
 }  // namespace
 
 // Output format of a corpus decode: float32 (sink, checksum), int16 (POV_PCM_S16: sink16, sum16), or the caller's device
-// memory (dev: float32 or int16 by dev->pcm_layout; no PCM leaves the device).
+// memory (dev: float32 or int16 by dev->pcm_layout; no PCM leaves the device), optionally resampled / downmixed (rs: the
+// synthesis writes a float32 arena of the slot, the resample kernel the caller's memory).
 struct CorpusOut {
 	bool s16 = false;
 	const pov_device_pcm* dev = nullptr;
+	const pov_resample* rs = nullptr;
 	pov_pcm_sink sink = nullptr;
 	pov_pcm_sink_s16 sink16 = nullptr;
 	void* user = nullptr;
@@ -482,8 +493,8 @@ extern "C" int pov_decode_corpus_s16(pov_ctx* ctx, uint32_t n_files, const uint8
 int pov_check_pcm_dev(pov_ctx* ctx, const void* p, size_t align, const char* fn);      // api.cu
 
 // Everything about the caller's regions that can be checked before a launch: pov_decode_corpus_device writes nothing otherwise.
-static int validate_device_pcm(pov_ctx* ctx, const pov_device_pcm* o) {
-	const char* fn = "pov_decode_corpus_device";
+// Stream i's region holds out_ch[i] channels of out_frames[i] frames (the table's channels and frames without resampling).
+static int validate_device_pcm(pov_ctx* ctx, const pov_device_pcm* o, const uint32_t* out_ch, const uint64_t* out_frames, const char* fn) {
 	if(!o) return pov_fail(ctx, POV_ERR_ARG, "%s: null output description", fn);
 	if((o->pcm_layout & ~POV_PCM_S16) != POV_PCM_PLANAR) return pov_fail(ctx, POV_ERR_ARG, "%s: pcm_layout 0x%x: only POV_PCM_PLANAR, optionally | POV_PCM_S16", fn, o->pcm_layout);
 	const uint32_t n = o->n_streams;
@@ -494,9 +505,9 @@ static int validate_device_pcm(pov_ctx* ctx, const pov_device_pcm* o) {
 	if(o->capacity > SIZE_MAX / pcm_elem_bytes(o->pcm_layout)) return pov_fail(ctx, POV_ERR_ARG, "%s: capacity of %llu samples does not fit the address space", fn, (unsigned long long) o->capacity);
 	std::vector<uint32_t> order(n);
 	for(uint32_t i = 0; i < n; ++i) {
-		const uint64_t base = o->stream_base[i], stride = o->channel_stride[i], C = o->channels[i];
-		if(C == 0 || C > POV_MAX_CHANNELS) return pov_fail(ctx, POV_ERR_ARG, "%s: stream %u: %llu channels", fn, i, (unsigned long long) C);
-		if(stride < o->frames[i]) return pov_fail(ctx, POV_ERR_ARG, "%s: stream %u: channel stride %llu < %llu frames", fn, i, (unsigned long long) stride, (unsigned long long) o->frames[i]);
+		const uint64_t base = o->stream_base[i], stride = o->channel_stride[i], C = out_ch[i];
+		if(o->channels[i] == 0 || o->channels[i] > POV_MAX_CHANNELS) return pov_fail(ctx, POV_ERR_ARG, "%s: stream %u: %u channels", fn, i, o->channels[i]);
+		if(stride < out_frames[i]) return pov_fail(ctx, POV_ERR_ARG, "%s: stream %u: channel stride %llu < %llu frames", fn, i, (unsigned long long) stride, (unsigned long long) out_frames[i]);
 		if(base > o->capacity || stride > (o->capacity - base) / C)          // (subtraction form: nothing may wrap)
 			return pov_fail(ctx, POV_ERR_ARG, "%s: stream %u: region [%llu, +%llu x %llu) exceeds the capacity of %llu samples", fn, i,
 			                (unsigned long long) base, (unsigned long long) C, (unsigned long long) stride, (unsigned long long) o->capacity);
@@ -508,7 +519,7 @@ static int validate_device_pcm(pov_ctx* ctx, const pov_device_pcm* o) {
 	for(uint32_t b : order) {
 		if(o->channel_stride[b] == 0) continue;
 		if(o->stream_base[b] < end) return pov_fail(ctx, POV_ERR_ARG, "%s: the regions of streams %u and %u overlap", fn, last, b);
-		const uint64_t e = o->stream_base[b] + o->channels[b] * o->channel_stride[b];
+		const uint64_t e = o->stream_base[b] + out_ch[b] * o->channel_stride[b];
 		if(e > end) { end = e; last = b; }
 	}
 	return POV_OK;
@@ -518,12 +529,80 @@ extern "C" int pov_decode_corpus_device(pov_ctx* ctx, uint32_t n_files, const ui
                                         const pov_device_pcm* out, uint64_t* frames_out, uint64_t* total_values_out) try {
 	if(!ctx) return POV_ERR_ARG;
 	cudaSetDevice(ctx->device);
-	const int rc = validate_device_pcm(ctx, out);
+	const bool tables = out && out->n_streams && out->channels && out->frames;
+	const int rc = validate_device_pcm(ctx, out, tables ? out->channels : nullptr, tables ? out->frames : nullptr, "pov_decode_corpus_device");
 	if(rc) return rc;
 	CorpusOut fmt;
 	fmt.s16 = (out->pcm_layout & POV_PCM_S16) != 0; fmt.dev = out;
 	return decode_corpus(ctx, n_files, data, len, host_threads, fmt, frames_out, total_values_out);
 } POV_NOTHROW_END(ctx)
+
+// (L, M) of stream i of a resampled decode; the ratio was checked before the decode started
+static void stream_ratio(const pov_resample& rs, uint32_t in_rate, uint32_t* L, uint32_t* M) {
+	uint32_t hl = 0;
+	if(rs.out_rate == 0) { *L = *M = 1; return; }
+	resample_design(in_rate, rs.out_rate, L, M, &hl, nullptr);
+}
+
+extern "C" int pov_decode_corpus_device_resampled(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* data, const size_t* len,
+                                                  uint32_t host_threads, const pov_device_pcm* out, const pov_resample* rs,
+                                                  uint64_t* frames_out, uint64_t* total_values_out) try {
+	if(!ctx) return POV_ERR_ARG;
+	cudaSetDevice(ctx->device);
+	const char* fn = "pov_decode_corpus_device_resampled";
+	if(!out) return pov_fail(ctx, POV_ERR_ARG, "%s: null output description", fn);
+	if(!rs) return pov_fail(ctx, POV_ERR_ARG, "%s: null resample description", fn);
+	if(rs->flags & ~POV_RESAMPLE_MONO) return pov_fail(ctx, POV_ERR_ARG, "%s: flags 0x%x: only POV_RESAMPLE_MONO", fn, rs->flags);
+	const uint32_t n = out->n_streams;
+	if(n && !rs->sample_rate) return pov_fail(ctx, POV_ERR_ARG, "%s: null sample_rate table", fn);
+	const bool tables = n && out->channels && out->frames;
+	std::vector<uint32_t> och(tables ? n : 0);
+	std::vector<uint64_t> ofr(tables ? n : 0);
+	for(uint32_t i = 0; i < n; ++i) {
+		const uint32_t in = rs->sample_rate[i];
+		uint32_t L = 1, M = 1, hl = 0;
+		if(in == 0) return pov_fail(ctx, POV_ERR_ARG, "%s: stream %u: sample rate 0", fn, i);
+		if(rs->out_rate && !resample_design(in, rs->out_rate, &L, &M, &hl, nullptr))
+			return pov_fail(ctx, POV_ERR_UNSUPPORTED, "%s: stream %u: %u Hz -> %u Hz needs %u filter phases (max(L, M) for L = %u, M = %u), "
+			                "past the supported %u", fn, i, in, rs->out_rate, std::max(L, M), L, M, POV_RESAMPLE_MAX_PHASES);
+		if(tables) {
+			och[i] = (rs->flags & POV_RESAMPLE_MONO) ? 1 : out->channels[i];
+			ofr[i] = resample_frames(out->frames[i], L, M);
+		}
+	}
+	const int rc = validate_device_pcm(ctx, out, och.data(), ofr.data(), fn);
+	if(rc) return rc;
+	CorpusOut fmt;
+	fmt.dev = out; fmt.rs = rs;                // the slots' arenas are float32 whatever the output type
+	return decode_corpus(ctx, n_files, data, len, host_threads, fmt, frames_out, total_values_out);
+} POV_NOTHROW_END(ctx)
+
+// The device table of ratio (L, M) in the kernel's order, [K][L] with K = ceil(N / L) and zeros past N; built on the calling
+// thread the first time the ratio appears and kept for the context's lifetime. A copy (L = M = 1) has none.
+static int resample_filter_table(pov_ctx* ctx, CorpusState& cs, uint32_t L, uint32_t M, const float** taps, uint32_t* K, uint32_t* hl) {
+	*taps = nullptr; *K = 0; *hl = 0;
+	if(L == 1 && M == 1) return POV_OK;
+	CorpusState::Filter& f = cs.filters[std::make_pair(L, M)];
+	if(!f.taps) {
+		uint32_t l = 0, m = 0, h = 0;
+		std::vector<float> taps_h;
+		if(!resample_design(M, L, &l, &m, &h, &taps_h)) return pov_fail(ctx, POV_ERR_UNSUPPORTED, "resample ratio %u/%u past the supported phases", L, M);
+		const uint32_t N = (uint32_t) taps_h.size(), k_n = (N + L - 1) / L;
+		std::vector<float> poly((size_t) k_n * L, 0.0f);
+		for(uint32_t k = 0; k < k_n; ++k)
+			for(uint32_t p = 0; p < L && p + k * L < N; ++p) poly[(size_t) k * L + p] = taps_h[p + k * L];
+		cudaError_t e = cudaMalloc((void**) &f.taps, poly.size() * sizeof(float));
+		if(e == cudaSuccess) e = cudaMemcpy(f.taps, poly.data(), poly.size() * sizeof(float), cudaMemcpyHostToDevice);
+		if(e != cudaSuccess) {
+			if(f.taps) cudaFree(f.taps);
+			f.taps = nullptr;
+			return pov_fail(ctx, POV_ERR_CUDA, "resample filter table: %s", cudaGetErrorString(e));
+		}
+		f.K = k_n; f.hl = h;
+	}
+	*taps = f.taps; *K = f.K; *hl = f.hl;
+	return POV_OK;
+}
 
 static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* data, const size_t* len, uint32_t host_threads,
                          const CorpusOut& fmt, uint64_t* frames_out, uint64_t* total_values_out) {
@@ -618,7 +697,8 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 			for(int attempt = 0; attempt < 2; ++attempt) {       // (second round only if a stream cannot be walked on the device)
 			bool mixed = false;
 			hb.clear(); hb.raw = opt.raw_packets;
-			ck->setups.clear(); ck->stream_file.clear(); ck->stream_channels.clear(); ck->stream_frames.clear(); ck->frames.assign(ck->n_files, 0);
+			ck->setups.clear(); ck->stream_file.clear(); ck->stream_channels.clear(); ck->stream_frames.clear(); ck->stream_rate.clear();
+			ck->frames.assign(ck->n_files, 0);
 			for(uint32_t i = 0; i < ck->n_files && ck->error.empty(); ++i) {
 				ParseError err;
 				file.clear();
@@ -636,6 +716,7 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 					ck->stream_file.push_back(ck->first_file + i);
 					ck->stream_channels.push_back(st.setup.channels);
 					ck->stream_frames.push_back(st.frames);
+					ck->stream_rate.push_back(st.setup.sample_rate);
 					if(k == ck->setups.size()) {
 						st.packets.clear(); st.ys.clear(); st.payload.clear();
 						ck->setups.push_back(std::move(st));
@@ -695,6 +776,7 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 	for(uint32_t t = 0; t < host_threads; ++t) pool.emplace_back(worker);
 
 	uint64_t total = 0;
+	std::vector<ResampleDesc> rs_descs;                  // resampled output: the descriptors of the chunk being queued
 	uint64_t dev_stream = 0;                             // device output: index of the next stream-table record
 	double h_sum = 0;
 	int64_t h_sum16 = 0;
@@ -764,6 +846,8 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 		if(timeline) tl_host[4 * ci] = t0 - t_begin;
 		if(!ck->error.empty()) { rc = pov_fail(ctx, POV_ERR_STREAM, "%s", ck->error.c_str()); cs.release(ck->buf); break; }
 		if(frames_out) for(uint32_t i = 0; i < ck->n_files; ++i) frames_out[ck->first_file + i] = ck->frames[i];
+		rs_descs.clear();
+		uint64_t rs_arena = 0, rs_tiles = 0, rs_values = 0;
 		if(fmt.dev) {
 			// each parsed stream against the caller's record at its index, then to the caller's region (the kernels address planar
 			// PCM as pcm_base + c * pcm_frames + f, so pcm_frames is the channel stride)
@@ -777,6 +861,33 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 					rc = pov_fail(ctx, POV_ERR_ARG, "file %u: pov_decode_corpus_device: stream %llu is (file %u, %u channels, %llu frames), the table says "
 					              "(file %u, %u channels, %llu frames)", ck->stream_file[i], (unsigned long long) k, ck->stream_file[i], ck->stream_channels[i],
 					              (unsigned long long) ck->stream_frames[i], o.file[k], o.channels[k], (unsigned long long) o.frames[k]);
+				else if(fmt.rs && fmt.rs->sample_rate[k] != ck->stream_rate[i])
+					rc = pov_fail(ctx, POV_ERR_ARG, "file %u: pov_decode_corpus_device_resampled: stream %llu has a sample rate of %u Hz, the table says %u Hz",
+					              ck->stream_file[i], (unsigned long long) k, ck->stream_rate[i], fmt.rs->sample_rate[k]);
+				else if(fmt.rs) {
+					// the stream's channels 4-aligned in the slot's arena (so the synthesis takes its vector stores, as into 4-aligned
+					// regions of pov_decode_corpus_device), and a descriptor from there to the caller's region
+					const uint64_t fr = ck->stream_frames[i], stride = (fr + 3) & ~3ull;
+					const uint32_t C = ck->stream_channels[i];
+					if(ck->view.n_packets) { ck->streams[i].pcm_base = rs_arena; ck->streams[i].pcm_frames = stride; }
+					ResampleDesc dsc;
+					memset(&dsc, 0, sizeof dsc);
+					stream_ratio(*fmt.rs, ck->stream_rate[i], &dsc.L, &dsc.M);
+					dsc.in_base = rs_arena; dsc.in_stride = stride; dsc.in_frames = fr; dsc.in_channels = C;
+					dsc.mono = (fmt.rs->flags & POV_RESAMPLE_MONO) != 0;
+					dsc.inv_c = 1.0f / (float) C;
+					dsc.out_channels = dsc.mono ? 1 : C;
+					dsc.out_base = o.stream_base[k]; dsc.out_stride = o.channel_stride[k]; dsc.out_frames = resample_frames(fr, dsc.L, dsc.M);
+					dsc.tile = resample_tile(dsc.L, dsc.M);
+					rs_arena += C * stride;
+					rs_values += dsc.out_channels * dsc.out_frames;
+					if(dsc.out_frames) {
+						rc = resample_filter_table(ctx, cs, dsc.L, dsc.M, &dsc.taps, &dsc.K, &dsc.hl);
+						dsc.tile_first = rs_tiles;
+						rs_tiles += dsc.out_channels * ((dsc.out_frames + dsc.tile - 1) / dsc.tile);
+						rs_descs.push_back(dsc);
+					}
+				}
 				else if(ck->view.n_packets) {
 					ck->streams[i].pcm_base = o.stream_base[k];
 					ck->streams[i].pcm_frames = o.channel_stride[k];
@@ -799,12 +910,13 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 		t_retire += now() - t0; t0 = now();
 		if(timeline) tl_host[4 * ci + 1] = t0 - t_begin;
 		pov_batch b = ck->view;
-		const uint64_t pcm_floats = b.pcm_floats;          // samples the chunk yields
-		if(fmt.dev) b.pcm_floats = fmt.dev->capacity;
+		const uint64_t pcm_floats = fmt.rs ? rs_values : b.pcm_floats;    // samples the chunk yields
+		if(fmt.rs) b.pcm_floats = rs_arena;
+		else if(fmt.dev) b.pcm_floats = fmt.dev->capacity;
 		const uint32_t n_packets = b.n_packets;
 		if(timing) cudaEventRecord(sl.t_begin, cx->stream);
 		if(timeline) cudaEventRecord(tl[4 * ci], cx->stream);
-		rc = fmt.dev ? pov_batch_upload_into(cx, &b, fmt.dev->pcm_dev, &sl.h) : pov_batch_upload(cx, &b, &sl.h);
+		rc = fmt.dev && !fmt.rs ? pov_batch_upload_into(cx, &b, fmt.dev->pcm_dev, &sl.h) : pov_batch_upload(cx, &b, &sl.h);
 		if(timeline) cudaEventRecord(tl[4 * ci + 1], cx->stream);      // pinned sources: the copies are queued, the chunk stays alive until retire()
 		sl.in_flight = std::move(ck);
 		sl.busy = true;                            // from here on retire() has to wait for the stream before the buffer is reused
@@ -833,6 +945,24 @@ static int decode_corpus(pov_ctx* ctx, uint32_t n_files, const uint8_t* const* d
 			if(!fmt.dev) {
 				cudaError_t e = pov_checksum_launch(pov_batch_pcm_dev(sl.h), fmt.s16, pcm_floats, sl.d_sum, cx->stream, &cx->launches);
 				if(e != cudaSuccess) { rc = pov_fail(ctx, POV_ERR_CUDA, "checksum kernel: %s", cudaGetErrorString(e)); break; }
+			} else if(fmt.rs && !rs_descs.empty()) {
+				// descriptors up through the slot's pinned buffer (its last copy ended when the slot retired), then one launch
+				const size_t bytes = rs_descs.size() * sizeof(ResampleDesc);
+				if(bytes > sl.rs_cap) {
+					if(sl.rs_host) cudaFreeHost(sl.rs_host);
+					sl.rs_host = nullptr;
+					sl.rs_cap = bytes + bytes / 4;
+					if(cudaMallocHost((void**) &sl.rs_host, sl.rs_cap) != cudaSuccess) { sl.rs_cap = 0; rc = pov_fail(ctx, POV_ERR_CUDA, "cudaMallocHost failed"); break; }
+				}
+				memcpy(sl.rs_host, rs_descs.data(), bytes);
+				cudaError_t e = sl.rs_dev.reserve(bytes);
+				if(e == cudaSuccess) e = cudaMemcpyAsync(sl.rs_dev.ptr, sl.rs_host, bytes, cudaMemcpyHostToDevice, cx->stream);
+				if(e == cudaSuccess) {
+					cx->h2d_bytes += bytes;
+					e = launch_resample((const float*) pov_batch_pcm_dev(sl.h), (const ResampleDesc*) sl.rs_dev.ptr, (uint32_t) rs_descs.size(), rs_tiles,
+					                    fmt.dev->pcm_dev, (fmt.dev->pcm_layout & POV_PCM_S16) != 0, cx->stream, &cx->launches);
+				}
+				if(e != cudaSuccess) { rc = pov_fail(ctx, POV_ERR_CUDA, "resample kernel: %s", cudaGetErrorString(e)); break; }
 			}
 			if(timing) cudaEventRecord(sl.t_kernels, cx->stream);
 			if(timeline) cudaEventRecord(tl[4 * ci + 2], cx->stream);

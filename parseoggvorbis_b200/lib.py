@@ -27,6 +27,7 @@ SYMBOLS = [
     "pov_ogg_vorbis_decode_memory_s16", "pov_decoded_s16_free", "pov_decode_corpus_s16",
     "pov_ogg_parse_memory", "pov_parsed_stream_count", "pov_parsed_get", "pov_parsed_free",
     "pov_batch_upload_into", "pov_corpus_streams", "pov_corpus_streams_free", "pov_decode_corpus_device",
+    "pov_resample_filter", "pov_decode_corpus_device_resampled",
 ]
 
 
@@ -119,6 +120,10 @@ def load() -> C.CDLL:
     L.pov_corpus_streams_free.restype = None
     L.pov_decode_corpus_device.argtypes = [vp, u32, C.POINTER(C.c_char_p), C.POINTER(C.c_size_t), u32, C.POINTER(abi.pov_device_pcm),
                                            C.POINTER(u64), C.POINTER(u64)]
+    L.pov_resample_filter.argtypes = [u32, u32, C.POINTER(u32), C.POINTER(u32), C.POINTER(u32), C.POINTER(C.c_float), u32]
+    L.pov_decode_corpus_device_resampled.argtypes = [vp, u32, C.POINTER(C.c_char_p), C.POINTER(C.c_size_t), u32,
+                                                     C.POINTER(abi.pov_device_pcm), C.POINTER(abi.pov_resample),
+                                                     C.POINTER(u64), C.POINTER(u64)]
     _LIB = L
     return L
 
@@ -162,6 +167,45 @@ def corpus_streams(files, allow_spanning: bool = False, host_threads: int = 0) -
         L.pov_corpus_streams_free(out)
 
 
+def _resample_ratio(in_rate: int, out_rate: int):
+    """(L, M, half_len) of in_rate -> out_rate; PovError past the supported ratios."""
+    up, down, hl = C.c_uint32(0), C.c_uint32(0), C.c_uint32(0)
+    rc = load().pov_resample_filter(in_rate, out_rate, C.byref(up), C.byref(down), C.byref(hl), None, 0)
+    if rc != 0:
+        raise PovError(rc, "%d Hz -> %d Hz: max(L, M) = %d is past the supported %d (or a rate is 0)"
+                       % (in_rate, out_rate, max(up.value, down.value), abi.POV_RESAMPLE_MAX_PHASES))
+    return int(up.value), int(down.value), int(hl.value)
+
+
+def resample_filter(in_rate: int, out_rate: int):
+    """The in_rate -> out_rate filter of the resampled corpus decode, without a GPU: (up L, down M, half_len, float32 taps
+    h[0 .. 2 half_len]). L = M = 1 is a copy: half_len 0 and no taps. scipy.signal.resample_poly's default design."""
+    L, M, hl = _resample_ratio(in_rate, out_rate)
+    if hl == 0:
+        return L, M, 0, np.zeros(0, np.float32)
+    taps = np.zeros(2 * hl + 1, np.float32)
+    up, down, h = C.c_uint32(0), C.c_uint32(0), C.c_uint32(0)
+    rc = load().pov_resample_filter(in_rate, out_rate, C.byref(up), C.byref(down), C.byref(h),
+                                    taps.ctypes.data_as(C.POINTER(C.c_float)), len(taps))
+    if rc != 0:
+        raise PovError(rc, "pov_resample_filter")
+    return L, M, hl, taps
+
+
+def resampled_frames(table: "StreamTable", out_rate: int) -> np.ndarray:
+    """uint64 output frames per record of `table` at out_rate (0: every stream keeps its rate): ceil(frames L / M)."""
+    frames = np.asarray(table.frames, np.uint64)
+    out = frames.copy()
+    if out_rate == 0:
+        return out
+    rates = np.asarray(table.sample_rate, np.uint32)
+    for r in np.unique(rates):
+        L, M, _ = _resample_ratio(int(r), int(out_rate))
+        sel = rates == r
+        out[sel] = (frames[sel] * np.uint64(L) + np.uint64(M - 1)) // np.uint64(M)
+    return out
+
+
 def _round4(x):
     return (np.asarray(x, np.uint64) + np.uint64(3)) // np.uint64(4) * np.uint64(4)
 
@@ -174,10 +218,16 @@ class DeviceCorpus(NamedTuple):
     stride: np.ndarray         # uint64 [streams], samples between channels
     frames_per_file: np.ndarray
     total_values: int
+    sample_rate: Optional[int] = None        # resampled / downmixed decode: the target rate (0 = each stream's own rate)
+    out_channels: Optional[np.ndarray] = None   # uint32 [streams], channels written per stream
+    out_frames: Optional[np.ndarray] = None     # uint64 [streams], frames written per stream
 
     def stream(self, i: int):
-        """(channels, frames) view of stream i."""
-        c, f = int(self.table.channels[i]), int(self.table.frames[i])
+        """(channels, frames) view of stream i (output channels and frames of a resampled / downmixed decode)."""
+        if self.out_frames is not None:
+            c, f = int(self.out_channels[i]), int(self.out_frames[i])
+        else:
+            c, f = int(self.table.channels[i]), int(self.table.frames[i])
         if self.pcm.dim() == 3:
             return self.pcm[i, :c, :f]
         b, s = int(self.base[i]), int(self.stride[i])
@@ -513,11 +563,14 @@ class SynthContext:
                                                  frames.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(total), C.byref(chk)))
         return frames, int(total.value), int(chk.value)
 
-    def decode_corpus_into(self, files, pcm, table: StreamTable, base, stride, s16: bool = False, host_threads: int = 0):
+    def decode_corpus_into(self, files, pcm, table: StreamTable, base, stride, s16: bool = False, host_threads: int = 0,
+                           sample_rate: Optional[int] = None, mono: bool = False):
         """pov_decode_corpus_device into a tensor the caller laid out: stream i of `table`, channel c, frame f lands at flat
         sample index base[i] + c * stride[i] + f of `pcm` (contiguous, on this context's GPU, float32 or int16 with s16).
         Nothing else of `pcm` is written. No PCM write starts before the work queued on torch's current stream, and the call
-        returns when the PCM is complete. Returns (frames per file, total PCM values)."""
+        returns when the PCM is complete. Returns (frames per file, total PCM values).
+        sample_rate / mono: every stream resampled to sample_rate (0: its own rate) and / or averaged to one channel on the
+        device (pov_decode_corpus_device_resampled); channels and frames are then the output's (resampled_frames)."""
         import torch
         n, m = len(files), len(table)
         base = np.ascontiguousarray(base, np.uint64)
@@ -543,34 +596,56 @@ class SynthContext:
         lens = (C.c_size_t * n)(*[len(f) for f in files])
         frames = np.zeros(n, np.uint64)
         total = C.c_uint64(0)
-        self._check(self.L.pov_decode_corpus_device(self.ctx, n, arr, lens, host_threads, C.byref(o),
-                                                    frames.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(total)))
+        if sample_rate is None and not mono:
+            self._check(self.L.pov_decode_corpus_device(self.ctx, n, arr, lens, host_threads, C.byref(o),
+                                                        frames.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(total)))
+            return frames, int(total.value)
+        rates = np.ascontiguousarray(table.sample_rate, np.uint32)
+        rs = abi.pov_resample()
+        rs.out_rate = int(sample_rate or 0)
+        rs.flags = abi.POV_RESAMPLE_MONO if mono else 0
+        rs.sample_rate = rates.ctypes.data_as(C.POINTER(C.c_uint32))
+        self._check(self.L.pov_decode_corpus_device_resampled(self.ctx, n, arr, lens, host_threads, C.byref(o), C.byref(rs),
+                                                              frames.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(total)))
         return frames, int(total.value)
 
-    def decode_corpus_device(self, files, layout: str = "padded", s16: bool = False, host_threads: int = 0) -> DeviceCorpus:
+    def decode_corpus_device(self, files, layout: str = "padded", s16: bool = False, host_threads: int = 0,
+                             sample_rate: Optional[int] = None, mono: bool = False) -> DeviceCorpus:
         """Decode a corpus straight into a new torch tensor on this context's GPU; only compressed packets go to the device
         and only status words come back. layout "padded": (streams, max channels, T) zeros, T = the longest stream rounded
         up to 4; "packed": one flat tensor, each stream's channels `frames rounded up to 4` apart, back to back. Padding
         stays 0. s16: int16 samples (the POV_PCM_S16 conversion). The stream table is parsed with this context's page-spanning
-        setting."""
+        setting. sample_rate (Hz, 0 = each stream's own) and mono resample / downmix every stream on the device, and the
+        layouts are then sized by output channels and frames (DeviceCorpus.out_channels / out_frames)."""
         import torch
         table = corpus_streams(files, allow_spanning=self._spanning, host_threads=host_threads)
         m = len(table)
-        ch = table.channels.astype(np.uint64)
+        resampled = sample_rate is not None or mono
+        if resampled:
+            out_frames = resampled_frames(table, int(sample_rate or 0))
+            out_channels = np.ones(m, np.uint32) if mono else table.channels.astype(np.uint32)
+            table_frames = out_frames
+        else:
+            out_frames = out_channels = None
+            table_frames = table.frames
+        ch = (out_channels if resampled else table.channels).astype(np.uint64)
         dtype = torch.int16 if s16 else torch.float32
         dev = torch.device("cuda", self.device)
         if layout == "padded":
-            T = int(_round4(table.frames.max())) if m else 0
+            T = int(_round4(table_frames.max())) if m else 0
             maxc = int(ch.max()) if m else 0
             pcm = torch.zeros((m, maxc, T), dtype=dtype, device=dev)
             stride = np.full(m, T, np.uint64)
             base = np.arange(m, dtype=np.uint64) * np.uint64(maxc * T)
         elif layout == "packed":
-            stride = _round4(table.frames)
+            stride = _round4(table_frames)
             sizes = ch * stride
             base = (np.cumsum(sizes) - sizes).astype(np.uint64)
             pcm = torch.zeros(int(sizes.sum()), dtype=dtype, device=dev)
         else:
             raise ValueError("layout must be 'padded' or 'packed'")
-        frames, total = self.decode_corpus_into(files, pcm, table, base, stride, s16=s16, host_threads=host_threads)
-        return DeviceCorpus(pcm, table, base, stride, frames, total)
+        frames, total = self.decode_corpus_into(files, pcm, table, base, stride, s16=s16, host_threads=host_threads,
+                                                sample_rate=sample_rate, mono=mono)
+        if not resampled:
+            return DeviceCorpus(pcm, table, base, stride, frames, total)
+        return DeviceCorpus(pcm, table, base, stride, frames, total, int(sample_rate or 0), out_channels, out_frames)
