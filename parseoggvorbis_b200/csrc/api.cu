@@ -75,6 +75,16 @@ cudaError_t DevBuf::reserve(size_t bytes) {
 }
 void DevBuf::release() { if(ptr) cudaFree(ptr); ptr = nullptr; cap = 0; }
 
+cudaError_t PinnedBuf::reserve(size_t bytes) {
+	if(bytes <= cap) return cudaSuccess;
+	release();
+	cudaError_t e = cudaHostAlloc(&ptr, bytes + bytes / 4, cudaHostAllocDefault);
+	if(e == cudaSuccess) cap = bytes + bytes / 4;
+	else ptr = nullptr;
+	return e;
+}
+void PinnedBuf::release() { if(ptr) cudaFreeHost(ptr); ptr = nullptr; cap = 0; }
+
 // ---------------------------------------------------------------------------------------------------------------
 // context
 // ---------------------------------------------------------------------------------------------------------------
@@ -623,7 +633,7 @@ static void release_batch(pov_batch_handle* h) {
 	h->d_feat_rows.release(); h->d_feat_floors.release(); h->d_feat_out.release();
 	h->st_final_ys.release(); h->st_flag.release(); h->st_floor.release(); h->st_floor_out.release();
 	h->st_env.release(); h->st_mdct.release();
-	if(h->h_derived) { cudaFreeHost(h->h_derived); h->h_derived = nullptr; h->h_derived_cap = 0; }
+	h->h_derived.release();
 	if(h->derived_copied) { cudaEventDestroy(h->derived_copied); h->derived_copied = nullptr; }
 }
 
@@ -634,7 +644,6 @@ extern "C" void pov_batch_free(pov_ctx* ctx, pov_batch_handle* h) {
 	delete h;
 }
 
-// Device memory of the context's GPU, aligned to `align` bytes: where pov_batch_upload_into / pov_decode_corpus_device may write.
 int pov_check_pcm_dev(pov_ctx* ctx, const void* p, size_t align, const char* fn) {
 	if(!p) return pov_fail(ctx, POV_ERR_ARG, "%s: null pcm_dev", fn);
 	if((uintptr_t) p % align) return pov_fail(ctx, POV_ERR_ARG, "%s: pcm_dev is not aligned to a %zu-byte sample", fn, align);
@@ -882,22 +891,18 @@ static int batch_upload(pov_ctx* ctx, const pov_batch* b, void* pcm_dev, pov_bat
 		const size_t need = std::max<size_t>(o_pk + b_pk, 16);
 		if(h->derived_copied) CUDA_TRY(ctx, cudaEventSynchronize(h->derived_copied));     // the previous upload through this handle has read them
 		else CUDA_TRY(ctx, cudaEventCreateWithFlags(&h->derived_copied, cudaEventDisableTiming));
-		if(need > h->h_derived_cap) {
-			if(h->h_derived) cudaFreeHost(h->h_derived);
-			h->h_derived = nullptr; h->h_derived_cap = 0;
-			CUDA_TRY(ctx, cudaHostAlloc(&h->h_derived, need + need / 4, cudaHostAllocDefault));
-			h->h_derived_cap = need + need / 4;
-		}
-		if(b_spec) memcpy(h->h_derived, h->spec_off.data(), b_spec);
-		if(b_runs) memcpy((uint8_t*) h->h_derived + o_runs, h->runs.data(), b_runs);
+		CUDA_TRY(ctx, h->h_derived.reserve(need));
+		uint8_t* hd = (uint8_t*) h->h_derived.ptr;
+		if(b_spec) memcpy(hd, h->spec_off.data(), b_spec);
+		if(b_runs) memcpy(hd + o_runs, h->runs.data(), b_runs);
 		if(b_pk) {
-			memcpy((uint8_t*) h->h_derived + o_pk, h->pk_ys_off.data(), b_pk / 3);
-			memcpy((uint8_t*) h->h_derived + o_pk + b_pk / 3, h->pk_ent_off.data(), b_pk / 3);
-			memcpy((uint8_t*) h->h_derived + o_pk + 2 * (b_pk / 3), h->pk_raw_off.data(), b_pk / 3);
-			CUDA_TRY(ctx, up(h->d_pk_off, (uint8_t*) h->h_derived + o_pk, b_pk));
+			memcpy(hd + o_pk, h->pk_ys_off.data(), b_pk / 3);
+			memcpy(hd + o_pk + b_pk / 3, h->pk_ent_off.data(), b_pk / 3);
+			memcpy(hd + o_pk + 2 * (b_pk / 3), h->pk_raw_off.data(), b_pk / 3);
+			CUDA_TRY(ctx, up(h->d_pk_off, hd + o_pk, b_pk));
 		}
-		CUDA_TRY(ctx, up(h->d_spec_off, h->h_derived, b_spec));
-		CUDA_TRY(ctx, up(h->d_runs, (uint8_t*) h->h_derived + o_runs, b_runs));
+		CUDA_TRY(ctx, up(h->d_spec_off, hd, b_spec));
+		CUDA_TRY(ctx, up(h->d_runs, hd + o_runs, b_runs));
 		CUDA_TRY(ctx, cudaEventRecord(h->derived_copied, st));
 	}
 	if(pcm_dev) h->d_pcm.release();          // (cudaFree waits for the device: the previous run has written its arena)
@@ -1090,15 +1095,16 @@ extern "C" int pov_batch_status(pov_ctx* ctx, pov_batch_handle* h, uint32_t* out
 	ctx->d2h_bytes += sizeof(uint32_t) * h->n_packets;
 	CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
 	if(out) memcpy(out, tmp.data(), sizeof(uint32_t) * std::min<uint32_t>(n, h->n_packets));
-	for(uint32_t p = 0; p < h->n_packets; ++p) {
-		if(!tmp[p]) continue;
-		const char* what = (tmp[p] & POV_PKT_FLOOR_PREDICTED) ? "predicted <= range (hpp:536)"
-		                 : (tmp[p] & POV_PKT_FLOOR_RANGE)     ? "floor[i] < 256 (hpp:587)"
-		                                                      : "temp.size() > 0 (hpp:739,748: VQ entry out of range)";
-		return pov_fail(ctx, POV_ERR_STREAM, "audio packet %u: check failed: %s", p, what);
-	}
+	for(uint32_t p = 0; p < h->n_packets; ++p)
+		if(tmp[p]) return pov_fail(ctx, POV_ERR_STREAM, "audio packet %u: check failed: %s", p, pov_status_text(tmp[p]));
 	return POV_OK;
 } POV_NOTHROW_END(ctx)
+
+const char* pov_status_text(uint32_t status) {
+	return (status & POV_PKT_FLOOR_PREDICTED) ? "predicted <= range (hpp:536)"
+	     : (status & POV_PKT_FLOOR_RANGE)     ? "floor[i] < 256 (hpp:587)"
+	                                          : "temp.size() > 0 (hpp:739,748: VQ entry out of range)";
+}
 
 extern "C" int pov_batch_fetch_stage(pov_ctx* ctx, pov_batch_handle* h, uint32_t packet, uint32_t channel, int stage,
                                      void* out, uint64_t out_bytes) try {

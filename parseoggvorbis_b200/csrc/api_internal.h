@@ -18,6 +18,15 @@ struct DevBuf {
 	void release();
 };
 
+// Growable pinned host buffer: the source or destination of asynchronous copies (a pageable one makes the "async" copy wait
+// for the stream). reserve() grows it to bytes + bytes / 4 and does not keep the contents.
+struct PinnedBuf {
+	void* ptr = nullptr;
+	size_t cap = 0;
+	cudaError_t reserve(size_t bytes);
+	void release();
+};
+
 struct BlockTables {              // per blocksize n: DCT-IV rotation, FFT twiddles, rising slope of n/2 samples
 	const float2* d_rot = nullptr;
 	const float2* d_fft = nullptr;
@@ -123,9 +132,8 @@ struct pov_batch_handle {
 	DevBuf d_entries, d_pk_off;                      // POV_INPUT_PACKETS: entries payload written by k_packet_decode; ys_off | ent_off
 	DevBuf d_res_cursor;                             // k_residue_apply's read cursors when they do not fit its shared memory
 	DevBuf st_final_ys, st_flag, st_floor, st_floor_out, st_env, st_mdct;
-	// pinned copy of the derived arrays (spec_off | runs): sources of asynchronous copies, so they must not be pageable
-	// (a pageable source makes the "async" copy wait for the stream) and must outlive the copy (derived_copied)
-	void* h_derived = nullptr; size_t h_derived_cap = 0;
+	// pinned copy of the derived arrays (spec_off | runs): sources of asynchronous copies, so they must outlive the copy (derived_copied)
+	PinnedBuf h_derived;
 	cudaEvent_t derived_copied = nullptr;
 };
 
@@ -144,5 +152,9 @@ int pov_fail(pov_ctx* ctx, int code, const char* fmt, ...);
 int pov_fail_exception(pov_ctx* ctx);
 #define POV_NOTHROW_END(ctx) catch(...) { return pov_fail_exception(ctx); }
 int pov_batch_fetch_stage_all(pov_ctx* ctx, pov_batch_handle* h, StageHost& out);
+// Device memory of the context's GPU, aligned to `align` bytes: where pov_batch_upload_into / pov_decode_corpus_device may write.
+int pov_check_pcm_dev(pov_ctx* ctx, const void* p, size_t align, const char* fn);
+// The reference's check that a non-zero packet status word (POV_PKT_*) reports, as error text.
+const char* pov_status_text(uint32_t status);
 
 #endif

@@ -75,4 +75,7 @@ cudaError_t launch_mdct_backward(const DevSetup* dummy, uint32_t n, uint64_t cou
                                  const float2* rot, const float2* fft, cudaStream_t st, uint64_t* launches);
 
 }  // namespace pov
+
+// float64 sum of a float arena into *(double*) d_sum, or (s16) exact int64 sum of an int16 arena into *(uint64_t*) d_sum
+cudaError_t pov_checksum_launch(const void* pcm, bool s16, uint64_t n, void* d_sum, cudaStream_t st, uint64_t* launches);
 #endif

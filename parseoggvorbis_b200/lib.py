@@ -35,6 +35,24 @@ SINK_FN = C.CFUNCTYPE(C.c_int, C.c_uint32, C.c_uint32, C.c_uint64, C.POINTER(C.c
 SINK_S16_FN = C.CFUNCTYPE(C.c_int, C.c_uint32, C.c_uint32, C.c_uint64, C.POINTER(C.c_int16), C.c_void_p)
 
 
+def _sink_fn(sink, fn_type):
+    """`sink(file_index, pcm)` as a C sink of fn_type (SINK_FN / SINK_S16_FN), pcm a (channels, frames) view that is only
+    valid during the call; a true return value asks the decode to stop. None: a null sink. Keep the result alive during the call."""
+    if sink is None:
+        return C.cast(None, fn_type)
+
+    @fn_type
+    def _sink(file_index, channels, nframes, planar, user):
+        pcm = np.ctypeslib.as_array(planar, shape=(int(channels), int(nframes)))
+        return 1 if sink(int(file_index), pcm) else 0
+    return _sink
+
+
+def _file_arrays(files):
+    """The ctypes file-pointer and length arrays of a corpus call."""
+    return (C.c_char_p * len(files))(*files), (C.c_size_t * len(files))(*[len(f) for f in files])
+
+
 class PovError(RuntimeError):
     def __init__(self, code: int, msg: str):
         super().__init__("pov error %d: %s" % (code, msg))
@@ -148,13 +166,11 @@ def corpus_streams(files, allow_spanning: bool = False, host_threads: int = 0) -
     what decode_corpus / decode_corpus_device produce. A framing or header error raises PovError with the corpus decode's
     text ("file k: check failed: ...")."""
     L = load()
-    n = len(files)
-    arr = (C.c_char_p * n)(*files)
-    lens = (C.c_size_t * n)(*[len(f) for f in files])
+    arr, lens = _file_arrays(files)
     out = C.POINTER(abi.pov_stream_info)()
     count = C.c_uint64(0)
     err = C.c_char_p(None)
-    rc = L.pov_corpus_streams(n, arr, lens, abi.POV_PARSE_ALLOW_SPANNING if allow_spanning else 0, host_threads, C.byref(out),
+    rc = L.pov_corpus_streams(len(files), arr, lens, abi.POV_PARSE_ALLOW_SPANNING if allow_spanning else 0, host_threads, C.byref(out),
                               C.byref(count), C.byref(err))
     if rc != 0:
         raise PovError(rc, (err.value or b"?").decode())
@@ -512,17 +528,7 @@ class SynthContext:
     def decode_corpus(self, files, host_threads: int = 0, s16: bool = False):
         """files: list of bytes. Returns (frames per file, total PCM values, checksum). s16: int16 PCM (pov_decode_corpus_s16,
         half the device -> host bytes); the checksum is then the exact integer sum of every sample."""
-        if s16:
-            return self._decode_corpus_s16(files, None, host_threads)
-        n = len(files)
-        arr = (C.c_char_p * n)(*files)
-        lens = (C.c_size_t * n)(*[len(f) for f in files])
-        frames = np.zeros(n, np.uint64)
-        total = C.c_uint64(0)
-        chk = C.c_double(0)
-        self._check(self.L.pov_decode_corpus(self.ctx, n, arr, lens, host_threads,
-                                             frames.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(total), C.byref(chk)))
-        return frames, int(total.value), float(chk.value)
+        return self.decode_corpus_pcm(files, None, host_threads, s16)
 
     def decode_corpus_pcm(self, files, sink, host_threads: int = 0, s16: bool = False):
         """The corpus decode with its output edge (pov_decode_corpus_pcm): `sink(file_index, pcm)` is called from this thread
@@ -530,38 +536,23 @@ class SynthContext:
         a true return value stops the decode (PovError, like the reference's CHECK(callbacks.gotPcmData(...))).
         s16: the arrays are int16 (pov_decode_corpus_s16) and the returned checksum is the exact integer sum."""
         if s16:
-            return self._decode_corpus_s16(files, sink, host_threads)
-        n = len(files)
-        arr = (C.c_char_p * n)(*files)
-        lens = (C.c_size_t * n)(*[len(f) for f in files])
-        frames = np.zeros(n, np.uint64)
-        total = C.c_uint64(0)
-        chk = C.c_double(0)
+            fn, chk, sink_args = self.L.pov_decode_corpus_s16, C.c_int64(0), (_sink_fn(sink, SINK_S16_FN), None)
+        elif sink is None:
+            fn, chk, sink_args = self.L.pov_decode_corpus, C.c_double(0), ()
+        else:
+            fn, chk, sink_args = self.L.pov_decode_corpus_pcm, C.c_double(0), (_sink_fn(sink, SINK_FN), None)
+        frames, total = self._decode_corpus_call(fn, files, host_threads, sink_args, (C.byref(chk),))
+        return frames, total, chk.value
 
-        @SINK_FN
-        def _sink(file_index, channels, nframes, planar, user):
-            pcm = np.ctypeslib.as_array(planar, shape=(int(channels), int(nframes)))
-            return 1 if sink(int(file_index), pcm) else 0
-        self._check(self.L.pov_decode_corpus_pcm(self.ctx, n, arr, lens, host_threads, _sink, None,
-                                                 frames.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(total), C.byref(chk)))
-        return frames, int(total.value), float(chk.value)
-
-    def _decode_corpus_s16(self, files, sink, host_threads: int):
-        n = len(files)
-        arr = (C.c_char_p * n)(*files)
-        lens = (C.c_size_t * n)(*[len(f) for f in files])
-        frames = np.zeros(n, np.uint64)
+    def _decode_corpus_call(self, fn, files, host_threads: int, before=(), after=()):
+        """fn(ctx, n, files, lengths, host_threads, *before, frames, &total, *after), one of the pov_decode_corpus* calls.
+        Returns (frames per file, total PCM values)."""
+        arr, lens = _file_arrays(files)
+        frames = np.zeros(len(files), np.uint64)
         total = C.c_uint64(0)
-        chk = C.c_int64(0)
-        _sink = C.cast(None, SINK_S16_FN)
-        if sink is not None:
-            @SINK_S16_FN
-            def _sink(file_index, channels, nframes, planar, user):
-                pcm = np.ctypeslib.as_array(planar, shape=(int(channels), int(nframes)))
-                return 1 if sink(int(file_index), pcm) else 0
-        self._check(self.L.pov_decode_corpus_s16(self.ctx, n, arr, lens, host_threads, _sink, None,
-                                                 frames.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(total), C.byref(chk)))
-        return frames, int(total.value), int(chk.value)
+        self._check(fn(self.ctx, len(files), arr, lens, host_threads, *before, frames.ctypes.data_as(C.POINTER(C.c_uint64)),
+                       C.byref(total), *after))
+        return frames, int(total.value)
 
     def decode_corpus_into(self, files, pcm, table: StreamTable, base, stride, s16: bool = False, host_threads: int = 0,
                            sample_rate: Optional[int] = None, mono: bool = False):
@@ -572,7 +563,7 @@ class SynthContext:
         sample_rate / mono: every stream resampled to sample_rate (0: its own rate) and / or averaged to one channel on the
         device (pov_decode_corpus_device_resampled); channels and frames are then the output's (resampled_frames)."""
         import torch
-        n, m = len(files), len(table)
+        m = len(table)
         base = np.ascontiguousarray(base, np.uint64)
         stride = np.ascontiguousarray(stride, np.uint64)
         if base.shape != (m,) or stride.shape != (m,):
@@ -592,22 +583,14 @@ class SynthContext:
         o.channels = channels.ctypes.data_as(C.POINTER(C.c_uint32))
         o.frames = tframes.ctypes.data_as(C.POINTER(C.c_uint64))
         o.cuda_stream = torch.cuda.current_stream(self.device).cuda_stream or None
-        arr = (C.c_char_p * n)(*files)
-        lens = (C.c_size_t * n)(*[len(f) for f in files])
-        frames = np.zeros(n, np.uint64)
-        total = C.c_uint64(0)
         if sample_rate is None and not mono:
-            self._check(self.L.pov_decode_corpus_device(self.ctx, n, arr, lens, host_threads, C.byref(o),
-                                                        frames.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(total)))
-            return frames, int(total.value)
+            return self._decode_corpus_call(self.L.pov_decode_corpus_device, files, host_threads, (C.byref(o),))
         rates = np.ascontiguousarray(table.sample_rate, np.uint32)
         rs = abi.pov_resample()
         rs.out_rate = int(sample_rate or 0)
         rs.flags = abi.POV_RESAMPLE_MONO if mono else 0
         rs.sample_rate = rates.ctypes.data_as(C.POINTER(C.c_uint32))
-        self._check(self.L.pov_decode_corpus_device_resampled(self.ctx, n, arr, lens, host_threads, C.byref(o), C.byref(rs),
-                                                              frames.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(total)))
-        return frames, int(total.value)
+        return self._decode_corpus_call(self.L.pov_decode_corpus_device_resampled, files, host_threads, (C.byref(o), C.byref(rs)))
 
     def decode_corpus_device(self, files, layout: str = "padded", s16: bool = False, host_threads: int = 0,
                              sample_rate: Optional[int] = None, mono: bool = False) -> DeviceCorpus:
