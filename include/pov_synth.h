@@ -227,6 +227,9 @@ void        pov_ctx_set_device_entropy(pov_ctx* ctx, int on);
 /* Whole-file and corpus decode accept packets spanning pages when `on` is non-zero (default off = the reference's hpp:89;
  * environment POV_ALLOW_SPANNING=1 turns it on). */
 void        pov_ctx_set_page_spanning(pov_ctx* ctx, int on);
+/* Corpus decodes of this context cut damaged streams instead of failing when `on` is non-zero (default off: the first damaged
+ * file fails the call). See "Cut mode" below; the whole-file and batch calls are not affected. */
+void        pov_ctx_set_cut_damage(pov_ctx* ctx, int on);
 /* Bytes this context has copied host -> device and device -> host so far (descriptor/payload arenas, PCM, status words). */
 void        pov_ctx_io_bytes(const pov_ctx* ctx, uint64_t* h2d_out, uint64_t* d2h_out);
 
@@ -362,8 +365,9 @@ int  pov_decode_corpus_s16(pov_ctx* ctx, uint32_t n_files, const uint8_t* const*
  * reaches a complete setup, in file order and, inside a file, in the order the corpus decode delivers them (a chained file has
  * several). It runs the corpus decode's own parse (raw-packet mode, `host_threads` threads, 0 = all cores but one) and discards
  * the packets, so `frames` is what the decode produces. flags: POV_PARSE_ALLOW_SPANNING (see pov_ogg_parse_memory_ex; the
- * corpus decode follows pov_ctx_set_page_spanning). A framing or header error fails with POV_ERR_STREAM and the text
- * pov_decode_corpus gives for it ("file k: check failed: ..."), in *error_out (per-thread buffer). On success *out holds
+ * corpus decode follows pov_ctx_set_page_spanning) and POV_PARSE_CUT_DAMAGE (cut mode, below; the corpus decode follows
+ * pov_ctx_set_cut_damage). Without it a framing or header error fails with POV_ERR_STREAM and the text pov_decode_corpus
+ * gives for it ("file k: check failed: ..."), in *error_out (per-thread buffer). On success *out holds
  * *n_streams_out records (NULL when there are none), allocated by the library: free with pov_corpus_streams_free.
  * Callers use it to size and lay out the output of pov_decode_corpus_device, or to bucket files by length. */
 typedef struct pov_stream_info {
@@ -459,6 +463,50 @@ int  pov_decode_corpus_device_resampled(pov_ctx* ctx, uint32_t n_files, const ui
                                         uint32_t host_threads, const pov_device_pcm* out, const pov_resample* rs,
                                         uint64_t* frames_out, uint64_t* total_values_out);
 
+/* Cut mode (pov_ctx_set_cut_damage, POV_PARSE_CUT_DAMAGE): every corpus call — pov_decode_corpus, _pcm, _s16, _device,
+ * _device_resampled — and pov_corpus_streams go on past damaged files; each damaged stream ends where its damage starts.
+ * Damage is found at two levels, and the level decides whether a stream's frame count changes.
+ * 1. Geometry damage: a failing check of the raw-packet parse that pov_corpus_streams runs — Ogg framing (capture pattern,
+ *    truncated segment table or body, CRC), stream bookkeeping (unknown serial, duplicate begin-of-stream, the continuation
+ *    flag), the three headers, an audio packet's type bit, mode number and window flags, and the granule checks. The parse of
+ *    the file stops there: every stream keeps the audio packets completed before the failure; the failing packet, the rest of
+ *    its page and all later pages are dropped; a stream without a complete setup has no record. Its `frames` shrink, in the
+ *    stream table and in the decode alike (they run the same parse).
+ * 2. Content damage: a non-zero status word (POV_PKT_*) of a stream's packet, or with the host walk (POV_DEVICE_ENTROPY=0, or
+ *    a setup the device walk cannot take) a failing walk of its floors and residues. The stream keeps its frames. With p its
+ *    first damaged packet, its valid frames are pcm_off[p], and samples [pcm_off[p], frames) of every channel are exact zeros.
+ *    A packet whose host walk fails enters the batch as silence (no floor used, residues that decode nothing), so the geometry
+ *    stays; every later packet of that stream is silence too, which does not matter because everything after the cut is zero.
+ * Consequences:
+ * - Before the cut the samples are bit-identical to a strict decode, with the same alignment, of the undamaged file (content
+ *   damage) or of the file truncated before the damaged page (geometry damage): packets < p are unchanged, and equal frames
+ *   give equal PCM.
+ * - Output regions keep their rule: exactly [base + c * stride, base + c * stride + frames) is written, padding is untouched.
+ * - Resampled output is the resample of the zero-tailed stream; int16 output is the POV_PCM_S16 rule applied to it (0 in the
+ *   tail). The float64 checksum, the int16 sum and the sinks see the zero-tailed PCM. frames_out stays the frames written.
+ * - The stream table and the decode must use the same mode (as with page spanning): otherwise the records do not match what is
+ *   parsed and the decode fails with POV_ERR_ARG as for any mismatch.
+ * - Out of memory, CUDA failures, a stream-table mismatch and a sink asking to stop still fail the call in both modes.
+ * Not done: resynchronising after damage (scanning for the next capture pattern and decoding on past a hole), concealing one
+ * bad packet and decoding on, and cut mode for pov_ogg_vorbis_decode_memory* and the batch calls. Strict-mode texts are as before.
+ *
+ * What the last successful corpus call of the context found, per file (pov_corpus_report), in both modes: */
+typedef struct pov_file_report {
+	uint32_t status;          /* POV_OK, or POV_ERR_STREAM: damaged, cut as above */
+	uint32_t n_streams;       /* its records in the stream table */
+	uint64_t frames;          /* = frames_out[file] */
+	uint64_t valid_frames;    /* summed over its streams: frames before each stream's cut */
+	char     message[192];    /* "" or the reason: for geometry damage exactly the strict decode's and pov_corpus_streams'
+	                             "file k: check failed: ..." text; otherwise "file k: stream s: check failed: audio packet p: <reason>"
+	                             with s the stream's index among the file's records, p its packet index and the status word's
+	                             reason. A file with both kinds reports its geometry damage. */
+} pov_file_report;
+/* Copies the report of the context's last corpus call when that call succeeded: files[n_files] and, when stream_valid_frames
+ * is not NULL, the valid frames of every record of its stream table, stream_valid_frames[n_streams] (n_streams is the sum of
+ * the files' n_streams). POV_ERR_ARG when the last corpus call failed in any way (argument checks included) or there was
+ * none, and when n_files, or with the array n_streams, is not that call's. */
+int  pov_corpus_report(const pov_ctx* ctx, uint32_t n_files, pov_file_report* files, uint64_t n_streams, uint64_t* stream_valid_frames);
+
 /* Host-only front-end (no GPU needed): parse a whole Ogg/Vorbis file into descriptor batches, one per logical stream
  * (Ogg framing hpp:51-102,1433-1484; headers hpp:1283-1373; per-packet entropy decode hpp:498-517, 711-757). The
  * setup/batch returned by pov_parsed_get point into memory owned by the handle (POV_INPUT_ENTRIES, setup_id 0). */
@@ -470,6 +518,9 @@ int      pov_ogg_parse_memory(const uint8_t* data, size_t len, pov_parsed** out,
 /*        POV_PARSE_ALLOW_SPANNING — accept packets that continue on the next page of their stream (RFC 3533). The reference
  * refuses such files (hpp:89: "we don't support packets spanning pages"), which stays the default for parity. */
 #define POV_PARSE_ALLOW_SPANNING 2u
+/*        POV_PARSE_CUT_DAMAGE — cut mode (above): geometry damage ends the parse with success and the packets before it; with
+ * the host walk a packet whose walk fails is kept as silence. Also a flag of pov_corpus_streams, whose records then shrink. */
+#define POV_PARSE_CUT_DAMAGE 4u
 int      pov_ogg_parse_memory_ex(const uint8_t* data, size_t len, uint32_t flags, pov_parsed** out, const char** error_out);
 uint32_t pov_parsed_stream_count(const pov_parsed* p);
 int      pov_parsed_get(const pov_parsed* p, uint32_t stream, pov_setup* setup_out, pov_batch* batch_out);

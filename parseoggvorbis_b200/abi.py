@@ -26,6 +26,7 @@ POV_INPUT_DENSE, POV_INPUT_ENTRIES, POV_INPUT_PACKETS = 0, 1, 2
 POV_PCM_PLANAR, POV_PCM_INTERLEAVED = 0, 1
 POV_PCM_S16 = 0x100          # OR-ed into pcm_layout: the kernels store int16 PCM (see include/pov_synth.h)
 POV_PARSE_RAW_PACKETS, POV_PARSE_ALLOW_SPANNING = 1, 2     # flags of pov_ogg_parse_memory_ex / pov_corpus_streams
+POV_PARSE_CUT_DAMAGE = 4     # cut mode: damage ends the damaged stream instead of failing (see include/pov_synth.h)
 POV_RESAMPLE_MONO = 1        # pov_resample.flags: average the channels before resampling
 POV_RESAMPLE_MAX_PHASES = 2048   # largest max(L, M) of a supported resampling ratio
 
@@ -114,6 +115,12 @@ class pov_stream_info(C.Structure):
     """One record of pov_corpus_streams' stream table."""
     _fields_ = [("file", C.c_uint32), ("channels", C.c_uint32), ("sample_rate", C.c_uint32), ("reserved", C.c_uint32),
                 ("frames", C.c_uint64)]
+
+
+class pov_file_report(C.Structure):
+    """One file of pov_corpus_report: what the last corpus call found in it."""
+    _fields_ = [("status", C.c_uint32), ("n_streams", C.c_uint32), ("frames", C.c_uint64), ("valid_frames", C.c_uint64),
+                ("message", C.c_char * 192)]
 
 
 class pov_device_pcm(C.Structure):

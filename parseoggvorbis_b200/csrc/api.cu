@@ -163,6 +163,7 @@ extern "C" void* pov_ctx_stream(pov_ctx* ctx) { return ctx ? (void*) ctx->stream
 extern "C" uint64_t pov_ctx_launch_count(const pov_ctx* ctx) { return ctx ? ctx->launches : 0; }
 extern "C" void pov_ctx_set_device_entropy(pov_ctx* ctx, int on) { if(ctx) ctx->device_entropy = on != 0; }
 extern "C" void pov_ctx_set_page_spanning(pov_ctx* ctx, int on) { if(ctx) ctx->allow_spanning = on != 0; }
+extern "C" void pov_ctx_set_cut_damage(pov_ctx* ctx, int on) { if(ctx) ctx->cut_damage = on != 0; }
 extern "C" void pov_ctx_io_bytes(const pov_ctx* ctx, uint64_t* h2d, uint64_t* d2h) {
 	if(h2d) *h2d = ctx ? ctx->h2d_bytes : 0;
 	if(d2h) *d2h = ctx ? ctx->d2h_bytes : 0;

@@ -90,6 +90,10 @@ struct pov_ctx {
 	int kernel_choice = 0;        // POV_KERNEL: 0 automatic, 1 force the CTA-per-run fused kernel, 2 require the warp kernel
 	bool allow_spanning = false;  // accept packets that span pages (the reference refuses them, hpp:89)
 	bool device_entropy = true;   // whole-file / corpus decode: audio packets are entropy-decoded on the device (POV_DEVICE_ENTROPY=0: on the host)
+	bool cut_damage = false;      // corpus decode: cut damaged streams and go on (pov_ctx_set_cut_damage)
+	std::vector<pov_file_report> corpus_files;   // pov_corpus_report: the last corpus call's per-file report
+	std::vector<uint64_t> corpus_valid;          // and its valid frames per stream-table record
+	bool corpus_report_ok = false;               // that call succeeded (every corpus entry point resets it first)
 	uint32_t* d_counter = nullptr; // work counter of the persistent kernel
 	const float* d_inv_db = nullptr;
 	const DevSetup* d_setups = nullptr;

@@ -71,6 +71,25 @@ cudaError_t launch_features(int kind, const FeatRow* rows, uint64_t n_rows, cons
                             const uint32_t* final_ys, const uint16_t* floor, const float* residue, float* out, cudaStream_t st, uint64_t* launches);
 cudaError_t launch_packet_decode(const DevBatchView& b, pov_packet* packets, uint16_t* ys_out, uint8_t* ent_out, const uint64_t* ys_off,
                                  const uint64_t* ent_off, const uint64_t* raw_off, uint32_t n_packets, cudaStream_t st, uint64_t* launches);
+// Cut mode of the corpus decode (kernel_cut.cu): one logical stream of a chunk, where the synthesis wrote it. Blocks
+// [tile_first, tile_first + channels * tiles) of the launch work on it, tiles = max(1, ceil(frames / kCutTile)).
+constexpr uint64_t kCutTile = 32768;               // frames per block
+struct CutDesc {
+	uint64_t base, stride, frames;                 // sample index of channel 0, samples between channels, frames
+	uint64_t tile_first;
+	uint32_t first_packet, n_packets;              // the stream's packets (and status words) in the chunk's batch
+	uint32_t walk_bad;                             // stream-relative packet whose host walk failed, or 0xFFFFFFFF
+	uint32_t channels;
+	uint64_t tiles;
+};
+struct CutResult {
+	uint64_t valid_frames;                         // pcm_off of the first damaged packet, or frames
+	uint32_t packet;                               // that packet (stream-relative), 0xFFFFFFFF: none
+	uint32_t status;                               // its status word (0: only its host walk failed)
+};
+// descs ascending by tile_first, n_tiles = last tile_first + its blocks; pcm: float, or int16_t when s16.
+cudaError_t launch_cut_damaged(void* pcm, bool s16, const CutDesc* descs, uint32_t n_descs, uint64_t n_tiles, const uint32_t* status,
+                               const pov_packet* packets, CutResult* results, cudaStream_t st, uint64_t* launches);
 cudaError_t launch_mdct_backward(const DevSetup* dummy, uint32_t n, uint64_t count, const float* in, float* out,
                                  const float2* rot, const float2* fft, cudaStream_t st, uint64_t* launches);
 

@@ -521,37 +521,12 @@ static bool decode_residue_submap(BitCursor& br, const VorbisSetup& s, const Res
 	return true;
 }
 
-static bool decode_audio_packet(StreamWork& st, const uint8_t* p, size_t len, int64_t expected_end, const Fail& fail, const ParseOptions& opt) {
+// The host walk of one audio packet (floor Y lists and residue entry numbers) into st.ys / st.payload. *status: the POV_PKT_*
+// word the device walk (k_packet_decode) reports for the same failure, 0 when none does.
+static bool walk_audio_packet(StreamWork& st, BitCursor& br, const MappingSetup& mp, uint32_t half, pov_packet& pk, uint32_t* status,
+                              const Fail& fail) {
 	const VorbisSetup& s = st.setup;
-	BitCursor br;
-	br.reset(p, len);
-	st.abs_total_pos.push_back(st.total_pos);
-	st.expected_end.push_back(expected_end);
-	REQUIRE(br.get(1) == 0, "audio packet: packet type bit set (hpp:1142)");
-	const uint32_t mode_idx = br.get(ilog((uint32_t) s.modes.size() - 1));
-	REQUIRE(mode_idx < s.modes.size(), "audio packet: mode %u out of range (hpp:1147)", mode_idx);
-	const ModeSetup& mode = s.modes[mode_idx];
-	const MappingSetup& mp = s.mappings[mode.mapping];
-	uint32_t wflags = 0;
-	if(mode.blockflag) { wflags = br.get(1); wflags |= br.get(1) << 1; }          // hpp:1150-1153
-	const uint32_t n = s.blocksize[mode.blockflag ? 1 : 0], half = n / 2;
 	const uint32_t C = s.channels;
-
-	pov_packet pk;
-	memset(&pk, 0, sizeof pk);
-	pk.mode = (uint8_t) mode_idx;
-	pk.window_flags = (uint8_t) wflags;
-	pk.ys_off = st.ys.size();
-	pk.spec_off = st.payload.size();
-	if(st.raw) {
-		// the device walks the packet from here (POV_INPUT_PACKETS): hand over the bytes, zero padded to a multiple of 4.
-		// The checks the host walk would have made on the way (floor0, hpp:402; empty submap, hpp:680) depend on the setup
-		// only and are made once, by setup_supports_device_entropy(), before a stream is decoded this way.
-		REQUIRE(len <= 0xFFFFFFFFull, "audio packet too large");
-		pk.packet_bytes = (uint32_t) len;
-		st.payload.insert(st.payload.end(), p, p + len);
-		st.payload.resize((st.payload.size() + 3) & ~(size_t) 3, 0);
-	} else {
 	// 4.3.2 floor curve decode (hpp:478-518): Y values only, the curve itself is rendered on the GPU
 	uint32_t used = 0;
 	for(uint32_t c = 0; c < C; ++c) {
@@ -593,13 +568,69 @@ static bool decode_audio_packet(StreamWork& st, const uint8_t* p, size_t len, in
 			// hpp:680 CHECK(num_channel > 0): a submap without channels is fatal in the reference
 			return fail("residue: submap %u has no channels (hpp:680)", sm);
 		}
-		if(r.type == 2) {
-			const uint8_t one = 1;                       // hpp:688: always decoded, whatever the floors said
-			if(!decode_residue_submap(br, s, r, 1, &one, nch * half, st.payload, fail)) return false;
-		} else {
-			if(!decode_residue_submap(br, s, r, nch, ch_used, half, st.payload, fail)) return false;
-		}
+		const uint8_t one = 1;                           // type 2, hpp:688: always decoded, whatever the floors said
+		const bool ok = r.type == 2 ? decode_residue_submap(br, s, r, 1, &one, nch * half, st.payload, fail)
+		                            : decode_residue_submap(br, s, r, nch, ch_used, half, st.payload, fail);
+		if(!ok) { *status = POV_PKT_VQ_ENTRY; return false; }
 	}
+	return true;
+}
+
+// A packet whose walk failed, as silence: no floor used, and per submap the residue payload of a packet in which no channel is
+// used (entry count 0, every classification 0), the bytes decode_residue_submap writes for it.
+static void silence_audio_packet(StreamWork& st, const MappingSetup& mp, uint32_t half, pov_packet& pk) {
+	const VorbisSetup& s = st.setup;
+	pk.floor_used = 0;
+	for(uint32_t sm = 0; sm < mp.n_submaps; ++sm) {
+		uint32_t nch = 0;
+		for(uint32_t c = 0; c < s.channels; ++c) nch += mp.mux[c] == sm;
+		const ResidueSetup& r = s.residues[mp.submap_residue[sm]];
+		const uint32_t vch = r.type == 2 ? 1 : nch, vlen = r.type == 2 ? nch * half : half;
+		const uint32_t parts = (std::min(r.end, vlen) - std::min(r.begin, vlen)) / r.partition_size;
+		st.payload.resize(st.payload.size() + 4 + (((size_t) vch * parts + 3) & ~(size_t) 3), 0);
+	}
+}
+
+static bool decode_audio_packet(StreamWork& st, const uint8_t* p, size_t len, int64_t expected_end, const Fail& fail, const ParseOptions& opt) {
+	const VorbisSetup& s = st.setup;
+	BitCursor br;
+	br.reset(p, len);
+	st.abs_total_pos.push_back(st.total_pos);
+	st.expected_end.push_back(expected_end);
+	REQUIRE(br.get(1) == 0, "audio packet: packet type bit set (hpp:1142)");
+	const uint32_t mode_idx = br.get(ilog((uint32_t) s.modes.size() - 1));
+	REQUIRE(mode_idx < s.modes.size(), "audio packet: mode %u out of range (hpp:1147)", mode_idx);
+	const ModeSetup& mode = s.modes[mode_idx];
+	const MappingSetup& mp = s.mappings[mode.mapping];
+	uint32_t wflags = 0;
+	if(mode.blockflag) { wflags = br.get(1); wflags |= br.get(1) << 1; }          // hpp:1150-1153
+	const uint32_t n = s.blocksize[mode.blockflag ? 1 : 0], half = n / 2;
+
+	pov_packet pk;
+	memset(&pk, 0, sizeof pk);
+	pk.mode = (uint8_t) mode_idx;
+	pk.window_flags = (uint8_t) wflags;
+	pk.ys_off = st.ys.size();
+	pk.spec_off = st.payload.size();
+	if(st.raw) {
+		// the device walks the packet from here (POV_INPUT_PACKETS): hand over the bytes, zero padded to a multiple of 4.
+		// The checks the host walk would have made on the way (floor0, hpp:402; empty submap, hpp:680) depend on the setup
+		// only and are made once, by setup_supports_device_entropy(), before a stream is decoded this way.
+		REQUIRE(len <= 0xFFFFFFFFull, "audio packet too large");
+		pk.packet_bytes = (uint32_t) len;
+		st.payload.insert(st.payload.end(), p, p + len);
+		st.payload.resize((st.payload.size() + 3) & ~(size_t) 3, 0);
+	} else if(st.walk_bad != UINT32_MAX) {
+		silence_audio_packet(st, mp, half, pk);          // (cut_damage: after the stream's first failed walk)
+	} else {
+		uint32_t status = 0;
+		if(!walk_audio_packet(st, br, mp, half, pk, &status, fail)) {
+			if(!opt.cut_damage) return false;
+			st.walk_bad = (uint32_t) st.packets.size(); st.walk_status = status; st.walk_msg = fail.e.msg;
+			fail.e.failed = false; fail.e.msg.clear();
+			st.ys.resize(pk.ys_off); st.payload.resize(pk.spec_off);
+			silence_audio_packet(st, mp, half, pk);
+		}
 	}
 	// emit bookkeeping (hpp:1061-1067, 1019-1059)
 	st.prev_n = st.cur_n;
@@ -662,11 +693,31 @@ static bool check_comment_packet(const uint8_t* p, size_t len, const Fail& fail)
 	return true;
 }
 
-static bool parse_ogg_file_checked(const uint8_t* data, size_t len, std::vector<StreamWork>& streams, ParseError& err, const ParseOptions& opt);
+// The state of the stream an audio packet is being decoded into, from before the packet: what cut_damage rolls back to.
+struct PacketMark {
+	size_t stream = SIZE_MAX;                            // SIZE_MAX: no audio packet is being decoded
+	size_t ys = 0, payload = 0, positions = 0;
+	uint32_t prev_n = 0, cur_n = 0, walk_bad = UINT32_MAX;
+};
+
+static bool parse_ogg_file_checked(const uint8_t* data, size_t len, std::vector<StreamWork>& streams, ParseError& err, const ParseOptions& opt,
+                                   PacketMark& mark);
 // Never throws: an allocation failure (or any other exception) while parsing hostile input is a parse error like the rest.
 bool parse_ogg_file(const uint8_t* data, size_t len, std::vector<StreamWork>& streams, ParseError& err, const ParseOptions& opt) {
 	try {
-		return parse_ogg_file_checked(data, len, streams, err, opt);
+		PacketMark m;
+		if(parse_ogg_file_checked(data, len, streams, err, opt, m)) return true;
+		if(!opt.cut_damage) return false;
+		if(m.stream != SIZE_MAX) {                       // the failing packet leaves no trace: its stream is a strict parse's of the prefix
+			StreamWork& st = streams[m.stream];
+			st.ys.resize(m.ys); st.payload.resize(m.payload);
+			st.abs_total_pos.resize(m.positions); st.expected_end.resize(m.positions);
+			st.prev_n = m.prev_n; st.cur_n = m.cur_n;
+			if(m.walk_bad == UINT32_MAX) { st.walk_bad = UINT32_MAX; st.walk_status = 0; st.walk_msg.clear(); }
+		}
+		for(StreamWork& st : streams) st.pending.clear();
+		err.cut = true;
+		return true;
 	} catch(const std::bad_alloc&) {
 		err.failed = true; err.msg = "out of memory while parsing (sizes in the stream beyond what this machine can hold)";
 	} catch(const std::exception& e) {
@@ -677,7 +728,8 @@ bool parse_ogg_file(const uint8_t* data, size_t len, std::vector<StreamWork>& st
 	return false;
 }
 
-static bool parse_ogg_file_checked(const uint8_t* data, size_t len, std::vector<StreamWork>& streams, ParseError& err, const ParseOptions& opt) {
+static bool parse_ogg_file_checked(const uint8_t* data, size_t len, std::vector<StreamWork>& streams, ParseError& err, const ParseOptions& opt,
+                                   PacketMark& mark) {
 	Fail fail{err};
 	std::map<uint32_t, size_t> live;                     // serial -> index into streams (erased at EOS, hpp:1480)
 	size_t pos = 0;
@@ -758,10 +810,14 @@ static bool parse_ogg_file_checked(const uint8_t* data, size_t len, std::vector<
 				st.have_setup = true;
 				st.raw = opt.raw_packets && setup_supports_device_entropy(st.setup);
 			} else {
+				mark.stream = live[serial];
+				mark.ys = st.ys.size(); mark.payload = st.payload.size(); mark.positions = st.abs_total_pos.size();
+				mark.prev_n = st.prev_n; mark.cur_n = st.cur_n; mark.walk_bad = st.walk_bad;
 				if(!decode_audio_packet(st, pp, pbytes, expected, fail, opt)) {
 					err.msg = "audio packet " + std::to_string(st.packets.size()) + ": " + err.msg;
 					return false;
 				}
+				mark.stream = SIZE_MAX;
 			}
 			++st.packets_seen;
 			st.pending.clear();

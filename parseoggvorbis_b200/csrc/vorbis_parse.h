@@ -103,23 +103,34 @@ struct StreamWork {
 	std::vector<uint8_t> payload;
 	std::vector<uint64_t> abs_total_pos;      // before the packet (dump: "abs_total_pos")
 	std::vector<int64_t> expected_end;        // dump: "expected_ending_total_pos"
+	// cut_damage with the host walk: the first packet whose walk failed (it and every later packet of the stream are silence,
+	// see ParseOptions), the POV_PKT_* word the device walk reports for that failure (0: none matches) and the host's text
+	uint32_t walk_bad = UINT32_MAX, walk_status = 0;
+	std::string walk_msg;
 	// overlap bookkeeping (hpp:983-988)
 	uint32_t prev_n = 0, cur_n = 0;
 	uint64_t total_pos = 0;
 	uint64_t frames = 0;
 };
 
-struct ParseError { bool failed = false; std::string msg; };
+// cut: the parse ran with cut_damage, found damage and stopped there; msg holds what a strict parse fails with.
+struct ParseError { bool failed = false, cut = false; std::string msg; };
 
 // raw_packets: audio packets are not entropy-decoded here; the descriptors carry the packet bytes (POV_INPUT_PACKETS:
 // mode, window flags and the emit bookkeeping only need the first bits of a packet) and the device walks the rest.
 // allow_spanning: packets may continue on the next page of their stream (RFC 3533 lacing value 255 at a page end +
 // "continued" flag). The reference refuses such files (hpp:89) and so does the default here; real-world encoders produce
 // them routinely (setup headers above 4 KB, high bit rates).
-struct ParseOptions { bool raw_packets = false; bool allow_spanning = false; };
+// cut_damage (POV_PARSE_CUT_DAMAGE): the first failing check of the framing, headers or an audio packet's geometry ends the
+// parse of the file with success and err.cut set: every stream keeps the audio packets completed before it, the failing
+// packet and everything after it are dropped. A failing host walk of an audio packet's floors and residues instead keeps the
+// packet as silence (no floor used, residue payloads that decode nothing) and marks the stream (walk_bad); later packets of
+// that stream are not walked and are silence too.
+struct ParseOptions { bool raw_packets = false; bool allow_spanning = false; bool cut_damage = false; };
 
 // Parses a whole Ogg file from memory (hpp:1428 full_read_from_memory). Streams appear in order of their BOS page.
-// Returns false and fills err on the first failing check, like the reference's OkOrError chain.
+// Returns false and fills err on the first failing check, like the reference's OkOrError chain (with cut_damage, see above;
+// an exception is a failure in both modes).
 bool parse_ogg_file(const uint8_t* data, size_t len, std::vector<StreamWork>& streams, ParseError& err, const ParseOptions& opt = ParseOptions());
 
 // Huffman decode tables from codeword lengths (Vorbis I 3.2.1, hpp:151-185): a first-level table indexed by the next

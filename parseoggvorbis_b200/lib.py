@@ -27,7 +27,7 @@ SYMBOLS = [
     "pov_ogg_vorbis_decode_memory_s16", "pov_decoded_s16_free", "pov_decode_corpus_s16",
     "pov_ogg_parse_memory", "pov_parsed_stream_count", "pov_parsed_get", "pov_parsed_free",
     "pov_batch_upload_into", "pov_corpus_streams", "pov_corpus_streams_free", "pov_decode_corpus_device",
-    "pov_resample_filter", "pov_decode_corpus_device_resampled",
+    "pov_resample_filter", "pov_decode_corpus_device_resampled", "pov_ctx_set_cut_damage", "pov_corpus_report",
 ]
 
 
@@ -126,6 +126,9 @@ def load() -> C.CDLL:
     L.pov_ctx_set_device_entropy.restype = None
     L.pov_ctx_set_page_spanning.argtypes = [vp, i32]
     L.pov_ctx_set_page_spanning.restype = None
+    L.pov_ctx_set_cut_damage.argtypes = [vp, i32]
+    L.pov_ctx_set_cut_damage.restype = None
+    L.pov_corpus_report.argtypes = [vp, u32, C.POINTER(abi.pov_file_report), u64, C.POINTER(u64)]
     L.pov_parsed_stream_count.argtypes = [vp]
     L.pov_parsed_stream_count.restype = u32
     L.pov_parsed_get.argtypes = [vp, u32, C.POINTER(abi.pov_setup), C.POINTER(abi.pov_batch)]
@@ -161,17 +164,18 @@ _STREAM_INFO_DTYPE = np.dtype([("file", "<u4"), ("channels", "<u4"), ("sample_ra
 assert _STREAM_INFO_DTYPE.itemsize == C.sizeof(abi.pov_stream_info)
 
 
-def corpus_streams(files, allow_spanning: bool = False, host_threads: int = 0) -> StreamTable:
+def corpus_streams(files, allow_spanning: bool = False, host_threads: int = 0, cut_damage: bool = False) -> StreamTable:
     """The stream table of a corpus without a GPU: the corpus decode's own parse with the packets discarded, so `frames` is
     what decode_corpus / decode_corpus_device produce. A framing or header error raises PovError with the corpus decode's
-    text ("file k: check failed: ...")."""
+    text ("file k: check failed: ..."); with cut_damage (the table of a decode in cut mode) the damaged file's streams end
+    there instead."""
     L = load()
     arr, lens = _file_arrays(files)
     out = C.POINTER(abi.pov_stream_info)()
     count = C.c_uint64(0)
     err = C.c_char_p(None)
-    rc = L.pov_corpus_streams(len(files), arr, lens, abi.POV_PARSE_ALLOW_SPANNING if allow_spanning else 0, host_threads, C.byref(out),
-                              C.byref(count), C.byref(err))
+    flags = (abi.POV_PARSE_ALLOW_SPANNING if allow_spanning else 0) | (abi.POV_PARSE_CUT_DAMAGE if cut_damage else 0)
+    rc = L.pov_corpus_streams(len(files), arr, lens, flags, host_threads, C.byref(out), C.byref(count), C.byref(err))
     if rc != 0:
         raise PovError(rc, (err.value or b"?").decode())
     try:
@@ -237,6 +241,8 @@ class DeviceCorpus(NamedTuple):
     sample_rate: Optional[int] = None        # resampled / downmixed decode: the target rate (0 = each stream's own rate)
     out_channels: Optional[np.ndarray] = None   # uint32 [streams], channels written per stream
     out_frames: Optional[np.ndarray] = None     # uint64 [streams], frames written per stream
+    valid_frames: Optional[np.ndarray] = None   # uint64 [streams], native frames before each stream's cut (= table.frames if clean)
+    damaged: Optional[dict] = None              # {file index: message} of the damaged files (cut mode; {} when none is)
 
     def stream(self, i: int):
         """(channels, frames) view of stream i (output channels and frames of a resampled / downmixed decode)."""
@@ -250,17 +256,34 @@ class DeviceCorpus(NamedTuple):
         return self.pcm[b:b + c * s].view(c, s)[:, :f]
 
 
+class CorpusReport(NamedTuple):
+    """pov_corpus_report: what the context's last successful corpus call found, per file and per stream-table record."""
+    status: np.ndarray          # uint32 [files]: POV_OK, or POV_ERR_STREAM (damaged and cut)
+    n_streams: np.ndarray       # uint32 [files]: records of the file
+    frames: np.ndarray          # uint64 [files]: = frames_out
+    valid_frames: np.ndarray    # uint64 [files]: summed over the file's streams
+    messages: list              # str [files]: "" or the reason
+    stream_valid_frames: np.ndarray   # uint64 [records]
+
+    @property
+    def damaged(self) -> dict:
+        return {i: m for i, (st, m) in enumerate(zip(self.status, self.messages)) if st != abi.POV_OK}
+
+
 class ParsedOgg:
     """Host-only parse of one Ogg/Vorbis file into descriptor batches (no GPU involved)."""
 
-    def __init__(self, data: bytes, raw_packets: bool = False, allow_spanning: bool = False):
+    def __init__(self, data: bytes, raw_packets: bool = False, allow_spanning: bool = False, cut_damage: bool = False):
         """raw_packets: leave the audio packets as they are (POV_INPUT_PACKETS batches: entropy decode on the device).
-        allow_spanning: accept packets that continue on the next page (the reference refuses them, hpp:89)."""
+        allow_spanning: accept packets that continue on the next page (the reference refuses them, hpp:89).
+        cut_damage: damage ends the parse with the packets before it (POV_PARSE_CUT_DAMAGE)."""
         self.L = load()
         self.h = C.c_void_p(None)
         self._data = data
         err = C.c_char_p(None)
-        rc = self.L.pov_ogg_parse_memory_ex(data, len(data), (1 if raw_packets else 0) | (2 if allow_spanning else 0), C.byref(self.h), C.byref(err))
+        flags = ((abi.POV_PARSE_RAW_PACKETS if raw_packets else 0) | (abi.POV_PARSE_ALLOW_SPANNING if allow_spanning else 0) |
+                 (abi.POV_PARSE_CUT_DAMAGE if cut_damage else 0))
+        rc = self.L.pov_ogg_parse_memory_ex(data, len(data), flags, C.byref(self.h), C.byref(err))
         if rc != 0:
             raise PovError(rc, (err.value or b"?").decode())
 
@@ -320,6 +343,8 @@ class SynthContext:
         self._setups = []
         self.device = device
         self._spanning = int(os.environ.get("POV_ALLOW_SPANNING", "0") or 0) != 0     # the context's default (api.cu)
+        self._cut = False
+        self._corpus_files = None           # files of the last successful corpus call (corpus_report)
 
     def close(self):
         if self.ctx:
@@ -347,6 +372,27 @@ class SynthContext:
     def set_page_spanning(self, on: bool):
         self.L.pov_ctx_set_page_spanning(self.ctx, 1 if on else 0)
         self._spanning = bool(on)
+
+    def set_cut_damage(self, on: bool):
+        """Cut mode of every corpus call on this context (pov_ctx_set_cut_damage): a damaged stream ends where its damage
+        starts, the call goes on, and corpus_report() says what happened to each file."""
+        self.L.pov_ctx_set_cut_damage(self.ctx, 1 if on else 0)
+        self._cut = bool(on)
+
+    def corpus_report(self) -> CorpusReport:
+        """The report of the last successful corpus call on this context (PovError when there is none)."""
+        if self._corpus_files is None:
+            raise PovError(abi.POV_ERR_ARG, "corpus_report: no successful corpus call on this context")
+        n = self._corpus_files
+        files = (abi.pov_file_report * max(1, n))()
+        self._check(self.L.pov_corpus_report(self.ctx, n, files, 0, None))
+        rows = [files[i] for i in range(n)]
+        m = sum(int(r.n_streams) for r in rows)
+        valid = np.zeros(m, np.uint64)
+        self._check(self.L.pov_corpus_report(self.ctx, n, files, m, valid.ctypes.data_as(C.POINTER(C.c_uint64))))
+        return CorpusReport(np.array([r.status for r in rows], np.uint32), np.array([r.n_streams for r in rows], np.uint32),
+                            np.array([r.frames for r in rows], np.uint64), np.array([r.valid_frames for r in rows], np.uint64),
+                            [r.message.decode() for r in rows], valid)
 
     def set_device_entropy(self, on: bool):
         self.L.pov_ctx_set_device_entropy(self.ctx, 1 if on else 0)
@@ -550,8 +596,10 @@ class SynthContext:
         arr, lens = _file_arrays(files)
         frames = np.zeros(len(files), np.uint64)
         total = C.c_uint64(0)
+        self._corpus_files = None
         self._check(fn(self.ctx, len(files), arr, lens, host_threads, *before, frames.ctypes.data_as(C.POINTER(C.c_uint64)),
                        C.byref(total), *after))
+        self._corpus_files = len(files)
         return frames, int(total.value)
 
     def decode_corpus_into(self, files, pcm, table: StreamTable, base, stride, s16: bool = False, host_threads: int = 0,
@@ -593,15 +641,26 @@ class SynthContext:
         return self._decode_corpus_call(self.L.pov_decode_corpus_device_resampled, files, host_threads, (C.byref(o), C.byref(rs)))
 
     def decode_corpus_device(self, files, layout: str = "padded", s16: bool = False, host_threads: int = 0,
-                             sample_rate: Optional[int] = None, mono: bool = False) -> DeviceCorpus:
+                             sample_rate: Optional[int] = None, mono: bool = False, cut_damage: bool = False) -> DeviceCorpus:
         """Decode a corpus straight into a new torch tensor on this context's GPU; only compressed packets go to the device
         and only status words come back. layout "padded": (streams, max channels, T) zeros, T = the longest stream rounded
         up to 4; "packed": one flat tensor, each stream's channels `frames rounded up to 4` apart, back to back. Padding
         stays 0. s16: int16 samples (the POV_PCM_S16 conversion). The stream table is parsed with this context's page-spanning
         setting. sample_rate (Hz, 0 = each stream's own) and mono resample / downmix every stream on the device, and the
-        layouts are then sized by output channels and frames (DeviceCorpus.out_channels / out_frames)."""
+        layouts are then sized by output channels and frames (DeviceCorpus.out_channels / out_frames).
+        cut_damage: cut mode for this call (table and decode); DeviceCorpus.valid_frames and .damaged come from the report."""
+        was = self._cut
+        self.set_cut_damage(cut_damage)
+        try:
+            out = self._decode_corpus_device(files, layout, s16, host_threads, sample_rate, mono)
+        finally:
+            self.set_cut_damage(was)
+        rep = self.corpus_report()
+        return out._replace(valid_frames=rep.stream_valid_frames, damaged=rep.damaged)
+
+    def _decode_corpus_device(self, files, layout, s16, host_threads, sample_rate, mono) -> DeviceCorpus:
         import torch
-        table = corpus_streams(files, allow_spanning=self._spanning, host_threads=host_threads)
+        table = corpus_streams(files, allow_spanning=self._spanning, host_threads=host_threads, cut_damage=self._cut)
         m = len(table)
         resampled = sample_rate is not None or mono
         if resampled:
